@@ -2,6 +2,7 @@
 """bench.py -- rollout env-steps/s including the policy forward, puzzle15 PPO (BASELINE.json metric).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--precision fp32|f16x2|f16x2w16|f16f8c] [--no-extras]
+                  [--dump-outputs DIR]
 
 One "step" = one PPOCollector.collect of `--episodes` (default 65 536) puzzle15 episodes per GPU at
 difficulty 128 (<= 257 records each): reset, per-step policy forward + Gumbel-max sampling + env step +
@@ -15,6 +16,11 @@ The JSON line carries the headline workload (BASELINE.json configs[1]) at top le
 other BASELINE config: puzzle8 PPO, grid_world 5x5 PPO, AlphaZero on puzzle8 (100 simulations at 65 536 episodes and the
 reference's default 512 episodes x 1000 simulations), puzzle15 with twists at 1 M envs in total -- each with its own
 roofline and (at N = 1) cpu_baseline.
+
+`--dump-outputs DIR` writes what the last timed headline step returned -- the records and per-episode lengths of rank 0's
+collect in float32, their row indices and the collect's stats in float64 -- as DIR/<name>.npy.  Inputs are seeded, so the
+same arguments give the same inputs on every run; a collect of more than 2^18 records or episodes is stored as a fixed
+seeded sample of them.
 """
 from __future__ import annotations
 
@@ -199,6 +205,38 @@ class Timer:
         self.ms = self.e0.elapsed_time(self.e1)
 
 
+DUMP_ROWS = 1 << 18       # records (and episodes) --dump-outputs keeps: 104 B a record in float32, about 33 MB in all
+
+
+def dump_rows(n):
+    """All n rows, or a fixed seeded sample of DUMP_ROWS of them: the same indices whenever n is the same."""
+    if n <= DUMP_ROWS:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(0).choice(n, DUMP_ROWS, replace=False))
+
+
+def dump_outputs(out_dir, eng, twc, c):
+    """Write the arrays the last timed collect hands its caller (the CollectedData fields of PPOCollector.collect) to
+    out_dir/<name>.npy, so that two builds run with the same arguments can be compared output for output."""
+    import ctypes as C
+
+    from twisterl_b200 import _lib
+    R, E = int(c.n_records), int(c.num_episodes)
+    # the whole collect comes to the host through the library's own copy-out, as PPOCollector.collect receives it, and
+    # is sampled there: 66 B a puzzle15 record, about 1.1 GB of pageable host memory at 65 536 episodes of difficulty 128
+    # (outside the timed region, and only with --dump-outputs)
+    hb, arrs, _ = twc._host_buffers(R, c.n_cells, c.num_actions, E, pinned=False)
+    _lib.check(_lib.load().twr_collected_to_host(eng._h, C.byref(hb)))
+    rec, ep = dump_rows(R), dump_rows(E)
+    out_dir.mkdir(parents=True, exist_ok=True)
+    for k in ("obs", "logits", "values", "rewards", "advs", "rets", "actions", "perms"):
+        np.save(out_dir / f"{k}.npy", arrs[k][rec].astype(np.float32))
+    np.save(out_dir / "ep_len.npy", arrs["ep_len"][ep].astype(np.float32))
+    np.save(out_dir / "record_index.npy", rec.astype(np.float64))
+    np.save(out_dir / "episode_index.npy", ep.astype(np.float64))
+    np.save(out_dir / "stats.npy", np.array([R, E, c.successes, c.reward_sum], dtype=np.float64))
+
+
 def run_ours(args, rank, local_rank, world):
     import ctypes as C
 
@@ -226,7 +264,7 @@ def run_ours(args, rank, local_rank, world):
         c = collector.collect_device(environment, policy)
         # stats reduction (ncclAllReduce); the reduced numbers are read on the host every iteration, as a trainer logs them
         comm.allreduce([c.num_episodes, c.successes, c.reward_sum, c.n_records])
-        return int(c.n_records)
+        return c
 
     def barrier():
         comm.barrier()
@@ -243,7 +281,8 @@ def run_ours(args, rank, local_rank, world):
     records, fwd_ms, fwd_launches = 0, 0.0, 0
     with Timer(torch, stream) as tm:
         for _ in range(args.steps):
-            records += one_step()
+            last = one_step()
+            records += int(last.n_records)
             f, _, n = eng.last_timing()
             fwd_ms += f; fwd_launches += n
     barrier()
@@ -255,6 +294,8 @@ def run_ours(args, rank, local_rank, world):
     r0_records = records
     records, launches = comm.allreduce([records, launches])
     value = records / (ms * 1e-3)
+    if args.dump_outputs and rank == 0:               # before the e2e collects below replace the engine's last result
+        dump_outputs(Path(args.dump_outputs), eng, twc, last)
 
     # ---- e2e: the C-ABI call with HOST buffers (weights H2D, CollectedData D2H inside the timed region)
     cap = int(L.twr_max_records(C.byref(tw.env.spec_from_env(env)), args.episodes))
@@ -502,7 +543,13 @@ def main():
     ap.add_argument("--no-extras", action="store_true", help="headline workload only")
     ap.add_argument("--extra-steps", type=int, default=3)
     ap.add_argument("--twists", action="store_true", help="enable the {identity, transpose} twist set on the headline workload")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step of the headline workload computed (rank 0's collect) to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

@@ -1,12 +1,23 @@
-"""Shared test helpers: seeded synthetic weights, twist sets, fixtures.  No reference access."""
+"""Shared test helpers: seeded synthetic weights, twist sets, fixtures, and where to find a checkout of the reference."""
 from __future__ import annotations
 
 import json
+import os
 from pathlib import Path
 
 import numpy as np
 
 GOLDEN = Path(__file__).resolve().parent / "golden"
+STAGED_REFERENCE = Path(__file__).resolve().parent.parent / "oracle" / "_ref" / "reference"
+
+
+def reference_checkout() -> Path | None:
+    """A checkout of the reference, AI4quantum/twisteRL: $TWISTERL_REFERENCE, else a copy staged under the git-ignored
+    oracle/_ref/reference; None when neither holds one."""
+    for cand in (os.environ.get("TWISTERL_REFERENCE"), STAGED_REFERENCE):
+        if cand and (Path(cand) / "src" / "twisterl" / "rl" / "ppo.py").is_file():
+            return Path(cand)
+    return None
 
 
 def synth_state_dict(seed, obs_size, emb, hidden, n_act):

@@ -169,25 +169,26 @@ def test_max_records_and_spec_validation():
 
 
 def test_reference_python_half_builds_on_this_module():
-    """Drop-in check that needs the reference checkout (present in the build container only, skipped elsewhere):
-    with twisterl_b200 installed as `twisterl.twisterl`, the reference's own unmodified Python half
+    """Drop-in check that needs a checkout of the reference, AI4quantum/twisteRL (helpers.reference_checkout; skipped
+    without one): with twisterl_b200 installed as `twisterl.twisterl`, the reference's own unmodified Python half
     (twisterl.utils.load_config / prepare_algorithm, BasicPolicy.to_rust) builds PPO and AlphaZero from its own
     JSON configs and hands our nn.Policy / collectors the layouts they expect.  No device is touched."""
     import subprocess
     import sys
-    ref = Path("/root/reference")
-    if not (ref / "src" / "twisterl").is_dir():
-        pytest.skip("reference checkout not available")
+    from helpers import reference_checkout
+    ref = reference_checkout()
+    if ref is None:
+        pytest.skip("no checkout of the reference (set TWISTERL_REFERENCE or stage one under oracle/_ref/reference)")
     code = r'''
 import sys, json
 sys.path.insert(0, %r)
 import twisterl_b200
 twisterl_b200.install_as_twisterl()
-sys.path.insert(0, "/root/reference/src")
+sys.path.insert(0, %r)
 from twisterl.utils import load_config, prepare_algorithm
 out = {}
 for name in ("ppo_puzzle8_v1", "ppo_puzzle15_v1"):
-    algo = prepare_algorithm(load_config("/root/reference/examples/%%s.json" %% name))
+    algo = prepare_algorithm(load_config(%r %% name))
     pol = algo.policy.to_rust()
     out[name] = [type(algo).__name__, type(algo.env).__module__, type(algo.collector).__module__, type(pol).__module__,
                  int(pol.embeddings.vectors.shape[0]), int(pol.embeddings.bias.size), int(pol.num_actions),
@@ -207,7 +208,7 @@ td = td[0] if isinstance(td[0], tuple) else td
 out["torch_shapes"] = [list(t.shape) for t in td]
 algo.train_step(td)
 print(json.dumps(out))
-''' % str(ROOT)
+''' % (str(ROOT), str(ref / "src"), str(ref / "examples" / "%s.json"))
     r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=300, cwd="/tmp")
     assert r.returncode == 0, r.stderr[-2000:]
     import json

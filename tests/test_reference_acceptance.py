@@ -6,25 +6,26 @@ trainer -- `twisterl.utils.prepare_algorithm(load_config("examples/ppo_puzzle8_v
 `python -m twisterl.train` runs (src/twisterl/train.py:21-41) -- trains on this engine far enough for its curriculum to
 raise the difficulty, as does the same object after `twisterl_b200.accelerate()` (device hand-off + device weight sync).
 
-The checkout is looked for in $TWISTERL_REFERENCE, /root/reference (the build container) and oracle/_ref/reference (a staged
-copy for a GPU box; git-ignored).  Nothing here is read by the product or by the other tests."""
+The checkout is $TWISTERL_REFERENCE, else a copy staged under the git-ignored oracle/_ref/reference (helpers.reference_checkout).
+Nothing here is read by the product or by the other tests."""
 import json
-import os
 import subprocess
 import sys
 from pathlib import Path
 
 import pytest
 
+from helpers import reference_checkout
+
 ROOT = Path(__file__).resolve().parent.parent
 pytestmark = pytest.mark.gpu
 
 
 def _reference():
-    for cand in (os.environ.get("TWISTERL_REFERENCE"), "/root/reference", str(ROOT / "oracle" / "_ref" / "reference")):
-        if cand and (Path(cand) / "src" / "twisterl" / "rl" / "ppo.py").is_file():
-            return Path(cand)
-    pytest.skip("no checkout of the reference (set TWISTERL_REFERENCE)")
+    ref = reference_checkout()
+    if ref is None:
+        pytest.skip("no checkout of the reference (set TWISTERL_REFERENCE or stage one under oracle/_ref/reference)")
+    return ref
 
 
 PRELUDE = """
