@@ -181,6 +181,12 @@ int  twr_policy_forward(twr_engine* e, const twr_policy* p, twr_envs* v, const i
 int  twr_policy_forward_obs(twr_engine* e, const twr_policy* p, const int32_t* obs, int64_t n, int32_t n_obs,
                             const int32_t* perm_idx, float* logits, float* values);
 
+/* Policy::full_predict (nn/policy.rs:102-126) for every env of `v`: the raw logits and value of each twist, each divided
+ * by n_perms and added in twist order, then the masked exp / (sum + 1e-6) of Policy::predict.  probs [n][num_actions],
+ * values [n].  Without twists it is Policy::predict.  This is the leaf evaluation of the MCTS searches, by the same
+ * launches and the same averaging code. */
+int  twr_policy_full_predict(twr_engine* e, const twr_policy* p, twr_envs* v, float* probs, float* values);
+
 /* Debug: one forward over `v` with per-CTA cycle counters of the tensor-core kernel's pipeline waits
  * (16 int64 per CTA, max_ctas >= number of SMs; layout documented in twr_forward_tc.cu). */
 int  twr_debug_forward_profile(twr_engine* e, const twr_policy* p, twr_envs* v, int64_t* counters, int32_t max_ctas,
@@ -263,7 +269,9 @@ int  twr_ppo_collect_host(twr_engine* e, const twr_env_spec* spec, twr_policy* p
 /* collector.evaluate (rust/src/rl/evaluate.rs:22-89, python_interface/env.rs:194-207).  With num_mcts_searches > 0
  * every step's action distribution is predict_probs_mcts of the current state (rl/solve.rs:37-48) instead of Policy::predict:
  * num_episodes x [reset, best of num_searches rollouts of single_solve (rl/solve.rs:17-101)] run as one
- * device batch.  Returns (mean success, mean total reward) of the per-episode best (success, reward). */
+ * device batch.  Returns (mean success, mean total reward) of the per-episode best (success, reward).  The search
+ * evaluates its leaves with Policy::full_predict (rl/search.rs:113,150): a policy with twists averages every twist, as
+ * twr_policy_full_predict does. */
 int  twr_evaluate(twr_engine* e, const twr_env_spec* spec, const twr_policy* p, int64_t num_episodes,
                   int32_t deterministic, int32_t num_searches, int32_t num_mcts_searches, float C,
                   int32_t max_expand_depth, float* success_rate, float* mean_reward);
@@ -273,7 +281,8 @@ int  twr_evaluate_episodes(twr_engine* e, const twr_env_spec* spec, const twr_po
                            int32_t max_expand_depth, float* success_rate, float* mean_reward, float* best_success,
                            float* best_reward);
 /* collector.solve (rl/solve.rs:73-101) from the state held by the one-env batch `start`: best of
- * num_searches rollouts; writes its action list (actions may be NULL to only query the score). */
+ * num_searches rollouts; writes its action list (actions may be NULL to only query the score).  With
+ * num_mcts_searches > 0 a policy with twists is searched with full_predict over all of them, as in twr_evaluate. */
 int  twr_solve(twr_engine* e, twr_envs* start, const twr_policy* p, int32_t deterministic, int32_t num_searches,
                int32_t num_mcts_searches, float C, int32_t max_expand_depth,
                float* success, float* reward, int32_t* actions, int32_t max_actions, int32_t* n_actions);
@@ -282,11 +291,13 @@ int  twr_solve(twr_engine* e, twr_envs* start, const twr_policy* p, int32_t dete
  * batched MCTS (predict_probs_mcts, rust/src/rl/search.rs:104-189) whose leaves are evaluated by the same
  * forward kernel as the PPO path.  In the result `logits` holds the MCTS visit distribution (what the reference
  * stores in CollectedData.logits), `rets` holds additional_data["remaining_values"] (az.rs:93), `rewards` and
- * `actions` the per-record reward / drawn action; `values`, `advs` are zero and `perms` is -1. */
+ * `actions` the per-record reward / drawn action; `values`, `advs` are zero and `perms` is -1.  A policy with twists
+ * is refused (TWR_ERR_UNSUPPORTED): the reference's AlphaZero trainer clears them (rl/az.py:24-26). */
 int  twr_az_collect(twr_engine* e, const twr_env_spec* spec, const twr_policy* p, int64_t num_episodes,
                     int32_t num_mcts_searches, float C, int32_t max_expand_depth, twr_collected* out);
 /* predict_probs_mcts for every env of `v` at once (parity API): probs / visit counts [n][num_actions].  Env i
- * draws from Philox stream env_id_base + i at record index t. */
+ * draws from Philox stream env_id_base + i at record index t.  Leaves are evaluated with Policy::full_predict: a
+ * policy with twists averages all of them (twr_policy_full_predict). */
 int  twr_mcts_probs(twr_engine* e, const twr_policy* p, twr_envs* v, int32_t n_sims, float C, int32_t max_expand_depth,
                     uint32_t env_id_base, uint32_t collect_id, int32_t t, float* probs, int32_t* visits);
 

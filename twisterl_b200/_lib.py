@@ -72,7 +72,7 @@ SYMBOLS = [
     "twr_policy_create_from_safetensors", "twr_policy_blob_floats", "twr_policy_update_from_device", "twr_policy_blob_device_ptr", "twr_policy_destroy",
     "twr_envs_create", "twr_envs_destroy", "twr_envs_set_difficulty", "twr_envs_set_state", "twr_envs_set_cell", "twr_envs_reset",
     "twr_envs_step", "twr_envs_get_state", "twr_envs_observe", "twr_envs_masks", "twr_envs_reward",
-    "twr_envs_is_final", "twr_envs_success", "twr_envs_depth", "twr_policy_forward", "twr_policy_forward_obs", "twr_debug_forward_profile", "twr_debug_set_tc_terms", "twr_sample", "twr_gae",
+    "twr_envs_is_final", "twr_envs_success", "twr_envs_depth", "twr_policy_forward", "twr_policy_forward_obs", "twr_policy_full_predict", "twr_debug_forward_profile", "twr_debug_set_tc_terms", "twr_sample", "twr_gae",
     "twr_ppo_collect", "twr_engine_set_collect_id", "twr_collected_to_host", "twr_max_records",
     "twr_ppo_collect_host", "twr_evaluate", "twr_evaluate_episodes", "twr_solve", "twr_az_collect", "twr_mcts_probs", "twr_debug_mcts_trace", "twr_comm_version", "twr_comm_unique_id", "twr_comm_init", "twr_comm_destroy", "twr_broadcast_weights", "twr_allreduce_stats",
     "twr_host_alloc", "twr_host_free", "twr_engine_set_timing", "twr_engine_last_timing",
@@ -132,6 +132,7 @@ def load():
             getattr(L, "twr_envs_" + name).argtypes = [vp, vp]
         L.twr_policy_forward.argtypes = [vp, vp, vp, vp, C.c_int32, vp, vp]
         L.twr_policy_forward_obs.argtypes = [vp, vp, vp, C.c_int64, C.c_int32, vp, vp, vp]
+        L.twr_policy_full_predict.argtypes = [vp, vp, vp, vp, vp]
         L.twr_debug_forward_profile.argtypes = [vp, vp, vp, vp, C.c_int32, C.c_int32]
         L.twr_debug_set_tc_terms.argtypes = [vp, C.c_int32]
         L.twr_sample.argtypes = [vp, vp, C.c_int64, C.c_int32, C.c_uint32, C.c_uint32, C.c_uint32, vp, vp]

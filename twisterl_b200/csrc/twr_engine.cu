@@ -1441,8 +1441,35 @@ static int mcts_acquire(twr_engine* e, int64_t B, int P, MctsPool* pool, MctsArg
 
 static int mcts_pool_nodes(int A, int n_sims, int med) { return 1 + A * (n_sims * (med > 1 ? med : 1) + 1); }
 
-// predict_probs_mcts (rl/search.rs:104-189) for every live env, in lockstep over the simulations
-static void enqueue_mcts(twr_engine* e, const PolicyDev& dev, MctsArgs& a, const int32_t* live, const int32_t* n_live, int64_t B) {
+// Policy::full_predict evaluates every twist: for a twisted policy, a constant [n_perms][B] array whose row pi holds pi
+// (the perm_idx of twist pi's forward) and a.n_perms / a.twist_stride for the averaging; nothing for an untwisted one.
+// The caller sizes the forward outputs a.logits / a.values for n_perms slices of B.
+static int stage_twists(twr_engine* e, const PolicyDev& dev, int64_t B, Staging<int32_t>* idx, MctsArgs* a) {
+    a->n_perms = dev.n_perms; a->twist_stride = B;
+    if (dev.n_perms == 0) return TWR_OK;
+    int rc = idx->alloc((size_t)dev.n_perms * (size_t)B);
+    if (rc) return rc;
+    std::vector<int32_t> h((size_t)dev.n_perms * (size_t)B);
+    for (int pi = 0; pi < dev.n_perms; ++pi) std::fill(h.begin() + (size_t)pi * B, h.begin() + (size_t)(pi + 1) * B, pi);
+    CU_TRY(cudaMemcpyAsync(idx->d, h.data(), sizeof(int32_t) * h.size(), cudaMemcpyHostToDevice, e->stream));
+    return TWR_OK;
+}
+
+// the forward of a leaf batch: one launch, or for a twisted policy one per twist, twist pi's outputs in slice pi
+static void launch_forward_twists(twr_engine* e, const PolicyDev& dev, const ForwardArgs& fa, const int32_t* twist_idx, int64_t stride) {
+    if (dev.n_perms == 0) { launch_forward(e, dev, fa); return; }
+    for (int pi = 0; pi < dev.n_perms; ++pi) {
+        ForwardArgs f = fa;
+        f.perm_idx = twist_idx + (size_t)pi * stride;
+        f.logits = fa.logits + (size_t)pi * stride; f.values = fa.values + (size_t)pi * stride;
+        launch_forward(e, dev, f);
+    }
+}
+
+// predict_probs_mcts (rl/search.rs:104-189) for every live env, in lockstep over the simulations.  twist_idx: the array
+// of stage_twists (NULL for an untwisted policy)
+static void enqueue_mcts(twr_engine* e, const PolicyDev& dev, MctsArgs& a, const int32_t* live, const int32_t* n_live, int64_t B,
+                         const int32_t* twist_idx) {
     cudaStream_t st = e->stream;
     // small batches: one persistent launch runs every simulation of the search (twr_mcts.cu, k_mcts_persistent)
     if (!getenv("TWISTERL_B200_MCTS_LOCKSTEP") && launch_mcts_persistent(st, a, dev, live, n_live, B)) return;
@@ -1450,9 +1477,10 @@ static void enqueue_mcts(twr_engine* e, const PolicyDev& dev, MctsArgs& a, const
     fa.env = a.env; fa.seed = e->seed; fa.cid = a.cid; fa.ids = a.ids; fa.t = -1;
     fa.cells = a.pool.cells; fa.live = a.fwd_list; fa.n = B;
     fa.logits = const_cast<float4*>(a.logits); fa.values = const_cast<float*>(a.values);
+    auto forward = [&]() { launch_forward_twists(e, dev, fa, twist_idx, a.twist_stride); };
     launch_mcts_begin(st, a, live, n_live, B);
     fa.n_live_ptr = a.fwd_count;
-    launch_forward(e, dev, fa);
+    forward();
     launch_mcts_expand(st, a, 0, 0, 0, 0, B);
     if (a.max_expand_depth == 1 && a.n_sims > 0) {
         // one expansion round per simulation: expand/backup of simulation s and the descent of s+1 share a launch
@@ -1460,7 +1488,7 @@ static void enqueue_mcts(twr_engine* e, const PolicyDev& dev, MctsArgs& a, const
         launch_mcts_select(st, a, live, n_live, 0, which, B);
         for (int sim = 0; sim < a.n_sims; ++sim) {
             fa.n_live_ptr = a.fwd_count + which;
-            launch_forward(e, dev, fa);
+            forward();
             if (sim + 1 < a.n_sims) { launch_mcts_expand_select(st, a, live, n_live, sim, which, B); which ^= 1; }
             else launch_mcts_expand(st, a, 1, sim, 0, which, B);
         }
@@ -1474,10 +1502,43 @@ static void enqueue_mcts(twr_engine* e, const PolicyDev& dev, MctsArgs& a, const
         for (int d = 0; d < a.max_expand_depth; ++d) {
             if (d > 0) { which = round & 1; launch_mcts_pre(st, a, live, n_live, which, B); ++round; }
             fa.n_live_ptr = a.fwd_count + which;
-            launch_forward(e, dev, fa);
+            forward();
             launch_mcts_expand(st, a, 1, sim, d, which, B);
         }
     }
+}
+
+
+int twr_policy_full_predict(twr_engine* e, const twr_policy* p, twr_envs* v, float* probs, float* values) {
+    return twr_guard([&]() -> int {
+    if (!e || !p || !v || !probs || !values) return fail(TWR_ERR_INVALID, "NULL argument");
+    if (p->eng != e || v->eng != e) return fail(TWR_ERR_INVALID, "policy/envs belong to another engine");
+    if (v->n == 0) return TWR_OK;
+    PolicyDev dev;
+    int rc = check_policy_env(p, v->p, &dev);
+    if (rc) return rc;
+    CU_TRY(cudaSetDevice(e->device));
+    const int64_t n = v->n;
+    MctsArgs a{};
+    a.env = v->p; a.pool.A = dev.A;
+    const size_t slices = dev.n_perms > 0 ? (size_t)dev.n_perms : 1;
+    Staging<float4> d_logits; Staging<float> d_values, d_probs, d_out; Staging<int32_t> twist_idx;
+    if ((rc = d_logits.alloc(slices * (size_t)n)) || (rc = d_values.alloc(slices * (size_t)n)) || (rc = d_probs.alloc((size_t)n * dev.A)) ||
+        (rc = d_out.alloc((size_t)n)) || (rc = stage_twists(e, dev, n, &twist_idx, &a))) return rc;
+    // the leaf evaluation of the lockstep search: its forward launches, then its averaging and predict epilogue
+    ForwardArgs fa{};
+    fa.env = v->p; fa.seed = e->seed; fa.t = -1; fa.cells = v->cells; fa.n = n;
+    fa.logits = d_logits.d; fa.values = d_values.d;
+    launch_forward_twists(e, dev, fa, twist_idx.d, n);
+    a.logits = d_logits.d; a.values = d_values.d;
+    launch_full_predict(e->stream, a, v->cells, v->meta, n, d_probs.d, d_out.d);
+    CU_TRY(cudaGetLastError());
+    FWD_CHECK(e);
+    CU_TRY(cudaMemcpyAsync(probs, d_probs.d, sizeof(float) * (size_t)n * dev.A, cudaMemcpyDeviceToHost, e->stream));
+    CU_TRY(cudaMemcpyAsync(values, d_out.d, sizeof(float) * (size_t)n, cudaMemcpyDeviceToHost, e->stream));
+    CU_TRY(cudaStreamSynchronize(e->stream));
+    return TWR_OK;
+    });
 }
 
 
@@ -1494,16 +1555,18 @@ static int run_solve(twr_engine* e, const EnvParams& env, const PolicyDev& dev, 
     int rc;
     // num_mcts_searches > 0: every step's action distribution is predict_probs_mcts of the current state
     MctsArgs ma{};
-    Staging<float> mcts_probs; Staging<int32_t> mcts_vis;
+    Staging<float> mcts_probs; Staging<int32_t> mcts_vis, twist_idx;
+    size_t slices = 1;                       // forward output slices of B: one per twist in an MCTS with a twisted policy
     if (mo.n_sims > 0) {
-        if (dev.n_perms > 0) return fail(TWR_ERR_UNSUPPORTED, "MCTS with twists (full_predict over all perms) is not implemented; the AZ trainer clears them (rl/az.py:24-26)");
         const int P = mcts_pool_nodes(dev.A, mo.n_sims, mo.max_expand_depth);
         if ((double)B * P >= 2147483647.0) return fail(TWR_ERR_INVALID, "MCTS node pool too large");
         ma.pool.A = dev.A;
-        if ((rc = mcts_acquire(e, B, P, &ma.pool, &ma)) || (rc = mcts_probs.alloc((size_t)B * dev.A)) || (rc = mcts_vis.alloc((size_t)B * dev.A))) return rc;
+        if ((rc = mcts_acquire(e, B, P, &ma.pool, &ma)) || (rc = mcts_probs.alloc((size_t)B * dev.A)) || (rc = mcts_vis.alloc((size_t)B * dev.A)) ||
+            (rc = stage_twists(e, dev, B, &twist_idx, &ma))) return rc;
+        if (dev.n_perms > 0) slices = (size_t)dev.n_perms;
     }
     if ((rc = live_a.alloc((size_t)B)) || (rc = live_b.alloc((size_t)B)) || (rc = n_live.alloc((size_t)T + 2)) ||
-        (rc = logits.alloc((size_t)B)) || (rc = values.alloc((size_t)B))) return rc;
+        (rc = logits.alloc(slices * (size_t)B)) || (rc = values.alloc(slices * (size_t)B))) return rc;
     cudaStream_t st = e->stream;
     std::vector<int32_t> iota((size_t)B);
     for (int64_t i = 0; i < B; ++i) iota[(size_t)i] = (int32_t)i;
@@ -1532,7 +1595,7 @@ static int run_solve(twr_engine* e, const EnvParams& env, const PolicyDev& dev, 
         int32_t* nxt = (t & 1) ? live_a.d : live_b.d;
         if (mo.n_sims > 0) {
             ma.t = t;
-            enqueue_mcts(e, dev, ma, cur, n_live.d + t, B);
+            enqueue_mcts(e, dev, ma, cur, n_live.d + t, B, twist_idx.d);
             launch_mcts_read(st, ma, B, mcts_probs.d, mcts_vis.d);
         } else {
             fa.t = t; fa.live = cur; fa.n_live_ptr = n_live.d + t;
@@ -1679,7 +1742,6 @@ static int mcts_probs_impl(twr_engine* e, const twr_policy* p, twr_envs* v, int3
     if (!e || !p || !v || !probs || !visits) return fail(TWR_ERR_INVALID, "NULL argument");
     if (p->eng != e || v->eng != e) return fail(TWR_ERR_INVALID, "policy/envs belong to another engine");
     if (n_sims < 0 || max_expand_depth < 0 || t < 0) return fail(TWR_ERR_INVALID, "negative argument");
-    if (p->dev.n_perms > 0) return fail(TWR_ERR_UNSUPPORTED, "MCTS with twists (full_predict over all perms) is not implemented; the AZ trainer clears them (rl/az.py:24-26)");
     if (v->n == 0) return TWR_OK;
     PolicyDev dev;
     int rc = check_policy_env(p, v->p, &dev);
@@ -1691,9 +1753,10 @@ static int mcts_probs_impl(twr_engine* e, const twr_policy* p, twr_envs* v, int3
     MctsArgs a{};
     a.pool.A = dev.A;
     if ((rc = mcts_acquire(e, B, P, &a.pool, &a))) return rc;
-    Staging<float4> logits; Staging<float> values, d_probs; Staging<int32_t> live, n_live, d_vis;
-    if ((rc = logits.alloc((size_t)B)) || (rc = values.alloc((size_t)B)) || (rc = live.alloc((size_t)B)) || (rc = n_live.alloc(1)) ||
-        (rc = d_probs.alloc((size_t)B * dev.A)) || (rc = d_vis.alloc((size_t)B * dev.A))) return rc;
+    Staging<float4> logits; Staging<float> values, d_probs; Staging<int32_t> live, n_live, d_vis, twist_idx;
+    const size_t slices = dev.n_perms > 0 ? (size_t)dev.n_perms : 1;
+    if ((rc = logits.alloc(slices * (size_t)B)) || (rc = values.alloc(slices * (size_t)B)) || (rc = live.alloc((size_t)B)) || (rc = n_live.alloc(1)) ||
+        (rc = d_probs.alloc((size_t)B * dev.A)) || (rc = d_vis.alloc((size_t)B * dev.A)) || (rc = stage_twists(e, dev, B, &twist_idx, &a))) return rc;
     std::vector<int32_t> iota((size_t)B);
     for (int64_t i = 0; i < B; ++i) iota[(size_t)i] = (int32_t)i;
     const int32_t b32 = (int32_t)B;
@@ -1709,7 +1772,7 @@ static int mcts_probs_impl(twr_engine* e, const twr_policy* p, twr_envs* v, int3
         CU_TRY(cudaMemsetAsync(d_trace.d, 0xFF, sizeof(int32_t) * n_trace, e->stream));
         a.trace = d_trace.d;
     }
-    enqueue_mcts(e, dev, a, live.d, n_live.d, B);
+    enqueue_mcts(e, dev, a, live.d, n_live.d, B, twist_idx.d);
     launch_mcts_read(e->stream, a, B, d_probs.d, d_vis.d);
     CU_TRY(cudaGetLastError());
     FWD_CHECK(e);
@@ -1756,7 +1819,7 @@ int twr_az_collect(twr_engine* e, const twr_env_spec* spec, const twr_policy* p,
         int32_t* cur = (t & 1) ? b.live_b : b.live_a;
         int32_t* nxt = (t & 1) ? b.live_a : b.live_b;
         a.t = t;
-        enqueue_mcts(e, plan.dev, a, cur, b.n_live + t, B);
+        enqueue_mcts(e, plan.dev, a, cur, b.n_live + t, B, nullptr);
         launch_az_finish(st, a, b, cur, nxt);
         if ((t & 7) == 7) {                      // stop early once every episode has ended (MCTS steps are expensive)
             int32_t left = 0;

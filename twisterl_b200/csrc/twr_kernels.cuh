@@ -177,6 +177,8 @@ struct MctsArgs {
     int32_t* fwd_list; int32_t* fwd_env; int32_t* fwd_count;   // leaf batch: node indices, env ids, two counters
     int32_t* leaf_pos;                                          // [B] leaf-batch slot of env e in the current simulation
     const float4* logits; const float* values;           // forward outputs, indexed by leaf-batch position
+    // twisted policies (Policy::full_predict): one forward per twist pi, its outputs at logits / values + pi * twist_stride
+    int n_perms; int64_t twist_stride;
     int32_t* cur_node; float* cur_value; uint8_t* active; // per env, current simulation
     int32_t* trace;   // optional [n_sims][B][2] (parity API): leaf of the descent, node the value was backed up from
     long long* dbg;   // optional [8] cycle counters of cluster 0 / CTA 0 / thread 0 of k_mcts_persistent (TWISTERL_B200_MCTS_DEBUG)
@@ -188,5 +190,8 @@ void launch_mcts_expand_select(cudaStream_t s, const MctsArgs& a, const int32_t*
 void launch_mcts_pre(cudaStream_t s, const MctsArgs& a, const int32_t* live, const int32_t* n_live, int which, int64_t max_n);
 void launch_mcts_read(cudaStream_t s, const MctsArgs& a, int64_t n, float* probs, int32_t* visits);
 bool launch_mcts_persistent(cudaStream_t s, const MctsArgs& a, const PolicyDev& p, const int32_t* live, const int32_t* n_live, int64_t max_n);
+// Policy::full_predict of n envs from the forward outputs of every twist (a.logits / a.values, a.n_perms slices):
+// probs [n][a.pool.A], values [n]; the leaf evaluation of the lockstep search
+void launch_full_predict(cudaStream_t s, const MctsArgs& a, const uint4* cells, const uint32_t* meta, int64_t n, float* probs, float* values);
 void launch_az_finish(cudaStream_t s, const MctsArgs& a, const CollectBuffers& b, const int32_t* live, int32_t* live_next);
 void launch_az_remaining(cudaStream_t s, const CollectBuffers& b);

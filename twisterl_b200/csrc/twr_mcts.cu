@@ -10,8 +10,10 @@
 // of a parent-pointer walk.  All envs advance in lockstep, one simulation at a time:
 //   k_mcts_select : UCB descent to a leaf (search.rs:134-137, ucb :29-39, next :77-91); terminal leaves back up
 //                   their reward at once, the others are compacted (warp ballot) into the leaf batch
-//   forward       : the SAME policy forward kernel as the PPO path evaluates the whole leaf batch (K2)
-//   k_mcts_expand : Policy::predict epilogue (masked exp / (sum+1e-6)), expand (search.rs:56-75), child draw
+//   forward       : the SAME policy forward kernel as the PPO path evaluates the whole leaf batch (K2); a twisted policy
+//                   takes one forward per twist, each into its own slice of the outputs
+//   k_mcts_expand : Policy::full_predict's average of the twist slices (nn/policy.rs:102-126; one slice and no average
+//                   without twists), Policy::predict epilogue (masked exp / (sum+1e-6)), expand (search.rs:56-75), child draw
 //                   proportional to the priors (next_sample :94-100), backup (search.rs:45-53)
 // k_az_finish turns root visit counts into the MCTS policy (search.rs:166-188), draws the action
 // (az.rs:72), writes the record and steps the env; k_az_remaining computes az.rs:93's reward-to-go.
@@ -92,6 +94,25 @@ __device__ __forceinline__ void masked_probs(const float4 raw, uint32_t mask, in
     for (int i = 0; i < 4; ++i) { pr[i] = (i < A && ((mask >> i) & 1u)) ? expf(l[i]) : 0.0f; sum += pr[i]; }
 #pragma unroll
     for (int i = 0; i < 4; ++i) pr[i] = pr[i] / (sum + 0.000001f);
+}
+
+// one term of Policy::full_predict's average (nn/policy.rs:109-115): acc += raw / n_perms per logit and for the value,
+// each term divided before it is added; called for twists 0, 1, .. in that order
+__device__ __forceinline__ void twist_accumulate(float4& acc, float& vacc, const float4 raw, float v, float np) {
+    acc.x = __fadd_rn(acc.x, __fdiv_rn(raw.x, np)); acc.y = __fadd_rn(acc.y, __fdiv_rn(raw.y, np));
+    acc.z = __fadd_rn(acc.z, __fdiv_rn(raw.z, np)); acc.w = __fadd_rn(acc.w, __fdiv_rn(raw.w, np));
+    vacc = __fadd_rn(vacc, __fdiv_rn(v, np));
+}
+
+// raw logits and value of the leaf at forward-batch position pos: Policy::predict's without twists, full_predict's
+// average over the a.n_perms forward slices with them
+__device__ __forceinline__ float4 leaf_eval(const MctsArgs& a, int64_t pos, float& v) {
+    if (a.n_perms == 0) { v = a.values[pos]; return a.logits[pos]; }
+    const float np = (float)a.n_perms;
+    float4 acc = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+    v = 0.0f;
+    for (int pi = 0; pi < a.n_perms; ++pi) twist_accumulate(acc, v, a.logits[pi * a.twist_stride + pos], a.values[pi * a.twist_stride + pos], np);
+    return acc;
 }
 
 // MCTSTree::expand (search.rs:56-75): one child per action with prior > 0, in action order.  Returns the first
@@ -178,8 +199,8 @@ __device__ __forceinline__ void expand_body(const MctsArgs& a, int e, int pos, i
     const int64_t base = (int64_t)e * m.P;
     const int node = mode == 0 ? 0 : a.cur_node[e];
     const EnvState s = node_state(m, base + node);
-    float pr[4];
-    masked_probs(a.logits[pos], env_masks(a.env, s), m.A, pr);
+    float pr[4], v;
+    masked_probs(leaf_eval(a, pos, v), env_masks(a.env, s), m.A, pr);
     float cp[4];
     int nch;
     const int first = expand(m, a.env, e, base, node, pr, cp, nch);
@@ -191,7 +212,6 @@ __device__ __forceinline__ void expand_body(const MctsArgs& a, int e, int pos, i
                   (uint32_t)a.seed, (uint32_t)(a.seed >> 32), w);
     const int child = nch > 0 ? first + weighted_index(cp, nch, u32_to_unit_f32(w[0])) : node;
     if (a.trace) a.trace[((int64_t)sim * m.B + e) * 2 + 1] = child;
-    const float v = a.values[pos];
     int len = m.path_len[e];
     if (child != node && len >= 0) {                     // the drawn child joins the recorded path
         if (len < TWR_MCTS_PATH) { m.path[(int64_t)len * m.B + e] = child; ++len; } else len = -1;
@@ -350,6 +370,18 @@ __global__ void __launch_bounds__(128) k_mcts_read(MctsArgs a, int64_t n, float*
     for (int i = 0; i < a.pool.A; ++i) { probs[e * a.pool.A + i] = pr[i]; visits[e * a.pool.A + i] = vis[i]; }
 }
 
+// Policy::full_predict (nn/policy.rs:102-126) of env e from the forward slices at position e: what expand_body
+// computes for a leaf (parity API)
+__global__ void __launch_bounds__(128) k_full_predict(MctsArgs a, const uint4* __restrict__ cells, const uint32_t* __restrict__ meta,
+                                                      int64_t n, float* __restrict__ probs, float* __restrict__ values) {
+    const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= n) return;
+    float pr[4], v;
+    masked_probs(leaf_eval(a, e, v), env_masks(a.env, env_load(cells, meta, e)), a.pool.A, pr);
+    for (int i = 0; i < a.pool.A; ++i) probs[e * a.pool.A + i] = pr[i];
+    values[e] = v;
+}
+
 // one AZCollector loop iteration (az.rs:66-88) for every live env
 __global__ void __launch_bounds__(128) k_az_finish(MctsArgs a, CollectBuffers b, const int32_t* __restrict__ live,
                                                    int32_t* __restrict__ live_next) {
@@ -468,6 +500,12 @@ __device__ __forceinline__ T* pm_remote(T* p, uint32_t rank) {
     return reinterpret_cast<T*>(out);
 }
 
+// TW: a twisted policy (Policy::full_predict at every leaf).  A leaf slot is then a (tree, twist) pair: the PM_TPC slots hold
+// PM_CS * (PM_TPC / PM_CS / T) trees of T slots each.  Slot g belongs to owner CTA g % PM_CS and is that CTA's local slot
+// l = g / PM_CS; local slots l = w*T .. w*T + T-1 are the twists of the tree owned by warp w, so the T evaluations of a tree
+// meet in its owner CTA (phase C) and are averaged by its owner warp (phase D).  Phase A stays per tree.  The twist tables
+// are read through the read-only data path: GridWorld 5x5's table already fills shared memory (pm_layout).
+template <bool TW>
 __global__ void __launch_bounds__(PM_THREADS, 1)
 k_mcts_persistent(MctsArgs a, PolicyDev p, const int32_t* __restrict__ live, const int32_t* __restrict__ n_live, int pos0, int cap) {
     extern __shared__ __align__(16) unsigned char pm_smem[];
@@ -510,10 +548,19 @@ k_mcts_persistent(MctsArgs a, PolicyDev p, const int32_t* __restrict__ live, con
     const int ncl = (int)pm_nclusters();
     const int per = (n + ncl - 1) / ncl;
     const int first = pos0 + (int)pm_cluster_id() * per;
-    const int nt = max(0, min(per, pos0 + n - first));     // host guarantees per <= PM_TPC
+    const int nt = max(0, min(per, pos0 + n - first));     // host guarantees per <= PM_CS * (PM_TPC / PM_CS / T)
+    const int T = TW ? p.n_perms : 1;                      // leaf slots per tree
+    // leaf slots in use: g < ns (untwisted: slot g is tree g)
+    const int ns = TW ? PM_CS * ((nt + PM_CS - 1) / PM_CS) * T : nt;
+    auto slot_tree = [&](int g, int& pi) -> int {          // the tree of slot g (-1: none) and its twist
+        if (!TW) { pi = -1; return g; }
+        const int l = g / PM_CS, j = (l / T) * PM_CS + g % PM_CS;
+        pi = l % T;
+        return j < nt ? j : -1;
+    };
     const int warp = tid >> 5, lane = tid & 31;
-    const int j_own = warp * PM_CS + (int)rank;            // the tree this WARP owns (slot `warp` of this CTA)
-    const bool owner = warp < PM_TPC / PM_CS && j_own < nt;    // warp-uniform
+    const int j_own = warp * PM_CS + (int)rank;            // the tree this WARP owns (local slots warp*T .. warp*T + T-1 of this CTA)
+    const bool owner = warp < PM_TPC / PM_CS / T && j_own < nt;    // warp-uniform
     int e = 0, node = 0, len = 1;
     int64_t base = 0;
     bool need = false;
@@ -586,28 +633,33 @@ k_mcts_persistent(MctsArgs a, PolicyDev p, const int32_t* __restrict__ live, con
         pm_cluster_sync();
         if (prof) { const long long t = clock64(); tS1 += t - t0; t0 = t; }
         // ================= B: embedding slice (local), then this K-slice of W1.h1 for every column =================
-        for (int idx = tid; idx < nt * (EC / 4); idx += PM_THREADS) {
-            const int j = idx / (EC / 4), f4 = (idx % (EC / 4)) * 4;
-            if (!leaf_flag[j]) continue;
+        for (int idx = tid; idx < ns * (EC / 4); idx += PM_THREADS) {
+            const int g = idx / (EC / 4), f4 = (idx % (EC / 4)) * 4;
+            int pi;
+            const int j = slot_tree(g, pi);
+            if ((TW && j < 0) || !leaf_flag[j]) continue;
             const uint4 c = leaf_cells[j];
             EnvState s; s.blank = 0; s.depth = 0;
             s.lo = (uint64_t)c.x | ((uint64_t)c.y << 32); s.hi = (uint64_t)c.z | ((uint64_t)c.w << 32);
             float4 acc = *reinterpret_cast<const float4*>(embb + f4);                       // bias first, then the rows in
             for (int i = 0; i < a.env.N; ++i) {                                              // observation order (layers.rs:58-62)
-                const int r = i * a.env.N + (int)env_board(a.env, s, i);
+                int r = i * a.env.N + (int)env_board(a.env, s, i);
+                if (TW) r = __ldg(p.obs_perms + (size_t)pi * p.obs_size + r);               // twist-in, policy.rs:81-83
                 const float4 t4 = *reinterpret_cast<const float4*>(tab + (size_t)r * EC + f4);
                 acc.x = __fadd_rn(acc.x, t4.x); acc.y = __fadd_rn(acc.y, t4.y); acc.z = __fadd_rn(acc.z, t4.z); acc.w = __fadd_rn(acc.w, t4.w);
             }
             acc.x = fmaxf(acc.x, 0.f); acc.y = fmaxf(acc.y, 0.f); acc.z = fmaxf(acc.z, 0.f); acc.w = fmaxf(acc.w, 0.f);
-            *reinterpret_cast<float4*>(h1s + (size_t)j * EC + f4) = acc;
+            *reinterpret_cast<float4*>(h1s + (size_t)g * EC + f4) = acc;
         }
         __syncthreads();
-        for (int i = lg; i < nt; i += nlg) {
+        for (int i = lg; i < ns; i += nlg) {
             // leaf order rotated by the CTA rank: at any moment the PM_CS senders address PM_CS different owner CTAs
             // (all of them sending leaf j at once would queue on one shared-memory port: measured 2x on the whole search)
-            const int j = (i + (int)rank) % nt;
-            if (!leaf_flag[j]) continue;
-            const float4* x = reinterpret_cast<const float4*>(h1s + (size_t)j * EC);
+            const int g = (i + (int)rank) % ns;
+            int pi;
+            const int j = slot_tree(g, pi);
+            if ((TW && j < 0) || !leaf_flag[j]) continue;
+            const float4* x = reinterpret_cast<const float4*>(h1s + (size_t)g * EC);
             float acc = 0.0f;
 #pragma unroll
             for (int k4 = 0; k4 < PM_MAX_EC / 4; ++k4) {
@@ -617,19 +669,20 @@ k_mcts_persistent(MctsArgs a, PolicyDev p, const int32_t* __restrict__ live, con
                     acc = fmaf(wreg[4 * k4 + 2], v.z, acc); acc = fmaf(wreg[4 * k4 + 3], v.w, acc);
                 }
             }
-            // to the tree's owner CTA: part2[tree slot j / PM_CS][this rank][col]
-            pm_remote(part2, (uint32_t)(j % PM_CS))[((size_t)(j / PM_CS) * PM_CS + rank) * H + col] = acc;
+            // to the tree's owner CTA: part2[local slot g / PM_CS][this rank][col]
+            pm_remote(part2, (uint32_t)(g % PM_CS))[((size_t)(g / PM_CS) * PM_CS + rank) * H + col] = acc;
         }
         if (prof) { const long long t = clock64(); tB += t - t0; t0 = t; }
         pm_cluster_sync();
         if (prof) { const long long t = clock64(); tS2 += t - t0; t0 = t; }
         // ================= C: h2 and the heads of MY trees (local) =================
         {
-            const int my_slots = (nt - (int)rank + PM_CS - 1) / PM_CS;          // trees this CTA owns (slot jl <-> tree jl*PM_CS + rank)
+            // local slots of the trees this CTA owns (slot jl <-> tree (jl / T)*PM_CS + rank, twist jl % T)
+            const int my_slots = (nt - (int)rank + PM_CS - 1) / PM_CS * T;
             // C1: h2 of my trees, thread = column (independent loads per slot)
             for (int jl = lg; jl < my_slots; jl += nlg) {
                 float h = 0.0f;
-                if (leaf_flag[jl * PM_CS + rank]) {
+                if (leaf_flag[(TW ? jl / T : jl) * PM_CS + rank]) {
                     const float* q = part2 + (size_t)jl * PM_CS * H + col;
 #pragma unroll
                     for (int r = 0; r < PM_CS; ++r) h += q[r * H];               // the K-slices in ascending order
@@ -660,12 +713,30 @@ k_mcts_persistent(MctsArgs a, PolicyDev p, const int32_t* __restrict__ live, con
                 int child = node;
                 float v = 0.0f;
                 if (lane == 0) {
-                    float l[5];
+                    float4 raw;
+                    if (!TW) {
+                        float l[5];
 #pragma unroll
-                    for (int o = 0; o < 5; ++o) l[o] = red[warp * 8 + o];
-                    const float4 raw = make_float4(l[0] + (p.A > 0 ? p.ba[0] : 0.f), l[1] + (p.A > 1 ? p.ba[1] : 0.f), l[2] + (p.A > 2 ? p.ba[2] : 0.f),
-                                                   l[3] + (p.A > 3 ? p.ba[3] : 0.f));
-                    v = l[4] + p.bv[0];
+                        for (int o = 0; o < 5; ++o) l[o] = red[warp * 8 + o];
+                        raw = make_float4(l[0] + (p.A > 0 ? p.ba[0] : 0.f), l[1] + (p.A > 1 ? p.ba[1] : 0.f), l[2] + (p.A > 2 ? p.ba[2] : 0.f),
+                                          l[3] + (p.A > 3 ? p.ba[3] : 0.f));
+                        v = l[4] + p.bv[0];
+                    } else {                                    // full_predict: every twist's heads, twisted out, then averaged
+                        const float np = (float)T;
+                        raw = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+                        for (int pi = 0; pi < T; ++pi) {
+                            const float* rs = red + (warp * T + pi) * 8;
+                            float l[4], out[4];
+#pragma unroll
+                            for (int o = 0; o < 4; ++o) l[o] = rs[o] + (p.A > o ? p.ba[o] : 0.f);
+#pragma unroll
+                            for (int o = 0; o < 4; ++o) {                // twist-out, policy.rs:95-97 (bias included)
+                                const int src = o < p.A ? __ldg(p.act_perms + pi * p.A + o) : o;
+                                out[o] = src == 0 ? l[0] : src == 1 ? l[1] : src == 2 ? l[2] : l[3];
+                            }
+                            twist_accumulate(raw, v, make_float4(out[0], out[1], out[2], out[3]), rs[4] + p.bv[0], np);
+                        }
+                    }
                     const EnvState s = node_state(m, base + node);
                     float pr[4], cp[4];
                     masked_probs(raw, env_masks(a.env, s), m.A, pr);
@@ -725,6 +796,10 @@ void launch_mcts_read(cudaStream_t st, const MctsArgs& a, int64_t n, float* prob
     k_mcts_read<<<grid_for(n, 128), 128, 0, st>>>(a, n, probs, visits);
     TWR_COUNT_LAUNCH();
 }
+void launch_full_predict(cudaStream_t st, const MctsArgs& a, const uint4* cells, const uint32_t* meta, int64_t n, float* probs, float* values) {
+    k_full_predict<<<grid_for(n, 128), 128, 0, st>>>(a, cells, meta, n, probs, values);
+    TWR_COUNT_LAUNCH();
+}
 void launch_az_finish(cudaStream_t st, const MctsArgs& a, const CollectBuffers& b, const int32_t* live, int32_t* live_next) {
     k_az_finish<<<grid_for(b.B, 128), 128, 0, st>>>(a, b, live, live_next);
     TWR_COUNT_LAUNCH();
@@ -737,8 +812,14 @@ void launch_az_remaining(cudaStream_t st, const CollectBuffers& b) {
 // Whole-search persistent kernel (small batches, max_expand_depth == 1).  Returns false when it does not apply: the caller
 // then runs the lockstep path.
 bool launch_mcts_persistent(cudaStream_t st, const MctsArgs& a, const PolicyDev& p, const int32_t* live, const int32_t* n_live, int64_t max_n) {
-    if (p.generic || a.max_expand_depth != 1 || p.n_perms > 0 || max_n < 1) return false;
+    if (p.generic || a.max_expand_depth != 1 || max_n < 1) return false;
     if (p.E % (PM_CS * 4) || p.E > PM_CS * PM_MAX_EC || (p.H != 128 && p.H != 256) || p.A > 4) return false;
+    // a twisted search takes T = n_perms leaf slots per tree: whole trees per CTA, at least one
+    const int T = p.n_perms > 0 ? p.n_perms : 1;
+    const int tpc = PM_CS * (PM_TPC / PM_CS / T);          // trees per cluster
+    if (tpc < PM_CS) return false;
+    void (*kern)(MctsArgs, PolicyDev, const int32_t*, const int32_t*, int, int) =
+        p.n_perms > 0 ? k_mcts_persistent<true> : k_mcts_persistent<false>;
     const PmLayout L = pm_layout(p.E, p.H, p.obs_size);
     if (L.total > 227 * 1024) return false;
     int dev = 0;
@@ -748,24 +829,24 @@ bool launch_mcts_persistent(cudaStream_t st, const MctsArgs& a, const PolicyDev&
     at[0].id = cudaLaunchAttributeClusterDimension;
     at[0].val.clusterDim.x = PM_CS; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
     cfg.blockDim = dim3(PM_THREADS); cfg.dynamicSmemBytes = L.total; cfg.stream = st; cfg.attrs = at; cfg.numAttrs = 1;
-    if (cudaFuncSetAttribute(k_mcts_persistent, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)L.total) != cudaSuccess) { cudaGetLastError(); return false; }
+    if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)L.total) != cudaSuccess) { cudaGetLastError(); return false; }
     int sms = 0, nc = 0;
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
     cfg.gridDim = dim3((unsigned)((sms / PM_CS) * PM_CS));
     // clusters of this size and shared-memory footprint the device holds at once (a host-side computation): all of a
     // launch's clusters are then resident, although nothing here waits on another cluster
-    if (cudaOccupancyMaxActiveClusters(&nc, k_mcts_persistent, &cfg) != cudaSuccess) { cudaGetLastError(); nc = 0; }
+    if (cudaOccupancyMaxActiveClusters(&nc, kern, &cfg) != cudaSuccess) { cudaGetLastError(); nc = 0; }
     if (nc > sms / PM_CS) nc = sms / PM_CS;
     if (nc < 1) return false;
     // Searches cost the same whether a cluster holds 1 or PM_TPC trees (latency bound), so the batch is cut into as few
     // launches as the resident clusters allow; beyond a few thousand trees the lockstep path's batched forward wins.
-    const int64_t room = (int64_t)nc * PM_TPC;
+    const int64_t room = (int64_t)nc * tpc;
     const int n_launch = (int)((max_n + room - 1) / room);
     if (n_launch > 4) return false;
     const int slice = (int)((max_n + n_launch - 1) / n_launch);
     if (getenv("TWISTERL_B200_MCTS_DEBUG"))
-        fprintf(stderr, "[mcts] persistent: %lld trees, %d resident clusters of %d CTAs (%zu B shared memory), %d launch(es) of <= %d trees\n",
-                (long long)max_n, nc, PM_CS, L.total, n_launch, slice);
+        fprintf(stderr, "[mcts] persistent: %lld trees, %d twist(s), %d resident clusters of %d CTAs (%zu B shared memory), %d launch(es) of <= %d trees\n",
+                (long long)max_n, p.n_perms, nc, PM_CS, L.total, n_launch, slice);
     MctsArgs args = a;
     static long long* d_dbg_dev[64] = {nullptr};           // debug counters, one buffer per device
     long long* d_dbg = nullptr;
@@ -778,7 +859,7 @@ bool launch_mcts_persistent(cudaStream_t st, const MctsArgs& a, const PolicyDev&
         const int pos0 = i * slice;
         const int ncl = slice < nc ? slice : nc;
         cfg.gridDim = dim3((unsigned)(ncl * PM_CS));
-        if (cudaLaunchKernelEx(&cfg, k_mcts_persistent, args, p, live, n_live, pos0, slice) != cudaSuccess) { cudaGetLastError(); return false; }
+        if (cudaLaunchKernelEx(&cfg, kern, args, p, live, n_live, pos0, slice) != cudaSuccess) { cudaGetLastError(); return false; }
         TWR_COUNT_LAUNCH();
     }
     if (args.dbg) {

@@ -257,6 +257,17 @@ def forward_batch(engine: _lib.Engine, policy: Policy, batch, perm_idx=None, app
     return logits, values
 
 
+def full_predict_batch(engine: _lib.Engine, policy: Policy, batch):
+    """Batched Policy::full_predict (twr_policy_full_predict), the leaf evaluation of the MCTS searches:
+    (probs [n][A], values [n])."""
+    n, A = batch.n, policy.num_actions
+    probs = np.zeros((n, A), dtype=np.float32)
+    values = np.zeros(n, dtype=np.float32)
+    _lib.check(_lib.load().twr_policy_full_predict(engine._h, policy.device_handle(engine), batch._h,
+                                                   _lib.ptr(probs), _lib.ptr(values)))
+    return probs, values
+
+
 def forward_obs(engine: _lib.Engine, policy: Policy, obs, perm_idx=None):
     """Batched _raw_predict on sparse observations given directly (twr_policy_forward_obs)."""
     o = np.ascontiguousarray(obs, dtype=np.int32)
