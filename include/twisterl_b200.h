@@ -188,7 +188,8 @@ int  twr_policy_forward_obs(twr_engine* e, const twr_policy* p, const int32_t* o
 int  twr_policy_full_predict(twr_engine* e, const twr_policy* p, twr_envs* v, float* probs, float* values);
 
 /* Debug: one forward over `v` with per-CTA cycle counters of the tensor-core kernel's pipeline waits
- * (16 int64 per CTA, max_ctas >= number of SMs; layout documented in twr_forward_tc.cu). */
+ * (16 int64 per CTA, max_ctas >= number of SMs; the counters are written at the end of k_forward_tc2 in
+ * twr_forward_tc2.cu, and scripts/profile_tc.py names them). */
 int  twr_debug_forward_profile(twr_engine* e, const twr_policy* p, twr_envs* v, int64_t* counters, int32_t max_ctas,
                                int32_t experiment_flags /* 0 = none; results are invalid when non-zero */);
 /* Debug / precision ladder: which split-operand terms the tensor-core forward of this engine accumulates on top of the

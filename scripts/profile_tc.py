@@ -1,4 +1,4 @@
-"""Per-CTA pipeline wait counters of k_forward_tc (twr_debug_forward_profile)."""
+"""Per-CTA pipeline wait counters of k_forward_tc2 (twr_debug_forward_profile)."""
 import sys
 from pathlib import Path
 import numpy as np

@@ -777,10 +777,11 @@ def test_two_engines_on_two_devices_in_one_process():
         pol.release(); eng.close()
 
 
-@pytest.mark.parametrize("E,H", [(256, 256), (768, 256), (1024, 128), (256, 128)])
+@pytest.mark.parametrize("E,H", [(256, 256), (768, 256), (1024, 128), (256, 128), (128, 256), (384, 256), (640, 128), (896, 128)])
 def test_forward_and_collect_other_layer_widths(eng, E, H):
-    """Embedding widths of 2, 6 and 8 chunk pairs and both common widths of the pair kernel (the shipped configs are all
-    E = 512): forward against the oracle on scrambled states, and a collect replayed record by record."""
+    """Embedding widths of 1 to 8 chunks of 128 features (an odd count runs zero-padded to the next chunk pair) and both
+    common widths of the pair kernel (the shipped configs are all E = 512): forward against the oracle on scrambled states,
+    and a collect replayed record by record."""
     import twisterl_b200 as tw
     from parity import check_collect_against_oracle, make_policies
     from twisterl_b200.env import EnvBatch

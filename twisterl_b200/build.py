@@ -15,7 +15,7 @@ from pathlib import Path
 PKG = Path(__file__).resolve().parent
 CSRC = PKG / "csrc"
 LIB = PKG / "lib" / "libtwisterl_b200.so"
-SOURCES = ["twr_engine.cu", "twr_kernels.cu", "twr_forward_fp32.cu", "twr_forward_tc.cu", "twr_forward_tc2.cu", "twr_forward_generic.cu", "twr_mcts.cu", "twr_comm.cu", "twr_safetensors.cpp"]
+SOURCES = ["twr_engine.cu", "twr_kernels.cu", "twr_forward_fp32.cu", "twr_forward_tc2.cu", "twr_forward_generic.cu", "twr_mcts.cu", "twr_comm.cu", "twr_safetensors.cpp"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC", "-Xcompiler", "-Wall", "--expt-relaxed-constexpr"]
 

@@ -409,7 +409,7 @@ static int upload_policy(twr_policy* p, const twr_policy_desc* d) {
         CU_TRY(cudaMemcpyAsync(p->d_obs_perms, d->obs_perms, sizeof(int32_t) * (size_t)d->n_perms * d->obs_size, cudaMemcpyHostToDevice, st));
         CU_TRY(cudaMemcpyAsync(p->d_act_perms, d->act_perms, sizeof(int32_t) * (size_t)d->n_perms * A, cudaMemcpyHostToDevice, st));
     }
-    if (p->tc_pack) launch_forward_tc_pack(st, p->dev, p->tc_pack);
+    if (p->tc_pack) launch_forward_tc2_pack(st, p->dev, p->tc_pack);
     CU_TRY(cudaStreamSynchronize(st));   // host source buffers may be freed by the caller after return
     return TWR_OK;
 }
@@ -453,8 +453,8 @@ int twr_policy_create(twr_engine* e, const twr_policy_desc* d_in, twr_policy** o
         probe.n_obs = 1;
         EnvParams dummy{};
         const char* why = "";
-        // TWR_PREC_F16X2 = tensor cores where the shape fits the tcgen05 kernel (obs_size <= 256, E % 128 == 0, H in
-        // {128, 256}); other shapes (GridWorld's 625-row table) run the fp32 SIMT kernel -- still on the device.
+        // TWR_PREC_F16X2 = tensor cores where the shape fits the tcgen05 kernel (obs_size <= 256, E % 128 == 0 and
+        // E <= 1024, H in {128, 256}); other shapes (GridWorld's 625-row table) run the fp32 SIMT kernel -- still on the device.
         // GridWorld-shaped tables (obs_size = N*N > 256, only rows i*N + {0,1,2,3} reachable): the pair kernel runs on
         // the compact 4N-row table when the twists (if any) keep the reachable rows among themselves
         if (e->precision != TWR_PREC_FP32 && d->obs_size > 256) {
@@ -465,7 +465,7 @@ int twr_policy_create(twr_engine* e, const twr_policy_desc* d_in, twr_policy** o
                 if ((i % d->obs_size) % N < 4 && d->obs_perms[i] % N >= 4) ok = false;
             if (ok) probe.tc_compact_n = p->dev.tc_compact_n = N;
         }
-        use_tc = e->precision != TWR_PREC_FP32 && forward_tc_supported(probe, dummy, &why);
+        use_tc = e->precision != TWR_PREC_FP32 && forward_tc2_supported(probe);
         // a compact-table policy still meets non-GridWorld callers (twr_policy_forward_obs): those run the fp32 kernel
         if ((!use_tc || p->dev.tc_compact_n > 0) && !forward_fp32_supported(probe, dummy, &why)) {
             if (!use_tc) {
@@ -494,13 +494,13 @@ int twr_policy_create(twr_engine* e, const twr_policy_desc* d_in, twr_policy** o
     }
     p->dev.obs_perms = p->d_obs_perms; p->dev.act_perms = p->d_act_perms;
     if (use_tc) {
-        const size_t bytes = forward_tc_pack_bytes(p->dev);
+        const size_t bytes = forward_tc2_pack_bytes(p->dev);
         cudaError_t ce = cudaMalloc(&p->tc_pack, bytes);
         if (ce != cudaSuccess) { twr_policy_destroy(p); return fail(TWR_ERR_CUDA, cudaGetErrorString(ce)); }
         p->dev.tc_pack = p->tc_pack;
     }
     if ((rc = upload_policy(p, d))) { twr_policy_destroy(p); return rc; }
-    if (use_tc && !forward_tc_prepare(p->dev)) {
+    if (use_tc && !forward_tc2_prepare(p->dev, p->tc_pack)) {
         twr_policy_destroy(p);
         return fail(TWR_ERR_CUDA, "tensor-core forward: cuTensorMapEncodeTiled / kernel attributes unavailable on this device or driver");
     }
@@ -538,7 +538,7 @@ int twr_policy_update_from_device(twr_policy* p, const float* d_src) {
     CU_TRY(cudaSetDevice(e->device));
     if (d_src != p->d_blob)
         CU_TRY(cudaMemcpyAsync(p->d_blob, d_src, sizeof(float) * (size_t)p->blob_floats, cudaMemcpyDeviceToDevice, e->stream));
-    if (p->tc_pack) launch_forward_tc_pack(e->stream, p->dev, p->tc_pack);
+    if (p->tc_pack) launch_forward_tc2_pack(e->stream, p->dev, p->tc_pack);
     CU_TRY(cudaGetLastError());
     return TWR_OK;
 }
@@ -548,7 +548,7 @@ void twr_policy_destroy(twr_policy* p) {
     cudaSetDevice(p->eng->device);
     cudaStreamSynchronize(p->eng->stream);
     dev_free(p->d_blob); dev_free(p->d_obs_perms); dev_free(p->d_act_perms);
-    if (p->tc_pack) { forward_tc_forget(p->dev); cudaFree(p->tc_pack); }
+    if (p->tc_pack) { forward_tc2_forget(p->tc_pack); cudaFree(p->tc_pack); }
     delete p;
 }
 
@@ -687,7 +687,7 @@ static void launch_forward(twr_engine* e, const PolicyDev& dev, const ForwardArg
         ForwardArgs t = a;
         t.tc_terms = e->tc_terms;
         t.dbg_flags |= e->tc_flags;
-        ok = launch_forward_tc(e->stream, dev, t);
+        ok = launch_forward_tc2(e->stream, dev, t, dev.tc_pack);
     } else ok = launch_forward_fp32(e->stream, dev, a);
     if (!ok) e->launch_error = true;
 }
@@ -957,7 +957,7 @@ static int enqueue_collect(twr_engine* e, const EnvParams& env, const PolicyDev&
     ForwardArgs fa{};
     fa.env = env; fa.seed = e->seed; fa.cid = cid; fa.ids = ids; fa.perm_idx = nullptr;
     fa.cells = b.cells; fa.n = B; fa.logits = b.logits; fa.values = b.values;
-    const bool fused = dev.tc_pack && forward_tc_can_fuse(dev);
+    const bool fused = dev.tc_pack != nullptr;            // the tensor-core kernel runs the collect step in its epilogue
     int n_fwd = *n_fwd_out;
     if (fused) {
         // Persistent chunks: one launch covers `chunk` consecutive steps of every tile (envs stay with their

@@ -11,7 +11,7 @@
 // are staged in shared memory with cp.async (double buffered), the h1 slice is produced by a
 // conflict-free shared-memory gather, and the 128 x H output tile lives in registers
 // (8 envs x H/16 columns per thread).  Bound: fp32 FMA pipe (2*E*H flop per env) -- this variant
-// exists for the 1e-5 parity bar; the tensor-core variant is twr_forward_tc.cu.
+// exists for the 1e-5 parity bar; the tensor-core variant is twr_forward_tc2.cu.
 #include "twr_kernels.cuh"
 
 #include <atomic>

@@ -1,7 +1,17 @@
-// twr_forward_tc2.cu -- K2, tensor-core variant with CTA pairs (tcgen05 cta_group::2).
+// twr_forward_tc2.cu -- K2, tensor-core variant for sm_100a: batched Policy::_raw_predict (rust/src/nn/policy.rs:79-100)
+// as two chained tcgen05 GEMMs, run by CTA pairs (tcgen05 cta_group::2).
 //
-// Same math and pipeline as twr_forward_tc.cu (one-hot GEMM1 -> TMEM -> bias/ReLU/fp16 split in place
-// -> GEMM2 with A from TMEM -> heads), but two CTAs of a cluster cooperate on a 256-env tile:
+//   GEMM1 (embedding, layers.rs:56-86):     D1 = onehot(obs)[256 x K1] * Emb[K1 x E]
+//   epilogue-1:                             h1 = relu(D1 + emb_bias) -> fp16 hi + lo, stored back into the same TMEM columns
+//   GEMM2 (common Linear, layers.rs:31-37): D2 = h1[256 x E] * W1[E x H]   (A operand read from TMEM)
+//   epilogue-2 (heads, policy.rs:89-97):    h2 = relu(D2 + b1); logits = Wa h2 + ba; value = wv.h2 + bv
+//
+// Every fp32 operand is split into two fp16 terms (x = hi + lo); which of the products are accumulated is the engine's
+// precision (TERMS below).  E runs in chunks of 128 features and GEMM1 over PAIRS of chunks: an embedding of an odd
+// number of chunks is zero-padded to the next pair in the operand image (zero table columns, bias and W1 rows), so the
+// padded features give h1 = 0 and add exact zeros to D2.
+//
+// Two CTAs of a cluster cooperate on a 256-env tile:
 // every tcgen05.mma is M=256 (rows 0..127 live in CTA 0's TMEM, 128..255 in CTA 1's) and the B operand
 // (weights) is split along N between the two CTAs' shared memory -- each SM therefore streams only
 // HALF of the operand bytes per env and issues M = 256 instructions (see DESIGN.md for what bounds it).
@@ -42,7 +52,6 @@ constexpr int TILE_BYTES = 16384;
 constexpr int NSLOTS = 8;
 constexpr int MAX_KB1 = 4;
 constexpr int MAX_OBS = 32;
-constexpr int NCOPIES = 1;              // replicas of the operand image (8 copies measured: no gain -- the bound is per-SM ingest, not L2 slices)
 
 constexpr int SM_A1 = 0;
 constexpr int SM_RING = SM_A1 + MAX_KB1 * TILE_BYTES;
@@ -126,6 +135,8 @@ __device__ __forceinline__ void tc2_mma_ts(uint32_t d_tmem, uint32_t a_tmem, uin
         "tcgen05.mma.cta_group::2.kind::f16 [%0], [%1], %2, %3, p;\n\t}"
         ::"r"(d_tmem), "r"(a_tmem), "l"(b_desc), "r"(idesc), "r"(accumulate) : "memory");
 }
+// instruction descriptor (cute::UMMA::InstrDescriptor): c=F32 [4,6)=1, a=b=F16 (0), K-major both,
+// N>>3 at [17,23), M>>4 at [24,29)
 constexpr uint32_t IDESC_256x128 = (1u << 4) | ((128u >> 3) << 17) | ((256u >> 4) << 24);
 constexpr uint32_t IDESC_256x256 = (1u << 4) | ((256u >> 3) << 17) | ((256u >> 4) << 24);
 // kind::f8f6f4 (K = 32 per instruction): operand formats at [7,10) (A) and [10,13) (B), 0 = e4m3, 1 = e5m2
@@ -208,7 +219,7 @@ __global__ void __launch_bounds__(256) k_tc2_pack(PolicyDev p, Tc2Params t, __ha
             const int f = kb == t.NKB1 - 1 ? (2 * sc + (int)(row >> 6)) * 128 + r * 64 + (int)(row & 63u) : (2 * sc + r) * 128 + (int)row;
             int k = kb * 64 + (int)kk;
             if (t.cN > 0) k = (k >> 2) < t.cN ? (k >> 2) * t.cN + (k & 3) : p.obs_size;
-            if (k < p.obs_size) x = p.emb[(size_t)k * p.E + f];
+            if (k < p.obs_size && f < p.E) x = p.emb[(size_t)k * p.E + f];
             off = tile_off(row, kk);
         } else if (t.H == 256) {
             const size_t q = slot - n1;
@@ -216,7 +227,7 @@ __global__ void __launch_bounds__(256) k_tc2_pack(PolicyDev p, Tc2Params t, __ha
             lo_part = (int)(q % 2);
             const uint32_t row = within >> 6, kk = within & 63u;
             const int o = r * 128 + (int)row, f = j * 128 + kb * 64 + (int)kk;
-            x = p.w1[(size_t)f * p.H + o];
+            if (f < p.E) x = p.w1[(size_t)f * p.H + o];
             off = tile_off(row, kk);
         } else {
             const size_t q = slot - n1;
@@ -225,13 +236,12 @@ __global__ void __launch_bounds__(256) k_tc2_pack(PolicyDev p, Tc2Params t, __ha
             const uint32_t row = within >> 6, kk = within & 63u;
             const int kb = (int)(row >> 6);
             const int o = r * 64 + (int)(row & 63u), f = j * 128 + kb * 64 + (int)kk;
-            x = p.w1[(size_t)f * p.H + o];
+            if (f < p.E) x = p.w1[(size_t)f * p.H + o];
             off = (uint32_t)kb * 8192u + tile_off(row & 63u, kk);
         }
         const __half hi = __float2half_rn(x);
         const __half v = lo_part ? __float2half_rn(x - __half2float(hi)) : hi;
-        for (int cp = 0; cp < NCOPIES; ++cp)
-            *reinterpret_cast<__half*>(reinterpret_cast<unsigned char*>(pack) + ((size_t)cp * 2 * spr + gslot) * TILE_BYTES + off) = v;
+        *reinterpret_cast<__half*>(reinterpret_cast<unsigned char*>(pack) + gslot * TILE_BYTES + off) = v;
     }
 }
 
@@ -244,6 +254,7 @@ __global__ void __launch_bounds__(256) k_tc2_pack8(PolicyDev p, Tc2Params t, uns
     const size_t spr = slots_per_rank(t), n1 = slots_g1(t);
     const size_t total = 2 * spr * TILE_BYTES;                 // one thread per BYTE position (fp16 slots: even positions only)
     const int upc = t.NKB1 + t.NKB8;
+    auto w1s = [&](int f, int o) { return f < p.E ? p.w1[(size_t)f * p.H + o] * W8_SCALE : 0.0f; };   // scaled W1, padding rows 0
     for (size_t idx = (size_t)blockIdx.x * blockDim.x + threadIdx.x; idx < total; idx += (size_t)gridDim.x * blockDim.x) {
         const size_t gslot = idx / TILE_BYTES;
         const uint32_t within = (uint32_t)(idx % TILE_BYTES);
@@ -261,7 +272,7 @@ __global__ void __launch_bounds__(256) k_tc2_pack8(PolicyDev p, Tc2Params t, uns
             int k = is8 ? kb * 128 + (int)kk : kb * 64 + (int)kk;
             if (t.cN > 0) k = (k >> 2) < t.cN ? (k >> 2) * t.cN + (k & 3) : p.obs_size;
             // PolicyDev::tc_fold: the embedding bias rides on the rows of block 0 (exactly one of them is in every observation)
-            const float x = k < p.obs_size ? (p.emb[(size_t)k * p.E + f] + (k < t.fold ? p.emb_b[f] : 0.0f)) * H1_SCALE8 : 0.0f;
+            const float x = k < p.obs_size && f < p.E ? (p.emb[(size_t)k * p.E + f] + (k < t.fold ? p.emb_b[f] : 0.0f)) * H1_SCALE8 : 0.0f;
             const __half hi = __float2half_rn(x);
             if (is8) dst[tile_off8(row, kk)] = (unsigned char)__nv_cvt_float_to_fp8((x - __half2float(hi)) * TABLE8_SCALE, __NV_SATFINITE, __NV_E4M3);
             else *reinterpret_cast<__half*>(dst + tile_off(row, kk)) = hi;
@@ -272,10 +283,10 @@ __global__ void __launch_bounds__(256) k_tc2_pack8(PolicyDev p, Tc2Params t, uns
             if (u < 2) {
                 if (within & 1u) continue;
                 const uint32_t kk = (within & 127u) >> 1;
-                *reinterpret_cast<__half*>(dst + tile_off(row, kk)) = __float2half_rn(p.w1[(size_t)(j * 128 + u * 64 + (int)kk) * p.H + o] * W8_SCALE);
+                *reinterpret_cast<__half*>(dst + tile_off(row, kk)) = __float2half_rn(w1s(j * 128 + u * 64 + (int)kk, o));
             } else {
                 const uint32_t kk = within & 127u;
-                dst[tile_off8(row, kk)] = (unsigned char)__nv_cvt_float_to_fp8(p.w1[(size_t)(j * 128 + (int)kk) * p.H + o] * W8_SCALE, __NV_SATFINITE, __NV_E5M2);
+                dst[tile_off8(row, kk)] = (unsigned char)__nv_cvt_float_to_fp8(w1s(j * 128 + (int)kk, o), __NV_SATFINITE, __NV_E5M2);
             }
         } else {
             const size_t q = slot - n1;
@@ -285,10 +296,10 @@ __global__ void __launch_bounds__(256) k_tc2_pack8(PolicyDev p, Tc2Params t, uns
                 const uint32_t kk = (within & 127u) >> 1;
                 const int kb = (int)(row >> 6);
                 const int o = r * 64 + (int)(row & 63u);
-                *reinterpret_cast<__half*>(dst + (uint32_t)kb * 8192u + tile_off(row & 63u, kk)) = __float2half_rn(p.w1[(size_t)(j * 128 + kb * 64 + (int)kk) * p.H + o] * W8_SCALE);
+                *reinterpret_cast<__half*>(dst + (uint32_t)kb * 8192u + tile_off(row & 63u, kk)) = __float2half_rn(w1s(j * 128 + kb * 64 + (int)kk, o));
             } else {
                 const uint32_t kk = within & 127u;
-                const float w = row < 64 ? p.w1[(size_t)(j * 128 + (int)kk) * p.H + (r * 64 + (int)row)] * W8_SCALE : 0.0f;
+                const float w = row < 64 ? w1s(j * 128 + (int)kk, r * 64 + (int)row) : 0.0f;
                 dst[tile_off8(row, kk)] = (unsigned char)__nv_cvt_float_to_fp8(w, __NV_SATFINITE, __NV_E5M2);
             }
         }
@@ -424,7 +435,10 @@ k_forward_tc2(PolicyDev p, ForwardArgs a, Tc2Params t, const __grid_constant__ C
         headw[4 * H + i] = p.wv[i];
         b1s[i] = p.b1[i];
     }
-    for (int i = threadIdx.x; i < t.E; i += NTHREADS) embb[i] = F8 ? p.emb_b[i] * H1_SCALE8 : p.emb_b[i];
+    // zero bias on the padding features; kept rolled, since the unrolled loop shifts ptxas' register allocation of the
+    // whole kernel (spills in k_forward_tc2<128, 19>)
+#pragma unroll 1
+    for (int i = threadIdx.x; i < t.NC * 128; i += NTHREADS) embb[i] = i >= t.E ? 0.0f : F8 ? p.emb_b[i] * H1_SCALE8 : p.emb_b[i];
     if (operm_smem)
         for (int i = threadIdx.x; i < p.n_perms * p.obs_size; i += NTHREADS) operm_s[i] = (uint8_t)p.obs_perms[i];
     // action twists next to the barriers (the heads look one row up per item)
@@ -453,7 +467,7 @@ k_forward_tc2(PolicyDev p, ForwardArgs a, Tc2Params t, const __grid_constant__ C
         // Each CTA fetches ITS half of every operand tile into its own ring; both halves credit the
         // leader's `full` barrier, so the MMA issuer waits on one local barrier per ring slot.
         if (lane == 0) {
-            const int img_row0 = t.row0 + ((pair_id % NCOPIES) * 2 + crank) * (int)slots_per_rank(t) * (TILE_BYTES / 128);   // tensor-map row of this pair's copy, this rank's image
+            const int img_row0 = t.row0 + crank * (int)slots_per_rank(t) * (TILE_BYTES / 128);   // tensor-map row of this rank's image
             const int g1_row0 = img_row0, g2_row0 = img_row0 + (int)slots_g1(t) * (TILE_BYTES / 128);
             uint32_t use = 0;
             long long w_empty = 0;
@@ -1100,12 +1114,12 @@ k_forward_tc2(PolicyDev p, ForwardArgs a, Tc2Params t, const __grid_constant__ C
 
 Tc2Params make_params2(const PolicyDev& p, bool f8 = false) {
     Tc2Params t;
-    t.E = p.E; t.H = p.H; t.NC = p.E / 128; t.cN = p.tc_compact_n;
+    t.E = p.E; t.H = p.H; t.NC = 2 * ((p.E + 255) / 256); t.cN = p.tc_compact_n;   // E % 256 == 128: zero-padded to a chunk pair
     t.NKB1 = ((p.tc_compact_n > 0 ? 4 * p.tc_compact_n : p.obs_size) + 63) / 64;
     t.NKB8 = (t.NKB1 + 1) / 2;
     t.f8 = 0; t.row0 = 0; t.fold = 0;
     if (f8) {                                   // the fp8-correction image follows the standard one; it carries the folded bias
-        t.row0 = (int)((size_t)NCOPIES * 2 * slots_per_rank(t) * (TILE_BYTES / 128));
+        t.row0 = (int)(2 * slots_per_rank(t) * (TILE_BYTES / 128));
         t.f8 = 1;
         t.fold = p.tc_fold;
     }
@@ -1160,24 +1174,23 @@ bool get_tmap(DevState& d, const void* pack, size_t bytes, CUtensorMap* out) {
 
 }  // namespace
 
-// GEMM1 works on chunk pairs (E % 256), the one-hot operand holds <= 256 (compact) rows, GEMM2 is N = H in {128, 256}
+// E in 128-feature chunks (an odd count is padded to a pair), the one-hot operand holds <= 256 (compact) rows, GEMM2 is
+// N = H in {128, 256}
 int forward_tc2_supported(const PolicyDev& p) {
     const int k1 = p.tc_compact_n > 0 ? 4 * p.tc_compact_n : p.obs_size;
-    return (p.H == 256 || p.H == 128) && p.E % 256 == 0 && p.E <= 1024 && k1 <= 64 * MAX_KB1;
+    return (p.H == 256 || p.H == 128) && p.E % 128 == 0 && p.E <= 1024 && k1 <= 64 * MAX_KB1;
 }
 
 size_t forward_tc2_pack_bytes(const PolicyDev& p) {
     if (!forward_tc2_supported(p)) return 0;
-    return (size_t)NCOPIES * 2 * (slots_per_rank(make_params2(p)) + slots_per_rank(make_params2(p, true))) * TILE_BYTES;
+    return 2 * (slots_per_rank(make_params2(p)) + slots_per_rank(make_params2(p, true))) * TILE_BYTES;
 }
 
 void launch_forward_tc2_pack(cudaStream_t st, const PolicyDev& p, void* pack) {
     k_tc2_pack<<<1024, 256, 0, st>>>(p, make_params2(p), reinterpret_cast<__half*>(pack));
     const Tc2Params t8 = make_params2(p, true);
-    unsigned char* img8 = reinterpret_cast<unsigned char*>(pack) + (size_t)t8.row0 * 128;
-    for (int cp = 0; cp < NCOPIES; ++cp)
-        k_tc2_pack8<<<1024, 256, 0, st>>>(p, t8, img8 + (size_t)cp * 2 * slots_per_rank(t8) * TILE_BYTES);
-    g_twr_launches.fetch_add(1 + NCOPIES, std::memory_order_relaxed);
+    k_tc2_pack8<<<1024, 256, 0, st>>>(p, t8, reinterpret_cast<unsigned char*>(pack) + (size_t)t8.row0 * 128);
+    g_twr_launches.fetch_add(2, std::memory_order_relaxed);
 }
 
 // Everything a launch needs besides the arguments, resolved once (at policy creation) so that a launch cannot fail for

@@ -17,7 +17,8 @@ struct PolicyDev {
     const float* bv;      // [1]
     const int32_t* obs_perms;  // [n_perms][obs_size]
     const int32_t* act_perms;  // [n_perms][A]
-    // tensor-core operands (fp16 hi/lo split, UMMA canonical K-major tiles), see twr_forward_tc.cu
+    // operand image of the tensor-core kernel (fp16 hi/lo split and fp8 corrections, pre-swizzled K-major tiles in
+    // streaming order), see k_tc2_pack in twr_forward_tc2.cu; NULL: the policy runs another kernel
     const void* tc_pack;
     // > 0: the pair kernel's GEMM1 image holds only the 4 * tc_compact_n reachable rows of a GridWorld table
     // (row (i, v) = i * tc_compact_n + v, v in 0..3; examples/grid_world/src/lib.rs:74-81,161-163); such a policy takes
@@ -127,26 +128,19 @@ struct ForwardArgs {
     // | bit 1 h1_lo x W_hi | bit 2 h1_hi x W_lo on top of the hi x hi products (TWR_PREC_F16X2_W16 = 8 | 1 | 2)
     int tc_terms;
     int dbg_flags;    // ablations (k_forward_tc2, timing only): 1 skip epilogue-1 TMEM traffic, 2 no operand TMA traffic, 4 skip GEMM2 MMAs, 8 skip GEMM1 MMAs
-    long long* dbg;   // optional [gridDim][16] cycle counters written by k_forward_tc (debug/profiling)
+    long long* dbg;   // optional [gridDim][16] cycle counters written by k_forward_tc2 (debug/profiling)
 };
 int  forward_fp32_supported(const PolicyDev& p, const EnvParams& env, const char** why);
 bool launch_forward_fp32(cudaStream_t s, const PolicyDev& p, const ForwardArgs& a);   // false: shape does not fit shared memory
-int  forward_tc_supported(const PolicyDev& p, const EnvParams& env, const char** why);
-// builds / refreshes the packed fp16 hi/lo operand tiles from the fp32 blob
-size_t forward_tc_pack_bytes(const PolicyDev& p);
-void launch_forward_tc_pack(cudaStream_t s, const PolicyDev& p, void* pack);
-bool launch_forward_tc(cudaStream_t s, const PolicyDev& p, const ForwardArgs& a);   // false: the launch could not be made (see forward_tc_prepare)
-// resolves, at policy creation, everything a later launch depends on (tensor map of the operand image, kernel attributes)
-bool forward_tc_prepare(const PolicyDev& p);
-void forward_tc_forget(const PolicyDev& p);    // before the operand image is freed
-// CTA-pair (cta_group::2) variant, twr_forward_tc2.cu; `pack` is its own operand image
+// Tensor-core (CTA-pair, tcgen05 cta_group::2) variant, twr_forward_tc2.cu; `pack` is its operand image (PolicyDev::tc_pack)
 int    forward_tc2_supported(const PolicyDev& p);
+// builds / refreshes the packed operand tiles from the fp32 blob
 size_t forward_tc2_pack_bytes(const PolicyDev& p);
 void   launch_forward_tc2_pack(cudaStream_t s, const PolicyDev& p, void* pack);
-int    forward_tc_can_fuse(const PolicyDev& p);   // 1 when launch_forward_tc will run the fusable pair kernel
 bool   launch_forward_tc2(cudaStream_t s, const PolicyDev& p, const ForwardArgs& a, const void* pack);  // false: forward_tc2_prepare missing / failed
+// resolves, at policy creation, everything a later launch depends on (tensor map of the operand image, kernel attributes)
 bool   forward_tc2_prepare(const PolicyDev& p, const void* pack);
-void   forward_tc2_forget(const void* pack);
+void   forward_tc2_forget(const void* pack);    // before the operand image is freed
 
 // f1: batched single_solve step (rust/src/rl/solve.rs:17-71) for every live env
 struct SolveArgs {

@@ -1,5 +1,5 @@
-// twr_tc_ptx.cuh -- inline-PTX wrappers shared by the tensor-core kernels: mbarrier, cp.async.bulk (TMA),
-// tcgen05 (mma / commit / ld / st / fences), UMMA shared-memory and instruction descriptors.
+// twr_tc_ptx.cuh -- inline-PTX wrappers of the tensor-core kernel (twr_forward_tc2.cu) and scripts/mma_rate.cu:
+// mbarrier, cluster barrier, tcgen05 ld / st / fences, the UMMA shared-memory descriptor and the tile layout.
 #pragma once
 #include <cstdint>
 #include <cuda_runtime.h>
@@ -37,14 +37,6 @@ __device__ __forceinline__ void mbar_wait_t(uint32_t bar, uint32_t parity, long 
     mbar_wait(bar, parity);
     acc += clock64() - t0;
 }
-__device__ __forceinline__ void bulk_g2s(uint32_t dst, const void* src, uint32_t bytes, uint32_t bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                 ::"r"(dst), "l"(src), "r"(bytes), "r"(bar) : "memory");
-}
-__device__ __forceinline__ void bulk_g2s_mc(uint32_t dst, const void* src, uint32_t bytes, uint32_t bar, uint16_t mask) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1], %2, [%3], %4;"
-                 ::"r"(dst), "l"(src), "r"(bytes), "r"(bar), "h"(mask) : "memory");
-}
 __device__ __forceinline__ uint32_t cluster_ctarank() { uint32_t r; asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r)); return r; }
 __device__ __forceinline__ void cluster_sync_all() {
     asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
@@ -54,30 +46,6 @@ __device__ __forceinline__ void fence_async_smem() { asm volatile("fence.proxy.a
 __device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
 
-__device__ __forceinline__ void tc_commit(uint32_t bar) {   // arrives on `bar` when all prior MMAs of this thread finish
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
-}
-// same, arriving on the barrier at this offset in every CTA of `mask` (ring slots are shared by the cluster)
-__device__ __forceinline__ void tc_commit_mc(uint32_t bar, uint16_t mask) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-                 ::"r"(bar), "h"(mask) : "memory");
-}
-// D[tmem] (+)= A[smem] * B[smem]^T ; M=128, N=128, K=16, fp16 in, fp32 accumulate
-__device__ __forceinline__ void tc_mma(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc, uint32_t accumulate) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-        ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate) : "memory");
-}
-// same with the A operand read from TMEM (lane = row, 16-bit elements packed two per 32-bit column)
-__device__ __forceinline__ void tc_mma_ts(uint32_t d_tmem, uint32_t a_tmem, uint64_t b_desc, uint32_t idesc, uint32_t accumulate) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, p;\n\t}"
-        ::"r"(d_tmem), "r"(a_tmem), "l"(b_desc), "r"(idesc), "r"(accumulate) : "memory");
-}
 __device__ __forceinline__ void tc_st32(uint32_t taddr, const uint32_t (&v)[32]) {
     asm volatile(
         "tcgen05.st.sync.aligned.32x32b.x32.b32 [%0], "
@@ -107,9 +75,6 @@ __device__ __forceinline__ void tc_wait_ld() { asm volatile("tcgen05.wait::ld.sy
 __device__ __forceinline__ uint64_t make_desc(uint32_t saddr) {
     return (uint64_t)((saddr >> 4) & 0x3FFFu) | (1ull << 16) | (64ull << 32) | (1ull << 46) | (2ull << 61);
 }
-// instruction descriptor (cute::UMMA::InstrDescriptor): c=F32 [4,6)=1, a=b=F16 (0), K-major both,
-// N>>3 at [17,23), M>>4 at [24,29)
-constexpr uint32_t IDESC_128x128 = (1u << 4) | ((128u >> 3) << 17) | ((128u >> 4) << 24);
 
 // byte offset of element (row, k) inside one [128 x 64] fp16 tile, K-major with 128B swizzle
 __host__ __device__ __forceinline__ uint32_t tile_off(uint32_t row, uint32_t k) {
