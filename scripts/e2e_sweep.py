@@ -47,15 +47,13 @@ R1 = 18944
 cands = [None, "37888,27648", "18944,27648,18944", "18944,18944,27648", "27648,18944,18944", "18944,18944,18944,8704", "9472,28416,27648",
          "18944,37888,8704", "14208,23680,27648", "18944,23296,23296"]
 for parts in cands:
-    for nopack in ((False, True) if parts in (None, "37888,27648") else (False,)):
-        os.environ.pop("TWISTERL_B200_E2E_PARTS", None); os.environ.pop("TWISTERL_B200_E2E_NOPACK", None)
-        if parts: os.environ["TWISTERL_B200_E2E_PARTS"] = parts
-        if nopack: os.environ["TWISTERL_B200_E2E_NOPACK"] = "1"
-        for _ in range(2):
-            _lib.check(L.twr_ppo_collect_host(eng._h, C.byref(spec), hpol, C.byref(desc), E, 0.995, 0.995, C.byref(hb), C.byref(out)))
-        t0 = time.perf_counter(); n = 0
-        for _ in range(6):
-            _lib.check(L.twr_ppo_collect_host(eng._h, C.byref(spec), hpol, C.byref(desc), E, 0.995, 0.995, C.byref(hb), C.byref(out)))
-            n += int(out.n_records)
-        dt = time.perf_counter() - t0
-        print(f"parts={parts or 'default':28s} nopack={int(nopack)}  {n / dt:.4g} env-steps/s  {1e3 * dt / 6:.2f} ms/call", flush=True)
+    os.environ.pop("TWISTERL_B200_E2E_PARTS", None)
+    if parts: os.environ["TWISTERL_B200_E2E_PARTS"] = parts
+    for _ in range(2):
+        _lib.check(L.twr_ppo_collect_host(eng._h, C.byref(spec), hpol, C.byref(desc), E, 0.995, 0.995, C.byref(hb), C.byref(out)))
+    t0 = time.perf_counter(); n = 0
+    for _ in range(6):
+        _lib.check(L.twr_ppo_collect_host(eng._h, C.byref(spec), hpol, C.byref(desc), E, 0.995, 0.995, C.byref(hb), C.byref(out)))
+        n += int(out.n_records)
+    dt = time.perf_counter() - t0
+    print(f"parts={parts or 'default':28s}  {n / dt:.4g} env-steps/s  {1e3 * dt / 6:.2f} ms/call", flush=True)

@@ -1,5 +1,5 @@
 """Host-collect timeline (TWISTERL_B200_E2E_TRACE) of the benchmark workload for the environment's current settings.
-usage: e2e_trace.py [precision] ; knobs: TWISTERL_B200_E2E_PARTS / _NIB / _NOPACK / _THREADS"""
+usage: e2e_trace.py [precision] ; knob: TWISTERL_B200_E2E_PARTS"""
 import ctypes as C, os, sys, time
 from pathlib import Path
 sys.path.insert(0, str(Path(__file__).resolve().parents[1]))
@@ -22,7 +22,7 @@ t0 = time.perf_counter()
 for _ in range(5):
     _lib.check(L.twr_ppo_collect_host(eng._h, C.byref(spec), hpol, C.byref(desc), E, 0.995, 0.995, C.byref(hb), C.byref(out)))
 dt = (time.perf_counter() - t0) / 5
-print(f"{dt * 1e3:.2f} ms per call, {out.n_records / dt:.4g} env-steps/s  (NIB={os.environ.get('TWISTERL_B200_E2E_NIB')}, THREADS={os.environ.get('TWISTERL_B200_E2E_THREADS')}, cpus={os.cpu_count()})", flush=True)
+print(f"{dt * 1e3:.2f} ms per call, {out.n_records / dt:.4g} env-steps/s  (PARTS={os.environ.get('TWISTERL_B200_E2E_PARTS')}, cpus={os.cpu_count()})", flush=True)
 os.environ["TWISTERL_B200_E2E_TRACE"] = "1"
 _lib.check(L.twr_ppo_collect_host(eng._h, C.byref(spec), hpol, C.byref(desc), E, 0.995, 0.995, C.byref(hb), C.byref(out)))
 keep = None

@@ -471,18 +471,9 @@ def test_collect_host_pipelined_matches_plain(eng, monkeypatch, twists):
     L = _lib.load()
     spec = tw.env.spec_from_env(env)
     cap = int(L.twr_max_records(C.byref(spec), E))
-    # nib: the observations cross PCIe as 8 bytes of tile nibbles that host threads expand (opt-in wire format)
-    for split, parts, u8, nib in (("3", None, False, False), ("7", None, True, False), ("1", None, True, False),
-                                  (None, "600,300,100", True, False), ("3", None, True, True), ("2", None, False, True)):
-        monkeypatch.delenv("TWISTERL_B200_E2E_SPLIT", raising=False)
-        monkeypatch.delenv("TWISTERL_B200_E2E_PARTS", raising=False)
-        monkeypatch.delenv("TWISTERL_B200_E2E_NIB", raising=False)
-        if nib:
-            monkeypatch.setenv("TWISTERL_B200_E2E_NIB", "1")
-        if split:
-            monkeypatch.setenv("TWISTERL_B200_E2E_SPLIT", split)
-        if parts:
-            monkeypatch.setenv("TWISTERL_B200_E2E_PARTS", parts)     # unequal sub-batches
+    # "1000" with u8 still runs the pipelined body (one sub-batch); the last split is unequal
+    for parts, u8 in (("334,333,333", False), ("143,143,143,143,143,143,142", True), ("1000", True), ("600,300,100", True)):
+        monkeypatch.setenv("TWISTERL_B200_E2E_PARTS", parts)
         hb, arr, _ = twc._host_buffers(cap, 16, 4, E, pinned=True, obs_u8=u8)   # u8: one-byte observation indices
         out = _lib.Collected()
         eng.set_collect_id(21)
@@ -502,28 +493,28 @@ def test_collect_host_pipelined_matches_plain(eng, monkeypatch, twists):
 
 
 @pytest.mark.parametrize("E,difficulty", [(5000, 40), (33, 3), (20000, 128)])
-def test_collect_fused_gae_matches_stand_alone_kernels(eng, monkeypatch, E, difficulty):
+def test_collect_fused_gae_matches_twr_gae(eng, E, difficulty):
     """The PPO collect computes advantages and returns inside the compaction pass (k_compact<true>: reverse walk over the
-    time tiles, collector/ppo.rs:82-92 per episode); TWISTERL_B200_SPLIT_GAE=1 runs the stand-alone GAE kernel and the
-    plain compaction instead.  Every array must be identical, bit for bit (both are held to the oracle by the replays)."""
+    time tiles, collector/ppo.rs:82-92 per episode).  twr_gae, the stand-alone GAE held to the oracle by
+    test_gae_matches_oracle, run on the same collect's rewards and values must give the same arrays, bit for bit."""
     import twisterl_b200 as tw
     from parity import make_policies
+    from twisterl_b200 import _lib
     pol, _ = make_policies(synth_state_dict(5, 256, 512, 256, 4), 256)
     env = tw.env.Puzzle(4, 4, difficulty, 2, 256)
     col = tw.collector.PPOCollector(E, 0.97, 0.9, 32, engine=eng)
-    out = []
-    for split in (False, True):
-        monkeypatch.delenv("TWISTERL_B200_SPLIT_GAE", raising=False)
-        if split:
-            monkeypatch.setenv("TWISTERL_B200_SPLIT_GAE", "1")
-        eng.set_collect_id(4)
-        out.append(col.collect(env, pol))
-    a, b = out
-    assert len(a.values_array) == len(b.values_array) and len(a.values_array) > E
-    for f in ("obs_array", "logits_array", "values_array", "rewards_array", "actions_array", "perms_array", "ep_len"):
-        assert np.array_equal(getattr(a, f), getattr(b, f)), f
-    for k in ("advs", "rets"):
-        assert np.array_equal(a.additional_array(k), b.additional_array(k)), k
+    eng.set_collect_id(4)
+    d = col.collect(env, pol)
+    r, v = np.ascontiguousarray(d.rewards_array, np.float32), np.ascontiguousarray(d.values_array, np.float32)
+    R = len(v)
+    assert R > E
+    L = d.ep_len.astype(np.int64)[orc.merge_order(E)]
+    off = np.concatenate([[0], np.cumsum(L)]).astype(np.int64)
+    assert off[-1] == R
+    adv = np.zeros(R, np.float32); ret = np.zeros(R, np.float32)
+    _lib.check(_lib.load().twr_gae(eng._h, _lib.ptr(r), _lib.ptr(v), _lib.ptr(off), E, 0.97, 0.9, _lib.ptr(adv), _lib.ptr(ret)))
+    assert np.array_equal(d.additional_array("advs"), adv)
+    assert np.array_equal(d.additional_array("rets"), ret)
     pol.release()
 
 

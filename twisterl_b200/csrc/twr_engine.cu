@@ -2,9 +2,6 @@
 // validates env specs / policy shapes, drives the per-step kernel sequence of a collect on one CUDA
 // stream, and moves results to caller buffers.  No CPU compute path exists here: every Env / Policy /
 // collector operation is a kernel launch (twr_kernels.cu, twr_forward_*.cu).
-#if defined(__SSE2__)
-#include <emmintrin.h>
-#endif
 #include "../../include/twisterl_b200.h"
 #include "twr_kernels.cuh"
 
@@ -191,7 +188,6 @@ int twr_engine_create(const twr_engine_cfg* cfg, twr_engine** out) {
     for (int i = 0; i < TWR_MAX_SUBBATCH && ce2 == cudaSuccess; ++i) {
         ce2 = cudaEventCreate(&e->ev_copied[i]);   // timing on: TWISTERL_B200_E2E_TRACE
         if (ce2 == cudaSuccess) ce2 = cudaEventCreateWithFlags(&e->ev_small[i], cudaEventDisableTiming);
-        if (ce2 == cudaSuccess) ce2 = cudaEventCreateWithFlags(&e->ev_obs[i], cudaEventDisableTiming);
     }
     // collect statistics come back through MAPPED pinned memory written by a one-thread kernel, not through a D2H copy:
     // a 32-byte cudaMemcpyAsync queues on the copy engine behind the bulk D2H of the previous sub-batch (measured: the
@@ -238,12 +234,10 @@ void twr_engine_destroy(twr_engine* e) {
     for (int i = 0; i < TWR_MAX_SUBBATCH; ++i) {
         if (e->ev_copied[i]) cudaEventDestroy(e->ev_copied[i]);
         if (e->ev_small[i]) cudaEventDestroy(e->ev_small[i]);
-        if (e->ev_obs[i]) cudaEventDestroy(e->ev_obs[i]);
     }
     if (e->copy_stream) cudaStreamDestroy(e->copy_stream);
     if (e->bal_flags) cudaFree(e->bal_flags);
     if (e->h_stats) cudaFreeHost(e->h_stats);
-    if (e->h_obs_nib) cudaFreeHost(e->h_obs_nib);
     if (e->ev_t0) cudaEventDestroy(e->ev_t0);
     if (e->ev_t1) cudaEventDestroy(e->ev_t1);
     if (e->own_stream) cudaStreamDestroy(e->stream);
@@ -1044,14 +1038,11 @@ static int enqueue_collect(twr_engine* e, const EnvParams& env, const PolicyDev&
         }
     }
     *n_fwd_out = n_fwd;
-    // GAE rides on the compaction (one pass over the records); TWISTERL_B200_SPLIT_GAE=1 keeps the two stand-alone kernels
-    const bool split_gae = getenv("TWISTERL_B200_SPLIT_GAE") != nullptr;
-    if (split_gae) launch_gae_time_major(st, b, gamma, lambda);
     launch_episode_offsets(st, b, ids);
     // only the compaction writes the output set: a pipelined caller's "its previous copy is done" event is awaited here,
     // not in front of the rollout
     if (outset_free) CU_TRY(cudaStreamWaitEvent(st, outset_free, 0));
-    if (split_gae) launch_compact(st, env, b, dev.A); else launch_compact_gae(st, env, b, dev.A, gamma, lambda);
+    launch_compact_gae(st, env, b, dev.A, gamma, lambda);      // GAE rides on the compaction (one pass over the records)
     CU_TRY(cudaGetLastError());
     FWD_CHECK(e);
     return TWR_OK;
@@ -1183,31 +1174,6 @@ static void expand_packed(uint8_t* __restrict__ actions, int8_t* __restrict__ pe
     }
 }
 
-// Host side of CollectBuffers::obs_u8 == 2 for records [a, b): 8 bytes of tile nibbles -> the 16 one-hot indices
-// i * 16 + tile(i) the reference returns from Env::observe (puzzle.rs observe()), as bytes or as u16.
-static void expand_nibbles(const unsigned char* __restrict__ nib, uint8_t* __restrict__ obs8, uint16_t* __restrict__ obs16, int64_t a, int64_t b) {
-#if defined(__SSE2__)
-    const __m128i m = _mm_set1_epi8(0x0F), zero = _mm_setzero_si128();
-    const __m128i base = _mm_setr_epi8(0, 16, 32, 48, 64, 80, 96, 112, (char)128, (char)144, (char)160, (char)176, (char)192, (char)208, (char)224, (char)240);
-    for (int64_t r = a; r < b; ++r) {
-        const __m128i x = _mm_loadl_epi64(reinterpret_cast<const __m128i*>(nib + r * 8));
-        const __m128i lo = _mm_and_si128(x, m), hi = _mm_and_si128(_mm_srli_epi16(x, 4), m);
-        const __m128i idx = _mm_add_epi8(_mm_unpacklo_epi8(lo, hi), base);
-        if (obs8) _mm_storeu_si128(reinterpret_cast<__m128i*>(obs8 + r * 16), idx);
-        else {
-            _mm_storeu_si128(reinterpret_cast<__m128i*>(obs16 + r * 16), _mm_unpacklo_epi8(idx, zero));
-            _mm_storeu_si128(reinterpret_cast<__m128i*>(obs16 + r * 16 + 8), _mm_unpackhi_epi8(idx, zero));
-        }
-    }
-#else
-    for (int64_t r = a; r < b; ++r)
-        for (int i = 0; i < 16; ++i) {
-            const unsigned v = (nib[r * 8 + (i >> 1)] >> ((i & 1) * 4)) & 15u;
-            if (obs8) obs8[r * 16 + i] = (uint8_t)(i * 16 + v); else obs16[r * 16 + i] = (uint16_t)(i * 16 + v);
-        }
-#endif
-}
-
 static std::vector<int64_t> host_collect_parts(twr_engine* e, int64_t num_episodes) {
     std::vector<int64_t> parts;
     if (const char* ps = getenv("TWISTERL_B200_E2E_PARTS")) {         // explicit sizes "a,b,c" (must sum to num_episodes)
@@ -1219,15 +1185,6 @@ static std::vector<int64_t> host_collect_parts(twr_engine* e, int64_t num_episod
     int sms = 0;
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, e->device);
     const int64_t round = (int64_t)(sms / 2) * 256;      // envs the pair kernel works on at once
-    if (const char* sp = getenv("TWISTERL_B200_E2E_SPLIT")) {          // equal split into this many sub-batches
-        int split = atoi(sp);
-        if (split < 1) split = 1;
-        if (split > 64) split = 64;
-        if (split > num_episodes) split = (int)num_episodes;
-        const int64_t Bsub = (num_episodes + split - 1) / split;
-        for (int64_t lo = 0; lo < num_episodes; lo += Bsub) parts.push_back(lo + Bsub <= num_episodes ? Bsub : num_episodes - lo);
-        return parts;
-    }
     if (num_episodes < 32768 || e->precision == TWR_PREC_FP32 || round <= 0) { parts.push_back(num_episodes); return parts; }
     // Sub-batches of two kernel rounds -- the smallest shape the pair kernel runs at full rate (one round is a serial
     // chain of one tile per SM pair: 18 944 envs take 4.9 ms, 37 888 take 6.9 ms) -- and the remainder last, whose copy is
@@ -1259,21 +1216,8 @@ int twr_ppo_collect_host(twr_engine* e, const twr_env_spec* spec, twr_policy* p,
     for (int64_t v : parts) Bmax = v > Bmax ? v : Bmax;
     if ((rc = ensure_collect_buffers(e, Bmax, plan.T, plan.env.N, num_episodes))) return rc;
     // one byte for action / reward / twist when they fit: Puzzle rewards (three values) and at most 14 twists
-    const bool pack = plan.env.kind == TWR_ENV_PUZZLE && plan.dev.n_perms <= 14 && dst->actions && (!dst->advs || (dst->rets && dst->values)) &&
-                      !getenv("TWISTERL_B200_E2E_NOPACK");
+    const bool pack = plan.env.kind == TWR_ENV_PUZZLE && plan.dev.n_perms <= 14 && dst->actions && (!dst->advs || (dst->rets && dst->values));
     const float reward_of_code[4] = {-0.5f / (float)plan.env.max_depth, -0.5f, 1.0f, 0.0f};     // puzzle.rs:171-177
-    // 16-cell puzzles, opt-in (TWISTERL_B200_E2E_NIB=1): the observation crosses PCIe as 8 bytes of tile nibbles instead of
-    // 16 index bytes (the indices are i * 16 + tile(i)) and host threads expand them while the logits of the same
-    // sub-batch are still in flight.  33 instead of 41 B/record on the wire, but the expansion writes 16 B/record from
-    // the CPU: on the 16-vCPU benchmark hosts that costs more than the 2.4 ms of PCIe time it saves (measured: 22.9 vs
-    // 20.2 ms per 65 536-env call, DESIGN.md), so it is for hosts with cores to spare.
-    const char* nib_env = getenv("TWISTERL_B200_E2E_NIB");
-    const bool nib = pack && plan.env.N == 16 && (dst->obs || dst->obs_u8) && nib_env && atoi(nib_env) > 0;
-    if (nib && e->h_obs_nib_bytes < (size_t)dst->capacity * 8) {
-        if (e->h_obs_nib) { cudaFreeHost(e->h_obs_nib); e->h_obs_nib = nullptr; e->h_obs_nib_bytes = 0; }
-        CU_TRY(cudaHostAlloc(reinterpret_cast<void**>(&e->h_obs_nib), (size_t)dst->capacity * 8, cudaHostAllocDefault));
-        e->h_obs_nib_bytes = (size_t)dst->capacity * 8;
-    }
     e->has_last = false;
     const uint32_t cid = e->collect_id++;
     const uint32_t base = (uint32_t)((int64_t)e->rank * num_episodes);
@@ -1282,7 +1226,7 @@ int twr_ppo_collect_host(twr_engine* e, const twr_env_spec* spec, twr_policy* p,
     int n_fwd = 0;
     const bool timing = e->timing;
     e->timing = false;                                  // per-forward events are only kept for the device-resident path
-    e->buf.obs_u8 = nib ? 2 : u8 ? 1 : 0;
+    e->buf.obs_u8 = u8 ? 1 : 0;
     e->buf.pack_misc = pack ? 1 : 0;
     std::vector<std::thread> stages;                    // one per sub-batch: waits for its copy, then rebuilds the packed fields
     std::vector<std::function<void()>> deferred;        // stages whose thread could not be started: run on this thread at the end
@@ -1294,7 +1238,6 @@ int twr_ppo_collect_host(twr_engine* e, const twr_env_spec* spec, twr_policy* p,
     std::vector<size_t> tr_R;
     int hw = (int)std::thread::hardware_concurrency();
     int workers = hw / (2 * (e->world > 0 ? e->world : 1));
-    if (const char* w = getenv("TWISTERL_B200_E2E_THREADS")) workers = atoi(w);
     workers = workers < 1 ? 1 : (workers > 16 ? 16 : workers);
     auto body = [&]() -> int {
         for (size_t k = 0; k < parts.size(); ++k) {
@@ -1325,20 +1268,12 @@ int twr_ppo_collect_host(twr_engine* e, const twr_env_spec* spec, twr_policy* p,
                 if ((r2 = copy_out(e, e->copy_stream, &d2, at, R, plan.env.N, plan.dev.A))) return r2;
                 CU_TRY(cudaEventRecord(e->ev_small[k], e->copy_stream));
                 twr_host_buffers d3{};
-                d3.logits = dst->logits;
-                if (nib) {
-                    CU_TRY(cudaMemcpyAsync(e->h_obs_nib + (size_t)at * 8, e->buf.out_obs, R * 8, cudaMemcpyDeviceToHost, e->copy_stream));
-                    CU_TRY(cudaEventRecord(e->ev_obs[k], e->copy_stream));
-                } else {
-                    d3.obs = dst->obs; d3.obs_u8 = dst->obs_u8;
-                }
+                d3.logits = dst->logits; d3.obs = dst->obs; d3.obs_u8 = dst->obs_u8;
                 if ((r2 = copy_out(e, e->copy_stream, &d3, at, R, plan.env.N, plan.dev.A))) return r2;
             } else if ((r2 = copy_out(e, e->copy_stream, dst, at, R, plan.env.N, plan.dev.A))) return r2;
             CU_TRY(cudaEventRecord(e->ev_copied[k], e->copy_stream));
             if (pack) {
                 cudaEvent_t ev = e->ev_small[k];
-                cudaEvent_t ev_o = nib ? e->ev_obs[k] : nullptr;
-                const unsigned char* h_nib = e->h_obs_nib;
                 const int dev_id = e->device;
                 const int64_t at0 = at;
                 const twr_host_buffers d = *dst;
@@ -1346,17 +1281,10 @@ int twr_ppo_collect_host(twr_engine* e, const twr_env_spec* spec, twr_policy* p,
                 double* t_exp = trace ? &tr_exp[k] : nullptr;
                 // the rebuild of one sub-batch; a thread that cannot be started (resource limits) is run inline instead --
                 // no C++ exception may leave through the C boundary
-                auto stage = [ev, ev_o, h_nib, dev_id, at0, R, d, rtab, workers, t_exp, t_call]() {
+                auto stage = [ev, dev_id, at0, R, d, rtab, workers, t_exp, t_call]() {
                     cudaSetDevice(dev_id);
                     cudaEventSynchronize(ev);
-                    auto span = [&](int64_t a, int64_t b) {
-                        expand_packed(d.actions, d.perms, d.rewards, d.advs, d.rets, d.values, rtab[0], a, b);
-                        if (ev_o) {                                // the nibbles of this sub-batch land right after the small arrays
-                            cudaSetDevice(dev_id);
-                            cudaEventSynchronize(ev_o);
-                            expand_nibbles(h_nib, d.obs ? nullptr : d.obs_u8, d.obs, a, b);
-                        }
-                    };
+                    auto span = [&](int64_t a, int64_t b) { expand_packed(d.actions, d.perms, d.rewards, d.advs, d.rets, d.values, rtab[0], a, b); };
                     std::vector<std::thread> ws;
                     const int64_t per = ((int64_t)R + workers - 1) / workers;
                     for (int w = 1; w < workers; ++w) {

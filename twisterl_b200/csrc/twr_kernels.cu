@@ -233,39 +233,6 @@ __device__ __forceinline__ void gae_step(float r, float v, float v_next, float a
     adv = __fsub_rn(ret, v);
 }
 
-// One thread per env, reverse scan over its time-major records.  The loads of 8 steps are issued before the
-// (serial) recursion runs over them, so each warp keeps 16 independent 128-byte requests in flight.
-__global__ void __launch_bounds__(64) k_gae_time_major(CollectBuffers b, float gamma, float lambda) {
-    const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (e >= b.B) return;
-    const int n = b.ep_len[e];
-    if (n <= 0) return;
-    constexpr int U = 8;
-    float adv = 0.f, ret = 0.f, v_next = 0.f;
-    for (int t1 = n - 1; t1 >= 0; t1 -= U) {          // block of steps t1, t1-1, .., t1-U+1
-        float rw[U], vl[U];
-#pragma unroll
-        for (int j = 0; j < U; ++j) {
-            const int t = t1 - j;
-            if (t >= 0) {
-                const int64_t r = (int64_t)t * b.B + e;
-                rw[j] = __ldcs(b.rec_reward + r); vl[j] = __ldcs(b.rec_value + r);
-            }
-        }
-#pragma unroll
-        for (int j = 0; j < U; ++j) {
-            const int t = t1 - j;
-            if (t >= 0) {
-                if (t == n - 1) { adv = __fsub_rn(rw[j], vl[j]); ret = rw[j]; }
-                else gae_step(rw[j], vl[j], v_next, adv, gamma, lambda, adv, ret);
-                const int64_t r = (int64_t)t * b.B + e;
-                b.rec_adv[r] = adv; b.rec_ret[r] = ret;
-                v_next = vl[j];
-            }
-        }
-    }
-}
-
 __global__ void __launch_bounds__(256) k_gae_concat(const float* __restrict__ rw, const float* __restrict__ vl,
                                                     const int64_t* __restrict__ off, int64_t n_ep, float gamma, float lambda,
                                                     float* __restrict__ advs, float* __restrict__ rets) {
@@ -283,10 +250,6 @@ __global__ void __launch_bounds__(256) k_gae_concat(const float* __restrict__ rw
     }
 }
 
-void launch_gae_time_major(cudaStream_t st, const CollectBuffers& b, float gamma, float lambda) {
-    k_gae_time_major<<<grid_for(b.B, 64), 64, 0, st>>>(b, gamma, lambda);
-    TWR_COUNT_LAUNCH();
-}
 void launch_gae_concat(cudaStream_t st, const float* r, const float* v, const int64_t* off, int64_t n_ep, float gamma,
                        float lambda, float* adv, float* ret) {
     if (n_ep <= 0) return;
@@ -355,7 +318,8 @@ struct CompactTiles {
 // FUSE_GAE (the PPO collect): the block walks its 32 episodes' tiles from the LAST time tile to the first and computes
 // advantages and returns on the way (K4b's reverse recursion, one lane of warp 0 per episode, carried across tiles in
 // registers) -- the records are read once, and the time-major adv / ret arrays are neither written nor read: 42 B R + 66 B W
-// per record instead of 16 + 16 (GAE) + 50 + 66.  Same f32 operations in the same order as k_gae_time_major.
+// per record instead of 16 + 16 (GAE) + 50 + 66.  Same f32 operations (gae_step) in the same order as k_gae_concat, the
+// stand-alone GAE of twr_gae.
 template <bool FUSE_GAE>
 __global__ void __launch_bounds__(256) k_compact(EnvParams p, CollectBuffers b, int A, float gamma, float lambda) {
     extern __shared__ __align__(16) unsigned char compact_smem[];
@@ -460,15 +424,7 @@ __global__ void __launch_bounds__(256) k_compact(EnvParams p, CollectBuffers b, 
             if (x < nt) {
                 const uint4 q = tl.q[1][x][ey];
                 const uint32_t w[4] = {q.x, q.y, q.z, q.w};
-                if (b.obs_u8 == 2) {
-                    uint32_t h[4];
-#pragma unroll
-                    for (int k = 0; k < 4; ++k) {          // bytes (b0 b1 b2 b3), all < 16 -> (b0 | b1 << 4), (b2 | b3 << 4)
-                        const uint32_t t = (w[k] | (w[k] >> 4)) & 0x00FF00FFu;
-                        h[k] = (t | (t >> 8)) & 0xFFFFu;
-                    }
-                    reinterpret_cast<uint2*>(reinterpret_cast<uint8_t*>(b.out_obs) + r0 * 8)[x] = make_uint2(h[0] | (h[1] << 16), h[2] | (h[3] << 16));
-                } else if (b.obs_u8) {
+                if (b.obs_u8) {
                     uint32_t o[4];
 #pragma unroll
                     for (int k = 0; k < 4; ++k)            // cell i = 4k+j holds tile byte j of word k; index = i*16 + tile
@@ -520,7 +476,7 @@ void launch_compact(cudaStream_t st, const EnvParams& p, const CollectBuffers& b
     k_compact<false><<<grid, dim3(32, 8), sizeof(CompactTiles), st>>>(p, b, A, 0.f, 0.f);
     TWR_COUNT_LAUNCH();
 }
-// K4b + K5 in one pass (see k_compact<true>): the caller does not run launch_gae_time_major
+// K4b + K5 in one pass (see k_compact<true>)
 void launch_compact_gae(cudaStream_t st, const EnvParams& p, const CollectBuffers& b, int A, float gamma, float lambda) {
     cudaFuncSetAttribute(k_compact<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(CompactTiles));
     k_compact<true><<<dim3(grid_for(b.B, 32)), dim3(32, 8), sizeof(CompactTiles), st>>>(p, b, A, gamma, lambda);

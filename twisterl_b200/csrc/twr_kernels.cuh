@@ -57,9 +57,7 @@ struct CollectBuffers {
     int64_t* ep_off;      // [B] record offset of local episode e (plain local order; the id rotation gives merge order)
     int32_t* ep_len_id;   // [total episodes] episode length by episode id (filled by k_episode_offsets)
     int64_t out_base;     // records of earlier sub-batches (pipelined host collect)
-    int obs_u8;           // compaction writes one byte per observation index (twr_host_buffers.obs_u8); 2: 16-cell puzzles,
-                          // the 16 tile values as nibbles (8 bytes per record, cell 2j in the low half of byte j) -- the wire
-                          // format of twr_ppo_collect_host, expanded to indices by its host threads
+    int obs_u8;           // 1: compaction writes one byte per observation index (twr_host_buffers.obs_u8); 0: u16 indices
     int pack_misc;        // compaction writes ONE byte per record into out_actions -- action | reward code << 2 | (perm + 1) << 4 --
                           // and skips out_perms / out_rewards / out_advs: the pipelined host collect rebuilds those on the host
                           // (Puzzle rewards take three values, puzzle.rs:171-177; advs = rets - values, ppo.rs:87-91)
@@ -95,11 +93,10 @@ void launch_sample(cudaStream_t s, const float* d_logits, int64_t n, int A, uint
 // K3+K4a+K1 fused collect step: mask, Gumbel-max sample, trajectory write, env step, live compaction
 void launch_collect_step(cudaStream_t s, const StepArgs& a, const CollectBuffers& b, const int32_t* live_cur,
                          int32_t* live_next);
-// K4b GAE reverse scan (time-major records) and standalone (concatenated episodes)
 // survivors (ep_len == 0) of live_cur[0..*n_cur) -> live_next, count -> *n_next (must be zeroed)
 void launch_compact_live(cudaStream_t s, const int32_t* live_cur, const int32_t* n_cur, const int32_t* ep_len, int64_t max_n,
                          int32_t* live_next, int32_t* n_next);
-void launch_gae_time_major(cudaStream_t s, const CollectBuffers& b, float gamma, float lambda);
+// K4b GAE, stand-alone over concatenated episodes (the PPO collect runs it inside launch_compact_gae)
 void launch_gae_concat(cudaStream_t s, const float* r, const float* v, const int64_t* off, int64_t n_ep,
                        float gamma, float lambda, float* adv, float* ret);
 // K5 episode offsets in merged order + transpose/compaction into concatenated episodes

@@ -43,9 +43,7 @@ struct twr_engine {
     int32_t* bal_flags = nullptr;   // hand-off counters of the balanced pair-kernel schedule (one per CTA pair)
     int bal_delta = 3;
 #define TWR_MAX_SUBBATCH 64
-    cudaEvent_t ev_done[2] = {nullptr, nullptr}, ev_copied[TWR_MAX_SUBBATCH] = {}, ev_small[TWR_MAX_SUBBATCH] = {}, ev_obs[TWR_MAX_SUBBATCH] = {};
-    unsigned char* h_obs_nib = nullptr;      // pinned staging of twr_ppo_collect_host's nibble-packed observations (8 B / record)
-    size_t h_obs_nib_bytes = 0;
+    cudaEvent_t ev_done[2] = {nullptr, nullptr}, ev_copied[TWR_MAX_SUBBATCH] = {}, ev_small[TWR_MAX_SUBBATCH] = {};
     unsigned long long* h_stats = nullptr;   // pinned, mapped
     unsigned long long* d_hstats = nullptr;  // its device address
     bool has_last = false;
