@@ -1,7 +1,8 @@
 """GPU parity tests: the CUDA path (through the C ABI) against the CPU oracle on the same seeded inputs,
 against the committed golden fixtures, and -- at BASELINE.json's full size -- through size-independent
 properties.  Bars: bit-exact for env transitions / observations / masks / rewards / twists / episode
-layout; |d| <= 1e-5 * max(1,|ref|) for fp32 logits and values (1e-3 for the f16x2 tensor-core forward);
+layout; |d| <= 1e-5 * max(1,|ref|) for fp32 logits and values (1e-4 for the f16x2
+tensor-core forward, 1e-3 for f16x2w16 and f16f8c);
 1e-5 for GAE (the kernel is in fact bit-exact); chi-square p > 0.001 for sampled actions."""
 import os
 
@@ -17,7 +18,7 @@ from oracle import orc
 pytestmark = pytest.mark.gpu
 
 PRECISION = suite_precision(globals())
-TOL = 1e-5 if PRECISION == "fp32" else 1e-3
+TOL = {"fp32": 1e-5, "f16x2": 1e-4}.get(PRECISION, 1e-3)
 
 
 @pytest.fixture(scope="module")
