@@ -205,7 +205,14 @@ int twr_engine_create(const twr_engine_cfg* cfg, twr_engine** out) {
     });
 }
 
-static void mcts_release_fwd(twr_engine* e);
+static void mcts_release(twr_engine* e) {
+    MctsCache& c = e->mcts;
+    dev_free(c.cells); dev_free(c.node); dev_free(c.meta); dev_free(c.parent); dev_free(c.n_nodes); dev_free(c.fwd_list);
+    dev_free(c.fwd_env); dev_free(c.fwd_count); dev_free(c.cur_node); dev_free(c.path); dev_free(c.path_len); dev_free(c.leaf_pos);
+    dev_free(c.active); dev_free(c.cur_value);
+    c.cap_nodes = 0; c.cap_B = 0;
+}
+
 static void free_collect_buffers(twr_engine* e) {
     CollectBuffers& b = e->buf;
     dev_free(b.cells); dev_free(b.meta); dev_free(b.live_a); dev_free(b.live_b); dev_free(b.n_live);
@@ -225,7 +232,7 @@ void twr_engine_destroy(twr_engine* e) {
     cudaSetDevice(e->device);
     cudaStreamSynchronize(e->stream);
     twr_comm_destroy(e);
-    mcts_release_fwd(e);
+    mcts_release(e);
     if (e->trace_buf) { cudaFree(e->trace_buf); e->trace_buf = nullptr; }
     free_collect_buffers(e);
     for (auto ev : e->ev) cudaEventDestroy(ev);
@@ -361,10 +368,16 @@ static int expand_conv1d(const twr_policy_desc* d, twr_policy_desc* out, std::ve
     return TWR_OK;
 }
 
+// the largest N with N * N <= obs_size: the board side of a table whose rows are (cell, value) pairs of an N-cell board
+static int board_side(int obs_size) {
+    int N = 1;
+    while ((N + 1) * (N + 1) <= obs_size) ++N;
+    return N;
+}
+
 // PolicyDev::tc_fold: N when obs_size = N * N and every twist maps each block of N rows onto a block (all blocks hit once)
 static int fold_block(const twr_policy_desc* d) {
-    int N = 1;
-    while ((N + 1) * (N + 1) <= d->obs_size) ++N;
+    const int N = board_side(d->obs_size);
     if (N * N != d->obs_size || N > TWR_MAX_CELLS) return 0;
     for (int q = 0; q < d->n_perms; ++q) {
         const int32_t* pm = d->obs_perms + (size_t)q * d->obs_size;
@@ -452,8 +465,7 @@ int twr_policy_create(twr_engine* e, const twr_policy_desc* d_in, twr_policy** o
         // GridWorld-shaped tables (obs_size = N*N > 256, only rows i*N + {0,1,2,3} reachable): the pair kernel runs on
         // the compact 4N-row table when the twists (if any) keep the reachable rows among themselves
         if (e->precision != TWR_PREC_FP32 && d->obs_size > 256) {
-            int N = 1;
-            while ((N + 1) * (N + 1) <= d->obs_size) ++N;
+            const int N = board_side(d->obs_size);
             bool ok = N * N == d->obs_size && N <= TWR_MAX_CELLS && 4 * N <= 256;
             for (int64_t i = 0; ok && i < (int64_t)d->n_perms * d->obs_size; ++i)
                 if ((i % d->obs_size) % N < 4 && d->obs_perms[i] % N >= 4) ok = false;
@@ -664,14 +676,35 @@ int twr_envs_success(twr_envs* v, uint8_t* s) { return query_field<uint8_t>(v, s
 int twr_envs_depth(twr_envs* v, int32_t* d) { return query_field<int32_t>(v, d, 1, 6); }
 
 // -------------------------------------------------------------------- forward ---
+// The policy as one forward runs it, over envs `env` or (env NULL) the n rows of n_obs indices in `obs`: tc_pack cleared,
+// so the fp32 kernel runs, for a compact-table policy outside GridWorld envs of its size, or a row that repeats an index
+// (the one-hot GEMM operand cannot express one).
+static PolicyDev call_dev(const PolicyDev& pol, const EnvParams* env, const int32_t* obs, int64_t n, int n_obs) {
+    PolicyDev dev = pol;
+    dev.n_obs = env ? env->N : n_obs;
+    bool tc = pol.tc_pack && (pol.tc_compact_n == 0 || (env && env->kind == TWR_ENV_GRIDWORLD && env->N == pol.tc_compact_n));
+    for (int64_t i = 0; tc && obs && i < n; ++i)
+        for (int a = 0; tc && a < n_obs; ++a)
+            for (int b = a + 1; tc && b < n_obs; ++b) tc = obs[i * n_obs + a] != obs[i * n_obs + b];
+    if (!tc) dev.tc_pack = nullptr;
+    return dev;
+}
+
 static int check_policy_env(const twr_policy* p, const EnvParams& env, PolicyDev* dev) {
     if (p->dev.obs_size != env.N * env.N)
         return fail(TWR_ERR_INVALID, "policy obs_size does not match the env's obs_shape (cells*cells)");
     if (p->dev.A != 4) return fail(TWR_ERR_INVALID, "policy has " + std::to_string(p->dev.A) + " actions, env has 4");
-    *dev = p->dev;
-    dev->n_obs = env.N;
-    if (dev->tc_compact_n > 0 && (env.kind != TWR_ENV_GRIDWORLD || env.N != dev->tc_compact_n)) dev->tc_pack = nullptr;   // fp32 kernel
+    *dev = call_dev(p->dev, &env, nullptr, 0, 0);
     return TWR_OK;
+}
+
+// what every forward sets: its envs, its twist-pick stream (t = -1 outside a rollout) and its outputs
+static ForwardArgs forward_args(const twr_engine* e, const EnvParams& env, uint32_t cid, EnvIds ids, const uint4* cells,
+                                int64_t n, float4* logits, float* values) {
+    ForwardArgs a{};
+    a.env = env; a.seed = e->seed; a.cid = cid; a.ids = ids; a.t = -1;
+    a.cells = cells; a.n = n; a.logits = logits; a.values = values;
+    return a;
 }
 
 static void launch_forward(twr_engine* e, const PolicyDev& dev, const ForwardArgs& a) {
@@ -685,14 +718,51 @@ static void launch_forward(twr_engine* e, const PolicyDev& dev, const ForwardArg
     } else ok = launch_forward_fp32(e->stream, dev, a);
     if (!ok) e->launch_error = true;
 }
-// after the launches of a call: a forward that could not be launched must not look like success (no records, TWR_OK)
+// after the launches of a call: a launch error or an unlaunched forward must not look like success (no records, TWR_OK)
 #define FWD_CHECK(e)                                                                                          \
     do {                                                                                                      \
+        CU_TRY(cudaGetLastError());                                                                           \
         if ((e)->launch_error) {                                                                              \
             (e)->launch_error = false;                                                                        \
             return fail(TWR_ERR_CUDA, "policy forward kernel could not be launched (shape / shared memory / tensor map)"); \
         }                                                                                                     \
     } while (0)
+
+// A forward whose results go back to the caller: outputs for `slices` x n rows (full_predict: one slice per twist) and
+// the caller's perm_idx (NULL: Philox pick), range-checked before anything is allocated.
+struct HostForward {
+    Staging<float4> logits; Staging<float> values; Staging<int32_t> perm;
+    int64_t n = 0;
+    int stage(twr_engine* e, const PolicyDev& dev, const EnvParams& env, const uint4* cells, int64_t rows, size_t slices,
+              const int32_t* perm_idx, ForwardArgs* a) {
+        if (perm_idx)
+            for (int64_t i = 0; i < rows; ++i)
+                if (perm_idx[i] < -1 || perm_idx[i] >= dev.n_perms) return fail(TWR_ERR_INVALID, "perm_idx out of range");
+        CU_TRY(cudaSetDevice(e->device));
+        n = rows;
+        int rc;
+        if ((rc = logits.alloc(slices * (size_t)n)) || (rc = values.alloc(slices * (size_t)n))) return rc;
+        if (perm_idx) {
+            if ((rc = perm.alloc((size_t)n))) return rc;
+            CU_TRY(cudaMemcpyAsync(perm.d, perm_idx, sizeof(int32_t) * (size_t)n, cudaMemcpyHostToDevice, e->stream));
+        }
+        *a = forward_args(e, env, 0, EnvIds{}, cells, n, logits.d, values.d);
+        a->perm_idx = perm.d;
+        return TWR_OK;
+    }
+    // after FWD_CHECK: logits as [n][A] and values to the host
+    int to_host(twr_engine* e, int A, float* h_logits, float* h_values) {
+        std::vector<float4> h((size_t)n);
+        CU_TRY(cudaMemcpyAsync(h.data(), logits.d, sizeof(float4) * (size_t)n, cudaMemcpyDeviceToHost, e->stream));
+        CU_TRY(cudaMemcpyAsync(h_values, values.d, sizeof(float) * (size_t)n, cudaMemcpyDeviceToHost, e->stream));
+        CU_TRY(cudaStreamSynchronize(e->stream));
+        for (int64_t i = 0; i < n; ++i) {
+            const float l[4] = {h[i].x, h[i].y, h[i].z, h[i].w};
+            for (int k = 0; k < A; ++k) h_logits[i * A + k] = l[k];
+        }
+        return TWR_OK;
+    }
+};
 
 int twr_policy_forward(twr_engine* e, const twr_policy* p, twr_envs* v, const int32_t* perm_idx, int32_t apply_masks,
                        float* logits, float* values) {
@@ -703,35 +773,13 @@ int twr_policy_forward(twr_engine* e, const twr_policy* p, twr_envs* v, const in
     PolicyDev dev;
     int rc = check_policy_env(p, v->p, &dev);
     if (rc) return rc;
-    if (perm_idx) {
-        for (int64_t i = 0; i < v->n; ++i)
-            if (perm_idx[i] < -1 || perm_idx[i] >= p->dev.n_perms) return fail(TWR_ERR_INVALID, "perm_idx out of range");
-    }
-    CU_TRY(cudaSetDevice(e->device));
-    Staging<float4> d_logits; Staging<float> d_values; Staging<int32_t> d_perm;
-    if ((rc = d_logits.alloc((size_t)v->n)) || (rc = d_values.alloc((size_t)v->n))) return rc;
-    if (perm_idx) {
-        if ((rc = d_perm.alloc((size_t)v->n))) return rc;
-        CU_TRY(cudaMemcpyAsync(d_perm.d, perm_idx, sizeof(int32_t) * (size_t)v->n, cudaMemcpyHostToDevice, e->stream));
-    }
-    ForwardArgs a{};
-    a.env = v->p; a.seed = e->seed; a.cid = 0; a.ids = EnvIds{0u, 0u, 0u}; a.t = -1;
-    a.perm_idx = perm_idx ? d_perm.d : nullptr;
-    a.cells = v->cells; a.live = nullptr; a.n_live_ptr = nullptr; a.n = v->n;
-    a.logits = d_logits.d; a.values = d_values.d;
+    HostForward f;
+    ForwardArgs a;
+    if ((rc = f.stage(e, dev, v->p, v->cells, v->n, 1, perm_idx, &a))) return rc;
     launch_forward(e, dev, a);
-    if (apply_masks) launch_mask_logits(e->stream, v->p, v->cells, v->meta, v->n, dev.A, d_logits.d);
-    CU_TRY(cudaGetLastError());
+    if (apply_masks) launch_mask_logits(e->stream, v->p, v->cells, v->meta, v->n, dev.A, a.logits);
     FWD_CHECK(e);
-    std::vector<float4> h((size_t)v->n);
-    CU_TRY(cudaMemcpyAsync(h.data(), d_logits.d, sizeof(float4) * (size_t)v->n, cudaMemcpyDeviceToHost, e->stream));
-    CU_TRY(cudaMemcpyAsync(values, d_values.d, sizeof(float) * (size_t)v->n, cudaMemcpyDeviceToHost, e->stream));
-    CU_TRY(cudaStreamSynchronize(e->stream));
-    for (int64_t i = 0; i < v->n; ++i) {
-        const float l[4] = {h[i].x, h[i].y, h[i].z, h[i].w};
-        for (int a2 = 0; a2 < dev.A; ++a2) logits[i * dev.A + a2] = l[a2];
-    }
-    return TWR_OK;
+    return f.to_host(e, dev.A, logits, values);
     });
 }
 
@@ -741,18 +789,17 @@ int twr_debug_forward_profile(twr_engine* e, const twr_policy* p, twr_envs* v, i
     PolicyDev dev;
     int rc = check_policy_env(p, v->p, &dev);
     if (rc) return rc;
-    CU_TRY(cudaSetDevice(e->device));
-    Staging<float4> d_logits; Staging<float> d_values; Staging<long long> d_dbg;
-    if ((rc = d_logits.alloc((size_t)v->n)) || (rc = d_values.alloc((size_t)v->n)) || (rc = d_dbg.alloc((size_t)148 * 16 + 256))) return rc;
-    if (max_ctas < 148 + 16) return fail(TWR_ERR_INVALID, "counters buffer must hold 148*16 + 256 int64");
-    CU_TRY(cudaMemsetAsync(d_dbg.d, 0, sizeof(long long) * ((size_t)148 * 16 + 256), e->stream));
-    ForwardArgs a{};
-    a.env = v->p; a.seed = e->seed; a.t = -1; a.cells = v->cells; a.n = v->n;
-    a.logits = d_logits.d; a.values = d_values.d; a.dbg = d_dbg.d; a.dbg_flags = flags;
+    if (max_ctas < TWR_DBG_CTAS + 16)
+        return fail(TWR_ERR_INVALID, "counters buffer must hold " + std::to_string(TWR_DBG_CTAS) + "*16 + 256 int64");
+    HostForward f;
+    ForwardArgs a;
+    Staging<long long> d_dbg;
+    if ((rc = f.stage(e, dev, v->p, v->cells, v->n, 1, nullptr, &a)) || (rc = d_dbg.alloc(TWR_DBG_WORDS))) return rc;
+    CU_TRY(cudaMemsetAsync(d_dbg.d, 0, sizeof(long long) * TWR_DBG_WORDS, e->stream));
+    a.dbg = d_dbg.d; a.dbg_flags = flags;
     launch_forward(e, dev, a);
-    CU_TRY(cudaGetLastError());
     FWD_CHECK(e);
-    CU_TRY(cudaMemcpyAsync(counters, d_dbg.d, sizeof(long long) * ((size_t)148 * 16 + 256), cudaMemcpyDeviceToHost, e->stream));
+    CU_TRY(cudaMemcpyAsync(counters, d_dbg.d, sizeof(long long) * TWR_DBG_WORDS, cudaMemcpyDeviceToHost, e->stream));
     CU_TRY(cudaStreamSynchronize(e->stream));
     return TWR_OK;
     });
@@ -774,9 +821,6 @@ int twr_policy_forward_obs(twr_engine* e, const twr_policy* p, const int32_t* ob
     if (n <= 0) return TWR_OK;
     for (int64_t i = 0; i < n * n_obs; ++i)
         if (obs[i] < 0 || obs[i] >= p->dev.obs_size) return fail(TWR_ERR_INVALID, "observation index out of range");
-    if (perm_idx)
-        for (int64_t i = 0; i < n; ++i)
-            if (perm_idx[i] < -1 || perm_idx[i] >= p->dev.n_perms) return fail(TWR_ERR_INVALID, "perm_idx out of range");
     // one index per block of tc_fold rows? (then the bias-folded f16f8c image applies to these observations too)
     bool blocks = p->dev.tc_fold > 0 && n_obs == p->dev.tc_fold;
     for (int64_t i = 0; blocks && i < n; ++i) {
@@ -784,42 +828,19 @@ int twr_policy_forward_obs(twr_engine* e, const twr_policy* p, const int32_t* ob
         for (int a2 = 0; a2 < n_obs; ++a2) seen |= 1ull << (obs[i * n_obs + a2] / p->dev.tc_fold);
         blocks = seen == (n_obs >= 64 ? ~0ull : (1ull << n_obs) - 1);
     }
-    bool multiset = false;                   // the one-hot GEMM operand cannot express a repeated index: fp32 kernel then
-    if (p->dev.tc_pack) {
-        for (int64_t i = 0; i < n && !multiset; ++i)
-            for (int a2 = 0; a2 < n_obs && !multiset; ++a2)
-                for (int b2 = a2 + 1; b2 < n_obs; ++b2)
-                    if (obs[i * n_obs + a2] == obs[i * n_obs + b2]) { multiset = true; break; }
-    }
-    CU_TRY(cudaSetDevice(e->device));
-    PolicyDev dev = p->dev;
-    dev.n_obs = n_obs;
-    if (multiset || dev.tc_compact_n > 0) dev.tc_pack = nullptr;   // arbitrary indices: not the compact GridWorld table
-    Staging<float4> d_logits; Staging<float> d_values; Staging<int32_t> d_perm, d_obs;
+    const PolicyDev dev = call_dev(p->dev, nullptr, obs, n, n_obs);
+    EnvParams obs_env{};                     // only the index count: the rows are given, not read from env state
+    obs_env.N = n_obs;
+    HostForward f;
+    ForwardArgs a;
+    Staging<int32_t> d_obs;
     int rc;
-    if ((rc = d_logits.alloc((size_t)n)) || (rc = d_values.alloc((size_t)n)) || (rc = d_obs.alloc((size_t)n * n_obs))) return rc;
+    if ((rc = f.stage(e, dev, obs_env, nullptr, n, 1, perm_idx, &a)) || (rc = d_obs.alloc((size_t)n * n_obs))) return rc;
     CU_TRY(cudaMemcpyAsync(d_obs.d, obs, sizeof(int32_t) * (size_t)n * n_obs, cudaMemcpyHostToDevice, e->stream));
-    if (perm_idx) {
-        if ((rc = d_perm.alloc((size_t)n))) return rc;
-        CU_TRY(cudaMemcpyAsync(d_perm.d, perm_idx, sizeof(int32_t) * (size_t)n, cudaMemcpyHostToDevice, e->stream));
-    }
-    ForwardArgs a{};
-    a.env.N = n_obs; a.seed = e->seed; a.t = -1;
-    a.perm_idx = perm_idx ? d_perm.d : nullptr;
-    a.obs_rows = d_obs.d; a.n = n; a.obs_blocks = blocks ? 1 : 0;
-    a.logits = d_logits.d; a.values = d_values.d;
+    a.obs_rows = d_obs.d; a.obs_blocks = blocks ? 1 : 0;
     launch_forward(e, dev, a);
-    CU_TRY(cudaGetLastError());
     FWD_CHECK(e);
-    std::vector<float4> h((size_t)n);
-    CU_TRY(cudaMemcpyAsync(h.data(), d_logits.d, sizeof(float4) * (size_t)n, cudaMemcpyDeviceToHost, e->stream));
-    CU_TRY(cudaMemcpyAsync(values, d_values.d, sizeof(float) * (size_t)n, cudaMemcpyDeviceToHost, e->stream));
-    CU_TRY(cudaStreamSynchronize(e->stream));
-    for (int64_t i = 0; i < n; ++i) {
-        const float l[4] = {h[i].x, h[i].y, h[i].z, h[i].w};
-        for (int a2 = 0; a2 < dev.A; ++a2) logits[i * dev.A + a2] = l[a2];
-    }
-    return TWR_OK;
+    return f.to_host(e, dev.A, logits, values);
     });
 }
 
@@ -926,8 +947,6 @@ static int ensure_collect_buffers(twr_engine* e, int64_t B, int T, int cells, in
     return TWR_OK;
 }
 
-// Enqueue one (sub-)collect of B local episodes on the engine stream: reset -> T x (forward [+ step]) -> GAE ->
-// offsets -> compaction into output set `which`.  No host synchronisation.
 static uint64_t hint_key_of(const EnvParams& p, int64_t B) {
     uint64_t k = 1469598103934665603ull;
     const int64_t f[] = {p.kind, p.W, p.H, p.difficulty, p.depth_slope, p.max_depth, B};
@@ -935,22 +954,69 @@ static uint64_t hint_key_of(const EnvParams& p, int64_t B) {
     return k;
 }
 
+// the start of a collect of B episodes into output set `which`: its counters zeroed, every env reset and listed live
+static int begin_collect(twr_engine* e, const EnvParams& env, int64_t B, EnvIds ids, uint32_t cid, int which) {
+    CollectBuffers& b = e->buf;
+    b.B = B;
+    select_outset(e, which);
+    CU_TRY(cudaMemsetAsync(b.n_live, 0, sizeof(int32_t) * (size_t)(b.Tmax + 1), e->stream));
+    CU_TRY(cudaMemsetAsync(b.stats, 0, sizeof(unsigned long long) * 4, e->stream));
+    launch_envs_reset(e->stream, env, b.cells, b.meta, B, e->seed, ids, cid, b.live_a, b.n_live);
+    return TWR_OK;
+}
+
+// forward n_fwd of a collect, between its pair of timing events when timing is on (twr_engine_set_timing)
+static void launch_forward_timed(twr_engine* e, const PolicyDev& dev, const ForwardArgs& a, int n_fwd) {
+    const bool timed = e->timing && 2 * n_fwd + 1 < (int)e->ev.size();
+    if (timed) cudaEventRecord(e->ev[2 * n_fwd], e->stream);
+    launch_forward(e, dev, a);
+    if (timed) cudaEventRecord(e->ev[2 * n_fwd + 1], e->stream);
+}
+
+// TWISTERL_B200_TRACE=<chunk index>: zeroed pipeline counters for that chunk's launch (one buffer per engine), else NULL
+static long long* trace_counters(twr_engine* e, int ci) {
+    static const char* trace_env = getenv("TWISTERL_B200_TRACE");
+    if (!trace_env || ci != atoi(trace_env)) return nullptr;
+    if (!e->trace_buf) cudaMalloc(reinterpret_cast<void**>(&e->trace_buf), sizeof(long long) * TWR_DBG_WORDS);
+    cudaMemsetAsync(e->trace_buf, 0, sizeof(long long) * TWR_DBG_WORDS, e->stream);
+    return e->trace_buf;
+}
+
+// the counters of the traced launch (chunk ci of cnt steps over B envs) on stderr, once it has run
+static void print_trace(twr_engine* e, int ci, int cnt, int64_t B) {
+    std::vector<long long> h(TWR_DBG_WORDS);
+    cudaMemcpyAsync(h.data(), e->trace_buf, sizeof(long long) * h.size(), cudaMemcpyDeviceToHost, e->stream);
+    cudaStreamSynchronize(e->stream);
+    static const char* names[16] = {"mma total", "mma wait slot", "mma wait a1_full", "mma wait a2_full", "mma wait d2_empty", "lanes",
+                                    "mma slot wait G1", "mma slot wait G1 first", "producer wait empty", "epi total", "epi wait d1_full",
+                                    "epi wait d2_full", "epi wait a1_empty", "epi1 busy", "build_a1", "epi2+step busy"};
+    fprintf(stderr, "[trace] chunk %d, %d steps, %lld live envs\n", ci, cnt, (long long)B);
+    for (int k = 0; k < 16; ++k) {
+        double sum = 0; int n = 0; long long mx = 0;
+        for (int c = 0; c < TWR_DBG_CTAS; ++c) { const long long v = h[(size_t)c * 16 + k]; if (v) { sum += (double)v; ++n; if (v > mx) mx = v; } }
+        fprintf(stderr, "[trace] %-24s cta0 %10lld  mean(nonzero) %12.1f  max %10lld\n", names[k], h[k], n ? sum / n : 0.0, mx);
+    }
+    const long long* tr = h.data() + TWR_DBG_TRACE;
+    for (int item = 0; item < 8; ++item) {
+        fprintf(stderr, "[trace] item %d:", item);
+        for (int ev = 0; ev < 27; ++ev) if (tr[item * 32 + ev]) fprintf(stderr, " %d@%lld", ev, tr[item * 32 + ev] - tr[0]);
+        fprintf(stderr, "\n");
+    }
+}
+
+// Enqueue one (sub-)collect of B local episodes on the engine stream: reset -> T x (forward [+ step]) -> GAE ->
+// offsets -> compaction into output set `which`.  No host synchronisation.
 static int enqueue_collect(twr_engine* e, const EnvParams& env, const PolicyDev& dev, int64_t B, EnvIds ids, uint32_t cid,
                            float gamma, float lambda, int which, int* n_fwd_out, cudaEvent_t outset_free = nullptr) {
     CollectBuffers& b = e->buf;
     cudaStream_t st = e->stream;
     const int T = b.Tmax;
-    b.B = B;
-    select_outset(e, which);
-    CU_TRY(cudaMemsetAsync(b.n_live, 0, sizeof(int32_t) * (size_t)(T + 1), st));
-    CU_TRY(cudaMemsetAsync(b.stats, 0, sizeof(unsigned long long) * 4, st));
-    launch_envs_reset(st, env, b.cells, b.meta, B, e->seed, ids, cid, b.live_a, b.n_live);
+    int rc = begin_collect(e, env, B, ids, cid, which);
+    if (rc) return rc;
 
     StepArgs sa{};
     sa.env = env; sa.seed = e->seed; sa.cid = cid; sa.ids = ids; sa.n_perms = dev.n_perms; sa.A = dev.A;
-    ForwardArgs fa{};
-    fa.env = env; fa.seed = e->seed; fa.cid = cid; fa.ids = ids; fa.perm_idx = nullptr;
-    fa.cells = b.cells; fa.n = B; fa.logits = b.logits; fa.values = b.values;
+    ForwardArgs fa = forward_args(e, env, cid, ids, b.cells, B, b.logits, b.values);
     const bool fused = dev.tc_pack != nullptr;            // the tensor-core kernel runs the collect step in its epilogue
     int n_fwd = *n_fwd_out;
     if (fused) {
@@ -986,37 +1052,9 @@ static int enqueue_collect(twr_engine* e, const EnvParams& env, const PolicyDev&
                 CU_TRY(cudaMemsetAsync(e->bal_flags, 0, 1024 * sizeof(int32_t), st));
                 fa.bal_flags = e->bal_flags; fa.bal_delta = bal_delta;
             }
-            if (e->timing && 2 * n_fwd + 1 < (int)e->ev.size()) cudaEventRecord(e->ev[2 * n_fwd], st);
-            fa.dbg = nullptr;
-            long long*& trace_buf = e->trace_buf;             // TWISTERL_B200_TRACE=<chunk index>: pipeline counters of that launch (per engine)
-            static const char* trace_env = getenv("TWISTERL_B200_TRACE");
-            if (trace_env && ci == atoi(trace_env)) {
-                if (!trace_buf) cudaMalloc(reinterpret_cast<void**>(&trace_buf), sizeof(long long) * (148 * 16 + 256));
-                cudaMemsetAsync(trace_buf, 0, sizeof(long long) * (148 * 16 + 256), st);
-                fa.dbg = trace_buf;
-            }
-            launch_forward(e, dev, fa);
-            if (fa.dbg) {
-                std::vector<long long> h(148 * 16 + 256);
-                cudaMemcpyAsync(h.data(), trace_buf, sizeof(long long) * h.size(), cudaMemcpyDeviceToHost, st);
-                cudaStreamSynchronize(st);
-                static const char* names[16] = {"mma total", "mma wait slot", "mma wait a1_full", "mma wait a2_full", "mma wait d2_empty", "lanes",
-                                                "mma slot wait G1", "mma slot wait G1 first", "producer wait empty", "epi total", "epi wait d1_full",
-                                                "epi wait d2_full", "epi wait a1_empty", "epi1 busy", "build_a1", "epi2+step busy"};
-                fprintf(stderr, "[trace] chunk %d, %d steps, %lld live envs\n", ci, cnt, (long long)B);
-                for (int k = 0; k < 16; ++k) {
-                    double sum = 0; int n = 0; long long mx = 0;
-                    for (int c = 0; c < 148; ++c) { const long long v = h[(size_t)c * 16 + k]; if (v) { sum += (double)v; ++n; if (v > mx) mx = v; } }
-                    fprintf(stderr, "[trace] %-24s cta0 %10lld  mean(nonzero) %12.1f  max %10lld\n", names[k], h[k], n ? sum / n : 0.0, mx);
-                }
-                for (int item = 0; item < 8; ++item) {
-                    fprintf(stderr, "[trace] item %d:", item);
-                    for (int ev = 0; ev < 27; ++ev) if (h[148 * 16 + item * 32 + ev]) fprintf(stderr, " %d@%lld", ev, h[148 * 16 + item * 32 + ev] - h[148 * 16]);
-                    fprintf(stderr, "\n");
-                }
-            }
-            if (e->timing && 2 * n_fwd + 1 < (int)e->ev.size()) cudaEventRecord(e->ev[2 * n_fwd + 1], st);
-            ++n_fwd;
+            fa.dbg = trace_counters(e, ci);
+            launch_forward_timed(e, dev, fa, n_fwd++);
+            if (fa.dbg) print_trace(e, ci, cnt, B);
             if (cnt > 1) launch_compact_live(st, cur, b.n_live + ci, b.ep_len, B, nxt, b.n_live + ci + 1);
             int32_t* tmp = cur; cur = nxt; nxt = tmp;
         }
@@ -1030,10 +1068,7 @@ static int enqueue_collect(twr_engine* e, const EnvParams& env, const PolicyDev&
             int32_t* nxt = (t & 1) ? b.live_a : b.live_b;
             fa.t = t; fa.live = cur; fa.n_live_ptr = b.n_live + t;
             sa.t = t;
-            if (e->timing && 2 * n_fwd + 1 < (int)e->ev.size()) cudaEventRecord(e->ev[2 * n_fwd], st);
-            launch_forward(e, dev, fa);
-            if (e->timing && 2 * n_fwd + 1 < (int)e->ev.size()) cudaEventRecord(e->ev[2 * n_fwd + 1], st);
-            ++n_fwd;
+            launch_forward_timed(e, dev, fa, n_fwd++);
             launch_collect_step(st, sa, b, cur, nxt);
         }
     }
@@ -1043,7 +1078,6 @@ static int enqueue_collect(twr_engine* e, const EnvParams& env, const PolicyDev&
     // not in front of the rollout
     if (outset_free) CU_TRY(cudaStreamWaitEvent(st, outset_free, 0));
     launch_compact_gae(st, env, b, dev.A, gamma, lambda);      // GAE rides on the compaction (one pass over the records)
-    CU_TRY(cudaGetLastError());
     FWD_CHECK(e);
     return TWR_OK;
 }
@@ -1063,6 +1097,30 @@ static int plan_collect(twr_engine* e, const twr_env_spec* spec, const twr_polic
         return fail(TWR_ERR_INVALID, "GridWorld reset needs difficulty >= 1 (the reference loops forever at 0)");
     if ((rc = check_policy_env(p, plan->env, &plan->dev))) return rc;
     plan->T = horizon_of(plan->env) + 1;
+    return TWR_OK;
+}
+
+// the statistics words launch_publish_stats wrote for the collect just synchronised ([2] holds a double)
+struct CollectStats { int64_t successes, n_records; double reward_sum; };
+static CollectStats read_stats(const twr_engine* e) {
+    CollectStats s{(int64_t)e->h_stats[0], (int64_t)e->h_stats[1], 0.0};
+    memcpy(&s.reward_sum, &e->h_stats[2], sizeof(double));
+    return s;
+}
+
+// the end of a device-resident collect: its statistics to the host, then its result kept for twr_collected_to_host
+static int finish_collect(twr_engine* e, const CollectPlan& plan, int64_t num_episodes, twr_collected* out) {
+    launch_publish_stats(e->stream, e->buf.stats, e->d_hstats);
+    CU_TRY(cudaStreamSynchronize(e->stream));
+    const CollectStats s = read_stats(e);
+    const CollectBuffers& b = e->buf;
+    twr_collected& c = e->last;
+    c.n_records = s.n_records; c.num_episodes = num_episodes; c.n_cells = plan.env.N; c.num_actions = plan.dev.A;
+    c.successes = s.successes; c.reward_sum = s.reward_sum;
+    c.obs = b.out_obs; c.logits = b.out_logits; c.values = b.out_values; c.rewards = b.out_rewards;
+    c.advs = b.out_advs; c.rets = b.out_rets; c.actions = b.out_actions; c.perms = b.out_perms; c.ep_len = e->ep_len_id;
+    e->has_last = true;
+    *out = c;
     return TWR_OK;
 }
 
@@ -1097,21 +1155,9 @@ int twr_ppo_collect(twr_engine* e, const twr_env_spec* spec, const twr_policy* p
     int n_fwd = 0;
     if ((rc = enqueue_collect(e, plan.env, plan.dev, num_episodes, ids, cid, gamma, lambda, 0, &n_fwd))) return rc;
     if (e->timing) cudaEventRecord(e->ev_t1, st);
-    launch_publish_stats(st, e->buf.stats, e->d_hstats);
-    CU_TRY(cudaStreamSynchronize(st));
+    if ((rc = finish_collect(e, plan, num_episodes, out))) return rc;
     e->note_survival();
     finish_timing(e, n_fwd);
-    CollectBuffers& b = e->buf;
-    twr_collected& c = e->last;
-    c.n_records = (int64_t)e->h_stats[1];
-    c.num_episodes = num_episodes;
-    c.n_cells = plan.env.N; c.num_actions = plan.dev.A;
-    c.successes = (int64_t)e->h_stats[0];
-    double rs; memcpy(&rs, &e->h_stats[2], sizeof(double)); c.reward_sum = rs;
-    c.obs = b.out_obs; c.logits = b.out_logits; c.values = b.out_values; c.rewards = b.out_rewards;
-    c.advs = b.out_advs; c.rets = b.out_rets; c.actions = b.out_actions; c.perms = b.out_perms; c.ep_len = e->ep_len_id;
-    e->has_last = true;
-    *out = c;
     return TWR_OK;
     });
 }
@@ -1254,10 +1300,11 @@ int twr_ppo_collect_host(twr_engine* e, const twr_env_spec* spec, twr_policy* p,
             CU_TRY(cudaStreamSynchronize(e->stream));       // record count of this sub-batch -> host offsets
             FWD_CHECK(e);
             e->note_survival();
-            const size_t R = (size_t)e->h_stats[1];
+            const CollectStats s = read_stats(e);
+            const size_t R = (size_t)s.n_records;
             if (trace) { tr_done.push_back(now_ms()); tr_R.push_back(R); }
-            successes += (int64_t)e->h_stats[0];
-            double rs; memcpy(&rs, &e->h_stats[2], sizeof(double)); reward_sum += rs;
+            successes += s.successes;
+            reward_sum += s.reward_sum;
             if (at + (int64_t)R > dst->capacity) return fail(TWR_ERR_INVALID, "host buffers too small for the collected records");
             CU_TRY(cudaStreamWaitEvent(e->copy_stream, e->ev_done[which], 0));
             if (pack) {
@@ -1332,16 +1379,6 @@ int twr_ppo_collect_host(twr_engine* e, const twr_env_spec* spec, twr_policy* p,
 
 
 // ------------------------------------------------ batched MCTS driver (K6; also used by solve/evaluate) ---
-static void mcts_release(twr_engine* e);
-static void mcts_release_fwd(twr_engine* e) { mcts_release(e); }
-static void mcts_release(twr_engine* e) {
-    MctsCache& c = e->mcts;
-    dev_free(c.cells); dev_free(c.node); dev_free(c.meta); dev_free(c.parent); dev_free(c.n_nodes); dev_free(c.fwd_list);
-    dev_free(c.fwd_env); dev_free(c.fwd_count); dev_free(c.cur_node); dev_free(c.path); dev_free(c.path_len); dev_free(c.leaf_pos);
-    dev_free(c.active); dev_free(c.cur_value);
-    c.cap_nodes = 0; c.cap_B = 0;
-}
-
 // node pool of B trees x P nodes (+ per-env scratch) from the engine's cache, grown when a call needs more
 static int mcts_acquire(twr_engine* e, int64_t B, int P, MctsPool* pool, MctsArgs* a) {
     if (P >= (1 << 20)) return fail(TWR_ERR_INVALID, "MCTS tree too large (num_mcts_searches * max_expand_depth must stay below 2^18)");
@@ -1383,6 +1420,32 @@ static int stage_twists(twr_engine* e, const PolicyDev& dev, int64_t B, Staging<
     return TWR_OK;
 }
 
+// forward output slices of B rows in a search: one per twist of a twisted policy (Policy::full_predict), else one
+static size_t forward_slices(const PolicyDev& dev) { return dev.n_perms > 0 ? (size_t)dev.n_perms : 1; }
+
+struct MctsOpt { int n_sims; float C; int max_expand_depth; };
+
+// A search of B trees: its pool size checked before anything is allocated, the node pool from the engine's cache, the
+// twist rows of full_predict and the options.  mcts_target then sets what it runs on.
+static int mcts_reserve(twr_engine* e, const PolicyDev& dev, int64_t B, const MctsOpt& mo, Staging<int32_t>* twist_idx, MctsArgs* a) {
+    const int P = mcts_pool_nodes(dev.A, mo.n_sims, mo.max_expand_depth);
+    if ((double)B * P >= 2147483647.0)
+        return fail(TWR_ERR_INVALID, "MCTS node pool too large (num_episodes * (1 + A*(n_sims*depth+1)) must be < 2^31)");
+    *a = MctsArgs{};
+    a->pool.A = dev.A;
+    a->n_sims = mo.n_sims; a->max_expand_depth = mo.max_expand_depth; a->C = mo.C;
+    int rc;
+    if ((rc = mcts_acquire(e, B, P, &a->pool, a)) || (rc = stage_twists(e, dev, B, twist_idx, a))) return rc;
+    return TWR_OK;
+}
+
+// what a search runs on: its start envs, its Philox streams and its forward outputs (forward_slices slices of B rows)
+static void mcts_target(const twr_engine* e, MctsArgs* a, const EnvParams& env, uint32_t cid, EnvIds ids, const uint4* cells,
+                        const uint32_t* meta, const float4* logits, const float* values) {
+    a->env = env; a->seed = e->seed; a->cid = cid; a->ids = ids;
+    a->env_cells = cells; a->env_meta = meta; a->logits = logits; a->values = values;
+}
+
 // the forward of a leaf batch: one launch, or for a twisted policy one per twist, twist pi's outputs in slice pi
 static void launch_forward_twists(twr_engine* e, const PolicyDev& dev, const ForwardArgs& fa, const int32_t* twist_idx, int64_t stride) {
     if (dev.n_perms == 0) { launch_forward(e, dev, fa); return; }
@@ -1401,10 +1464,8 @@ static void enqueue_mcts(twr_engine* e, const PolicyDev& dev, MctsArgs& a, const
     cudaStream_t st = e->stream;
     // small batches: one persistent launch runs every simulation of the search (twr_mcts.cu, k_mcts_persistent)
     if (!getenv("TWISTERL_B200_MCTS_LOCKSTEP") && launch_mcts_persistent(st, a, dev, live, n_live, B)) return;
-    ForwardArgs fa{};
-    fa.env = a.env; fa.seed = e->seed; fa.cid = a.cid; fa.ids = a.ids; fa.t = -1;
-    fa.cells = a.pool.cells; fa.live = a.fwd_list; fa.n = B;
-    fa.logits = const_cast<float4*>(a.logits); fa.values = const_cast<float*>(a.values);
+    ForwardArgs fa = forward_args(e, a.env, a.cid, a.ids, a.pool.cells, B, const_cast<float4*>(a.logits), const_cast<float*>(a.values));
+    fa.live = a.fwd_list;
     auto forward = [&]() { launch_forward_twists(e, dev, fa, twist_idx, a.twist_stride); };
     launch_mcts_begin(st, a, live, n_live, B);
     fa.n_live_ptr = a.fwd_count;
@@ -1445,22 +1506,18 @@ int twr_policy_full_predict(twr_engine* e, const twr_policy* p, twr_envs* v, flo
     PolicyDev dev;
     int rc = check_policy_env(p, v->p, &dev);
     if (rc) return rc;
-    CU_TRY(cudaSetDevice(e->device));
     const int64_t n = v->n;
+    HostForward f;
+    ForwardArgs fa;
     MctsArgs a{};
     a.env = v->p; a.pool.A = dev.A;
-    const size_t slices = dev.n_perms > 0 ? (size_t)dev.n_perms : 1;
-    Staging<float4> d_logits; Staging<float> d_values, d_probs, d_out; Staging<int32_t> twist_idx;
-    if ((rc = d_logits.alloc(slices * (size_t)n)) || (rc = d_values.alloc(slices * (size_t)n)) || (rc = d_probs.alloc((size_t)n * dev.A)) ||
+    Staging<float> d_probs, d_out; Staging<int32_t> twist_idx;
+    if ((rc = f.stage(e, dev, v->p, v->cells, n, forward_slices(dev), nullptr, &fa)) || (rc = d_probs.alloc((size_t)n * dev.A)) ||
         (rc = d_out.alloc((size_t)n)) || (rc = stage_twists(e, dev, n, &twist_idx, &a))) return rc;
     // the leaf evaluation of the lockstep search: its forward launches, then its averaging and predict epilogue
-    ForwardArgs fa{};
-    fa.env = v->p; fa.seed = e->seed; fa.t = -1; fa.cells = v->cells; fa.n = n;
-    fa.logits = d_logits.d; fa.values = d_values.d;
     launch_forward_twists(e, dev, fa, twist_idx.d, n);
-    a.logits = d_logits.d; a.values = d_values.d;
+    a.logits = fa.logits; a.values = fa.values;
     launch_full_predict(e->stream, a, v->cells, v->meta, n, d_probs.d, d_out.d);
-    CU_TRY(cudaGetLastError());
     FWD_CHECK(e);
     CU_TRY(cudaMemcpyAsync(probs, d_probs.d, sizeof(float) * (size_t)n * dev.A, cudaMemcpyDeviceToHost, e->stream));
     CU_TRY(cudaMemcpyAsync(values, d_out.d, sizeof(float) * (size_t)n, cudaMemcpyDeviceToHost, e->stream));
@@ -1469,12 +1526,40 @@ int twr_policy_full_predict(twr_engine* e, const twr_policy* p, twr_envs* v, flo
     });
 }
 
+// every env of a batch of n live: the list 0..n-1 and its count n at n_live[0]
+static int upload_all_live(twr_engine* e, int32_t* live, int32_t* n_live, int64_t n) {
+    std::vector<int32_t> iota((size_t)n);
+    for (int64_t i = 0; i < n; ++i) iota[(size_t)i] = (int32_t)i;
+    const int32_t n32 = (int32_t)n;
+    CU_TRY(cudaMemcpyAsync(live, iota.data(), sizeof(int32_t) * (size_t)n, cudaMemcpyHostToDevice, e->stream));
+    CU_TRY(cudaMemcpyAsync(n_live, &n32, sizeof(int32_t), cudaMemcpyHostToDevice, e->stream));
+    return TWR_OK;
+}
+
+// MCTS steps are expensive: every few steps the searching loops synchronise to stop once no env is left live
+static int rollouts_ended(twr_engine* e, const int32_t* n_live, bool* ended) {
+    int32_t left = 0;
+    CU_TRY(cudaMemcpyAsync(&left, n_live, sizeof(int32_t), cudaMemcpyDeviceToHost, e->stream));
+    CU_TRY(cudaStreamSynchronize(e->stream));
+    *ended = left == 0;
+    return TWR_OK;
+}
 
 // ------------------------------------------------------------ evaluate / solve (f1) ---
+// The best of S searches by the tuple order (success, reward) of solve.rs:94, starting from best = ((0.0, -inf), [])
+// (solve.rs:82): writes it to (*bs, *br) and returns its index, or -1 when no search beats the start.
+static int best_of(const uint8_t* success, const float* total, int64_t S, float* bs, float* br) {
+    int best = -1;
+    *bs = 0.0f; *br = -INFINITY;
+    for (int64_t i = 0; i < S; ++i) {
+        const float s1 = success[i] ? 1.0f : 0.0f, r1 = total[i];
+        if (s1 > *bs || (s1 == *bs && r1 > *br)) { *bs = s1; *br = r1; best = (int)i; }
+    }
+    return best;
+}
+
 // Shared driver: B envs already initialised in (cells, meta); runs single_solve (rl/solve.rs:17-71) for all of
 // them in lockstep.  Fills total[B], success[B], n_steps[B] and (optionally) the per-step action record.
-struct MctsOpt { int n_sims; float C; int max_expand_depth; };
-
 static int run_solve(twr_engine* e, const EnvParams& env, const PolicyDev& dev, int64_t B, int T, EnvIds ids, uint32_t cid,
                      int deterministic, MctsOpt mo, uint4* cells, uint32_t* meta, float* total, uint8_t* success, int32_t* n_steps,
                      uint8_t* act_rec) {
@@ -1484,44 +1569,31 @@ static int run_solve(twr_engine* e, const EnvParams& env, const PolicyDev& dev, 
     // num_mcts_searches > 0: every step's action distribution is predict_probs_mcts of the current state
     MctsArgs ma{};
     Staging<float> mcts_probs; Staging<int32_t> mcts_vis, twist_idx;
-    size_t slices = 1;                       // forward output slices of B: one per twist in an MCTS with a twisted policy
-    if (mo.n_sims > 0) {
-        const int P = mcts_pool_nodes(dev.A, mo.n_sims, mo.max_expand_depth);
-        if ((double)B * P >= 2147483647.0) return fail(TWR_ERR_INVALID, "MCTS node pool too large");
-        ma.pool.A = dev.A;
-        if ((rc = mcts_acquire(e, B, P, &ma.pool, &ma)) || (rc = mcts_probs.alloc((size_t)B * dev.A)) || (rc = mcts_vis.alloc((size_t)B * dev.A)) ||
-            (rc = stage_twists(e, dev, B, &twist_idx, &ma))) return rc;
-        if (dev.n_perms > 0) slices = (size_t)dev.n_perms;
-    }
+    const bool search = mo.n_sims > 0;
+    if (search && ((rc = mcts_reserve(e, dev, B, mo, &twist_idx, &ma)) || (rc = mcts_probs.alloc((size_t)B * dev.A)) ||
+                   (rc = mcts_vis.alloc((size_t)B * dev.A)))) return rc;
+    const size_t slices = search ? forward_slices(dev) : 1;
     if ((rc = live_a.alloc((size_t)B)) || (rc = live_b.alloc((size_t)B)) || (rc = n_live.alloc((size_t)T + 2)) ||
         (rc = logits.alloc(slices * (size_t)B)) || (rc = values.alloc(slices * (size_t)B))) return rc;
     cudaStream_t st = e->stream;
-    std::vector<int32_t> iota((size_t)B);
-    for (int64_t i = 0; i < B; ++i) iota[(size_t)i] = (int32_t)i;
-    CU_TRY(cudaMemcpyAsync(live_a.d, iota.data(), sizeof(int32_t) * (size_t)B, cudaMemcpyHostToDevice, st));
     CU_TRY(cudaMemsetAsync(n_live.d, 0, sizeof(int32_t) * (size_t)(T + 2), st));
-    const int32_t b32 = (int32_t)B;
-    CU_TRY(cudaMemcpyAsync(n_live.d, &b32, sizeof(int32_t), cudaMemcpyHostToDevice, st));
+    if ((rc = upload_all_live(e, live_a.d, n_live.d, B))) return rc;
     CU_TRY(cudaMemsetAsync(total, 0, sizeof(float) * (size_t)B, st));
     CU_TRY(cudaMemsetAsync(success, 0, (size_t)B, st));
     CU_TRY(cudaMemsetAsync(n_steps, 0, sizeof(int32_t) * (size_t)B, st));
-    ForwardArgs fa{};
-    fa.env = env; fa.seed = e->seed; fa.cid = cid; fa.ids = ids; fa.cells = cells; fa.n = B;
-    fa.logits = logits.d; fa.values = values.d;
+    ForwardArgs fa = forward_args(e, env, cid, ids, cells, B, logits.d, values.d);
     SolveArgs sa{};
     sa.env = env; sa.seed = e->seed; sa.cid = cid; sa.ids = ids; sa.A = dev.A; sa.deterministic = deterministic; sa.B = B;
     sa.cells = cells; sa.meta = meta; sa.logits = logits.d; sa.n_live = n_live.d; sa.total = total; sa.success = success;
     sa.act_rec = act_rec; sa.n_steps = n_steps;
-    if (mo.n_sims > 0) {
-        ma.env = env; ma.seed = e->seed; ma.cid = cid; ma.ids = ids; ma.n_sims = mo.n_sims;
-        ma.max_expand_depth = mo.max_expand_depth; ma.C = mo.C;
-        ma.env_cells = cells; ma.env_meta = meta; ma.logits = logits.d; ma.values = values.d;
+    if (search) {
+        mcts_target(e, &ma, env, cid, ids, cells, meta, logits.d, values.d);
         sa.mcts_probs = mcts_probs.d;
     }
     for (int t = 0; t <= T; ++t) {          // at most T steps, then the terminal visit
         int32_t* cur = (t & 1) ? live_b.d : live_a.d;
         int32_t* nxt = (t & 1) ? live_a.d : live_b.d;
-        if (mo.n_sims > 0) {
+        if (search) {
             ma.t = t;
             enqueue_mcts(e, dev, ma, cur, n_live.d + t, B, twist_idx.d);
             launch_mcts_read(st, ma, B, mcts_probs.d, mcts_vis.d);
@@ -1531,14 +1603,10 @@ static int run_solve(twr_engine* e, const EnvParams& env, const PolicyDev& dev, 
         }
         sa.t = t;
         launch_solve_step(st, sa, cur, nxt);
-        if (mo.n_sims > 0 && (t & 3) == 3) {     // MCTS steps are expensive: stop once every rollout has ended
-            int32_t left = 0;
-            CU_TRY(cudaMemcpyAsync(&left, n_live.d + t + 1, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-            CU_TRY(cudaStreamSynchronize(st));
-            if (left == 0) break;
-        }
+        bool ended = false;
+        if (search && (t & 3) == 3 && (rc = rollouts_ended(e, n_live.d + t + 1, &ended))) return rc;
+        if (ended) break;
     }
-    CU_TRY(cudaGetLastError());
     FWD_CHECK(e);
     CU_TRY(cudaStreamSynchronize(st));       // staging buffers are freed on return
     return TWR_OK;
@@ -1584,11 +1652,8 @@ int twr_evaluate_episodes(twr_engine* e, const twr_env_spec* spec, const twr_pol
     CU_TRY(cudaMemcpy(h_succ.data(), success.d, (size_t)B, cudaMemcpyDeviceToHost));
     float succ = 0.0f, rew = 0.0f;
     for (int64_t ep = 0; ep < num_episodes; ++ep) {
-        float bs = 0.0f, br = -INFINITY;                       // solve.rs:82: best = ((0.0, -inf), [])
-        for (int sidx = 0; sidx < S; ++sidx) {
-            const float s1 = h_succ[(size_t)(ep * S + sidx)] ? 1.0f : 0.0f, r1 = h_total[(size_t)(ep * S + sidx)];
-            if (s1 > bs || (s1 == bs && r1 > br)) { bs = s1; br = r1; }   // tuple '>' (lexicographic), solve.rs:94
-        }
+        float bs, br;
+        best_of(h_succ.data() + ep * S, h_total.data() + ep * S, S, &bs, &br);
         succ += bs; rew += br;
         if (best_success) best_success[ep] = bs;
         if (best_reward) best_reward[ep] = br;
@@ -1629,12 +1694,7 @@ int twr_solve(twr_engine* e, twr_envs* start, const twr_policy* p, int32_t deter
     CU_TRY(cudaMemcpy(h_total.data(), total.d, sizeof(float) * (size_t)B, cudaMemcpyDeviceToHost));
     CU_TRY(cudaMemcpy(h_succ.data(), succ.d, (size_t)B, cudaMemcpyDeviceToHost));
     CU_TRY(cudaMemcpy(h_n.data(), n_steps.d, sizeof(int32_t) * (size_t)B, cudaMemcpyDeviceToHost));
-    float bs = 0.0f, br = -INFINITY; int best = -1;
-    for (int64_t i = 0; i < B; ++i) {
-        const float s1 = h_succ[(size_t)i] ? 1.0f : 0.0f, r1 = h_total[(size_t)i];
-        if (s1 > bs || (s1 == bs && r1 > br)) { bs = s1; br = r1; best = (int)i; }
-    }
-    *success = bs; *reward = br;
+    const int best = best_of(h_succ.data(), h_total.data(), B, success, reward);
     if (best >= 0) {
         const int n = h_n[(size_t)best];
         *n_actions = n;
@@ -1676,23 +1736,15 @@ static int mcts_probs_impl(twr_engine* e, const twr_policy* p, twr_envs* v, int3
     if (rc) return rc;
     CU_TRY(cudaSetDevice(e->device));
     const int64_t B = v->n;
-    const int P = mcts_pool_nodes(dev.A, n_sims, max_expand_depth);
-    if ((double)B * P >= 2147483647.0) return fail(TWR_ERR_INVALID, "MCTS node pool too large");
-    MctsArgs a{};
-    a.pool.A = dev.A;
-    if ((rc = mcts_acquire(e, B, P, &a.pool, &a))) return rc;
+    MctsArgs a;
     Staging<float4> logits; Staging<float> values, d_probs; Staging<int32_t> live, n_live, d_vis, twist_idx;
-    const size_t slices = dev.n_perms > 0 ? (size_t)dev.n_perms : 1;
-    if ((rc = logits.alloc(slices * (size_t)B)) || (rc = values.alloc(slices * (size_t)B)) || (rc = live.alloc((size_t)B)) || (rc = n_live.alloc(1)) ||
-        (rc = d_probs.alloc((size_t)B * dev.A)) || (rc = d_vis.alloc((size_t)B * dev.A)) || (rc = stage_twists(e, dev, B, &twist_idx, &a))) return rc;
-    std::vector<int32_t> iota((size_t)B);
-    for (int64_t i = 0; i < B; ++i) iota[(size_t)i] = (int32_t)i;
-    const int32_t b32 = (int32_t)B;
-    CU_TRY(cudaMemcpyAsync(live.d, iota.data(), sizeof(int32_t) * (size_t)B, cudaMemcpyHostToDevice, e->stream));
-    CU_TRY(cudaMemcpyAsync(n_live.d, &b32, sizeof(int32_t), cudaMemcpyHostToDevice, e->stream));
-    a.env = v->p; a.seed = e->seed; a.cid = collect_id; a.ids = EnvIds{env_id_base, 0u, 0u, 0u};
-    a.t = t; a.n_sims = n_sims; a.max_expand_depth = max_expand_depth; a.C = C;
-    a.env_cells = v->cells; a.env_meta = v->meta; a.logits = logits.d; a.values = values.d;
+    const size_t slices = forward_slices(dev);
+    if ((rc = mcts_reserve(e, dev, B, MctsOpt{n_sims, C, max_expand_depth}, &twist_idx, &a)) ||
+        (rc = logits.alloc(slices * (size_t)B)) || (rc = values.alloc(slices * (size_t)B)) || (rc = live.alloc((size_t)B)) ||
+        (rc = n_live.alloc(1)) || (rc = d_probs.alloc((size_t)B * dev.A)) || (rc = d_vis.alloc((size_t)B * dev.A))) return rc;
+    if ((rc = upload_all_live(e, live.d, n_live.d, B))) return rc;
+    mcts_target(e, &a, v->p, collect_id, EnvIds{env_id_base, 0u, 0u, 0u}, v->cells, v->meta, logits.d, values.d);
+    a.t = t;
     Staging<int32_t> d_trace;
     const size_t n_trace = (size_t)(n_sims > 0 ? n_sims : 1) * (size_t)B * 2;
     if (trace) {
@@ -1702,7 +1754,6 @@ static int mcts_probs_impl(twr_engine* e, const twr_policy* p, twr_envs* v, int3
     }
     enqueue_mcts(e, dev, a, live.d, n_live.d, B, twist_idx.d);
     launch_mcts_read(e->stream, a, B, d_probs.d, d_vis.d);
-    CU_TRY(cudaGetLastError());
     FWD_CHECK(e);
     if (trace) CU_TRY(cudaMemcpyAsync(trace, d_trace.d, sizeof(int32_t) * (size_t)n_sims * (size_t)B * 2, cudaMemcpyDeviceToHost, e->stream));
     CU_TRY(cudaMemcpyAsync(probs, d_probs.d, sizeof(float) * (size_t)B * dev.A, cudaMemcpyDeviceToHost, e->stream));
@@ -1723,57 +1774,33 @@ int twr_az_collect(twr_engine* e, const twr_env_spec* spec, const twr_policy* p,
     CU_TRY(cudaSetDevice(e->device));
     const int64_t B = num_episodes;
     const int T = plan.T;
-    const int P = mcts_pool_nodes(plan.dev.A, num_mcts_searches, max_expand_depth);
-    if ((double)B * P >= 2147483647.0) return fail(TWR_ERR_INVALID, "MCTS node pool too large (num_episodes * (1 + A*(n_sims*depth+1)) must be < 2^31)");
-    if ((rc = ensure_collect_buffers(e, B, T, plan.env.N, B))) return rc;
-    MctsArgs a{};
-    a.pool.A = plan.dev.A;
-    if ((rc = mcts_acquire(e, B, P, &a.pool, &a))) return rc;
+    MctsArgs a;
+    Staging<int32_t> no_twists;                 // stays empty: twists are refused above
+    if ((rc = mcts_reserve(e, plan.dev, B, MctsOpt{num_mcts_searches, C, max_expand_depth}, &no_twists, &a)) ||
+        (rc = ensure_collect_buffers(e, B, T, plan.env.N, B))) return rc;
     CollectBuffers& b = e->buf;
     cudaStream_t st = e->stream;
     e->has_last = false;
-    b.B = B;
     b.obs_u8 = 0;
-    select_outset(e, 0);
     const uint32_t cid = e->collect_id++;
     const EnvIds ids{(uint32_t)((int64_t)e->rank * B), (uint32_t)(B - 1), (uint32_t)B, 0u};
-    CU_TRY(cudaMemsetAsync(b.n_live, 0, sizeof(int32_t) * (size_t)(T + 1), st));
-    CU_TRY(cudaMemsetAsync(b.stats, 0, sizeof(unsigned long long) * 4, st));
-    launch_envs_reset(st, plan.env, b.cells, b.meta, B, e->seed, ids, cid, b.live_a, b.n_live);
-    a.env = plan.env; a.seed = e->seed; a.cid = cid; a.ids = ids; a.n_sims = num_mcts_searches;
-    a.max_expand_depth = max_expand_depth; a.C = C;
-    a.env_cells = b.cells; a.env_meta = b.meta; a.logits = b.logits; a.values = b.values;
+    if ((rc = begin_collect(e, plan.env, B, ids, cid, 0))) return rc;
+    mcts_target(e, &a, plan.env, cid, ids, b.cells, b.meta, b.logits, b.values);
     for (int t = 0; t < T; ++t) {
         int32_t* cur = (t & 1) ? b.live_b : b.live_a;
         int32_t* nxt = (t & 1) ? b.live_a : b.live_b;
         a.t = t;
         enqueue_mcts(e, plan.dev, a, cur, b.n_live + t, B, nullptr);
         launch_az_finish(st, a, b, cur, nxt);
-        if ((t & 7) == 7) {                      // stop early once every episode has ended (MCTS steps are expensive)
-            int32_t left = 0;
-            CU_TRY(cudaMemcpyAsync(&left, b.n_live + t + 1, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-            CU_TRY(cudaStreamSynchronize(st));
-            if (left == 0) break;
-        }
+        bool ended = false;
+        if ((t & 7) == 7 && (rc = rollouts_ended(e, b.n_live + t + 1, &ended))) return rc;
+        if (ended) break;
     }
     launch_az_remaining(st, b);
     launch_episode_offsets(st, b, ids);
     launch_compact(st, plan.env, b, plan.dev.A);
-    CU_TRY(cudaGetLastError());
     FWD_CHECK(e);
-    launch_publish_stats(st, b.stats, e->d_hstats);
-    CU_TRY(cudaStreamSynchronize(st));
-    twr_collected& c = e->last;
-    c.n_records = (int64_t)e->h_stats[1];
-    c.num_episodes = num_episodes;
-    c.n_cells = plan.env.N; c.num_actions = plan.dev.A;
-    c.successes = (int64_t)e->h_stats[0];
-    double rs; memcpy(&rs, &e->h_stats[2], sizeof(double)); c.reward_sum = rs;
-    c.obs = b.out_obs; c.logits = b.out_logits; c.values = b.out_values; c.rewards = b.out_rewards;
-    c.advs = b.out_advs; c.rets = b.out_rets; c.actions = b.out_actions; c.perms = b.out_perms; c.ep_len = e->ep_len_id;
-    e->has_last = true;
-    *out = c;
-    return TWR_OK;
+    return finish_collect(e, plan, num_episodes, out);
     });
 }
 

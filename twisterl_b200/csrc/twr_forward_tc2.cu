@@ -459,7 +459,7 @@ k_forward_tc2(PolicyDev p, ForwardArgs a, Tc2Params t, const __grid_constant__ C
     const uint32_t D2_COL = 0, D1_COL = 256;
     const bool timed = a.dbg != nullptr;
     // event trace of CTA 0 (first 8 items, 32 slots each) behind the per-CTA counters: clock64 stamps
-    long long* trace = (timed && blockIdx.x == 0) ? a.dbg + 148 * 16 : nullptr;
+    long long* trace = (timed && blockIdx.x == 0) ? a.dbg + TWR_DBG_TRACE : nullptr;
     auto stamp = [&](int item, int ev) { if (trace && item < 8) trace[item * 32 + ev] = clock64(); };
 
     if (warp == 0) {

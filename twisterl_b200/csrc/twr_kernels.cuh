@@ -125,8 +125,13 @@ struct ForwardArgs {
     // | bit 1 h1_lo x W_hi | bit 2 h1_hi x W_lo on top of the hi x hi products (TWR_PREC_F16X2_W16 = 8 | 1 | 2)
     int tc_terms;
     int dbg_flags;    // ablations (k_forward_tc2, timing only): 1 skip epilogue-1 TMEM traffic, 2 no operand TMA traffic, 4 skip GEMM2 MMAs, 8 skip GEMM1 MMAs
-    long long* dbg;   // optional [gridDim][16] cycle counters written by k_forward_tc2 (debug/profiling)
+    long long* dbg;   // optional [gridDim][16] cycle counters written by k_forward_tc2 (debug/profiling), TWR_DBG_WORDS long
 };
+// ForwardArgs::dbg: 16 counters for each of up to TWR_DBG_CTAS CTAs (one per SM of a B200), then at TWR_DBG_TRACE the
+// event trace of CTA 0 (8 items x 32 clock64 stamps)
+#define TWR_DBG_CTAS 148
+#define TWR_DBG_TRACE (TWR_DBG_CTAS * 16)
+#define TWR_DBG_WORDS (TWR_DBG_TRACE + 256)
 int  forward_fp32_supported(const PolicyDev& p, const EnvParams& env, const char** why);
 bool launch_forward_fp32(cudaStream_t s, const PolicyDev& p, const ForwardArgs& a);   // false: shape does not fit shared memory
 // Tensor-core (CTA-pair, tcgen05 cta_group::2) variant, twr_forward_tc2.cu; `pack` is its operand image (PolicyDev::tc_pack)
