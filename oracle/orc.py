@@ -348,19 +348,24 @@ def mcts_probs(env: Env, policy: Policy, n_sims, c_puct, max_expand_depth, seed=
     return probs, visits
 
 
-def mcts_trace(env: Env, policy: Policy, n_sims, c_puct, max_expand_depth, seed=0, collect_id=0, stream_id=0, t=0):
-    """mcts_probs plus the per-simulation trace: (probs, visits, leaf[n_sims], backed_up_node[n_sims], margin[n_sims])."""
+def mcts_trace(env: Env, policy: Policy, n_sims, c_puct, max_expand_depth, seed=0, collect_id=0, stream_id=0, t=0,
+               path_lengths=False):
+    """mcts_probs plus the per-simulation trace: (probs, visits, leaf[n_sims], backed_up_node[n_sims], margin[n_sims]),
+    with path_lengths=True also path_len[n_sims], the number of nodes each simulation's backup updated (root and
+    backed-up node included)."""
     probs = np.zeros(policy.num_actions, dtype=np.float32)
     visits = np.zeros(policy.num_actions, dtype=np.int32)
     leaf = np.zeros(max(n_sims, 1), dtype=np.int32); child = np.zeros(max(n_sims, 1), dtype=np.int32)
-    margin = np.zeros(max(n_sims, 1), dtype=np.float32)
+    margin = np.zeros(max(n_sims, 1), dtype=np.float32); path_len = np.zeros(max(n_sims, 1), dtype=np.int32)
     f = lib().orc_mcts_trace
     f.argtypes = [C.POINTER(_Env), C.c_void_p, C.c_int32, C.c_float, C.c_int32, C.c_uint64, C.c_uint32, C.c_uint32, C.c_int32,
-                  C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+                  C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
     f.restype = None
     f(C.byref(env._e), policy._h, int(n_sims), float(c_puct), int(max_expand_depth), int(seed), int(collect_id),
-      int(stream_id), int(t), probs.ctypes.data, visits.ctypes.data, leaf.ctypes.data, child.ctypes.data, margin.ctypes.data)
-    return probs, visits, leaf[:n_sims], child[:n_sims], margin[:n_sims]
+      int(stream_id), int(t), probs.ctypes.data, visits.ctypes.data, leaf.ctypes.data, child.ctypes.data, margin.ctypes.data,
+      path_len.ctypes.data)
+    out = (probs, visits, leaf[:n_sims], child[:n_sims], margin[:n_sims])
+    return out + (path_len[:n_sims],) if path_lengths else out
 
 
 def az_collect(spec: EnvSpec, policy: Policy, num_episodes, n_sims, c_puct, max_expand_depth, seed=0, collect_id=0,

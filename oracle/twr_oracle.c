@@ -857,11 +857,12 @@ static float weighted_margin(const float* w, int n, float u) {
 /* search.rs:104-189.  Optional per-simulation trace (test infrastructure): the leaf the UCB descent of simulation s
  * ended on, the node its value was backed up from (the sampled child, or the leaf itself when it was terminal), and the
  * smallest decision margin of that simulation -- best minus second-best UCB over the levels of the descent and the
- * bin-edge distance of the child draw.  Node indices count expansions in order, so two implementations that made the
- * same decisions so far agree on them. */
+ * bin-edge distance of the child draw -- and the number of nodes its backup updated (the root and the backed-up node
+ * included).  Node indices count expansions in order, so two implementations that made the same decisions so far agree
+ * on them. */
 static void mcts_core(const orc_env* env, const orc_policy* p, int32_t n_sims, float C, int32_t max_expand_depth,
                       uint64_t seed, uint32_t collect_id, uint32_t stream_id, int32_t t_step, float* probs, int32_t* visits,
-                      int32_t* trace_leaf, int32_t* trace_child, float* trace_margin) {
+                      int32_t* trace_leaf, int32_t* trace_child, float* trace_margin, int32_t* trace_len) {
     const uint32_t key[2] = {(uint32_t)seed, (uint32_t)(seed >> 32)};
     const int nc = orc_env_num_cells(env), na = orc_env_num_actions(env);
     const int med = max_expand_depth > 1 ? max_expand_depth : 1;
@@ -918,7 +919,9 @@ static void mcts_core(const orc_env* env, const orc_policy* p, int32_t n_sims, f
         if (trace_child) trace_child[sim] = node;
         if (trace_margin) trace_margin[sim] = margin;
         note_margin(margin);
-        for (int b = node; b >= 0; b = tr.nodes[b].parent) { tr.nodes[b].value_sum += v; tr.nodes[b].visits += 1; }
+        int len = 0;
+        for (int b = node; b >= 0; b = tr.nodes[b].parent) { tr.nodes[b].value_sum += v; tr.nodes[b].visits += 1; ++len; }
+        if (trace_len) trace_len[sim] = len;
     }
     float sum = 0.0f;
     for (int a = 0; a < na; ++a) { probs[a] = 0.0f; if (visits) visits[a] = 0; }
@@ -935,13 +938,14 @@ static void mcts_core(const orc_env* env, const orc_policy* p, int32_t n_sims, f
 
 void orc_mcts_probs(const orc_env* env, const orc_policy* p, int32_t n_sims, float C, int32_t max_expand_depth,
                     uint64_t seed, uint32_t collect_id, uint32_t stream_id, int32_t t_step, float* probs, int32_t* visits) {
-    mcts_core(env, p, n_sims, C, max_expand_depth, seed, collect_id, stream_id, t_step, probs, visits, NULL, NULL, NULL);
+    mcts_core(env, p, n_sims, C, max_expand_depth, seed, collect_id, stream_id, t_step, probs, visits, NULL, NULL, NULL, NULL);
 }
 
 void orc_mcts_trace(const orc_env* env, const orc_policy* p, int32_t n_sims, float C, int32_t max_expand_depth,
                     uint64_t seed, uint32_t collect_id, uint32_t stream_id, int32_t t_step, float* probs, int32_t* visits,
-                    int32_t* trace_leaf, int32_t* trace_child, float* trace_margin) {
-    mcts_core(env, p, n_sims, C, max_expand_depth, seed, collect_id, stream_id, t_step, probs, visits, trace_leaf, trace_child, trace_margin);
+                    int32_t* trace_leaf, int32_t* trace_child, float* trace_margin, int32_t* trace_len) {
+    mcts_core(env, p, n_sims, C, max_expand_depth, seed, collect_id, stream_id, t_step, probs, visits, trace_leaf, trace_child, trace_margin,
+              trace_len);
 }
 
 int orc_az_collect(const orc_env_spec* spec, const orc_policy* p, int32_t num_episodes, int32_t n_sims, float C,

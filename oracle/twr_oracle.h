@@ -175,10 +175,11 @@ void orc_evaluate_margins(const orc_env_spec* spec, const orc_policy* p, int32_t
 void orc_mcts_probs(const orc_env* env, const orc_policy* p, int32_t n_sims, float C, int32_t max_expand_depth,
                     uint64_t seed, uint32_t collect_id, uint32_t stream_id, int32_t t, float* probs, int32_t* visits);
 /* same search with a per-simulation trace [n_sims]: the leaf the UCB descent ended on, the node the value was backed up
- * from, and the simulation's smallest decision margin (UCB best - second best; child-draw distance to a bin edge) */
+ * from, the simulation's smallest decision margin (UCB best - second best; child-draw distance to a bin edge) and the
+ * length of its backup path (nodes from the root to the backed-up node, both included).  Any trace pointer may be NULL. */
 void orc_mcts_trace(const orc_env* env, const orc_policy* p, int32_t n_sims, float C, int32_t max_expand_depth,
                     uint64_t seed, uint32_t collect_id, uint32_t stream_id, int32_t t, float* probs, int32_t* visits,
-                    int32_t* trace_leaf, int32_t* trace_child, float* trace_margin);
+                    int32_t* trace_leaf, int32_t* trace_child, float* trace_margin, int32_t* trace_len);
 typedef struct {
     int64_t n_records; int32_t num_episodes, n_cells, num_actions;
     int32_t* ep_len; int32_t* obs; float* probs; float* rewards; int32_t* actions; float* remaining_values;

@@ -95,3 +95,34 @@ def test_trace_and_margin_instrumentation_leave_results_unchanged():
         bs2, bt2, mm = orc.evaluate_margins(spec, pol, 12, det, 2, seed=9, collect_id=2, num_mcts_searches=mcts)
         assert np.array_equal(bs, bs2) and np.array_equal(bt, bt2)
         assert (mm >= 0).all() and np.isfinite(mm).any()
+
+
+def test_trace_reports_backup_path_lengths_of_a_known_chain():
+    """A policy whose logits are its action biases alone (all weights zero): the prior is one-hot, up to e^-20, on the
+    first legal move in the order left, up, right, down, and the value is 0.  Every simulation then descends the one chain
+    to its end, expands it and backs up from the new child, so simulation s updates s + 3 nodes (root, s + 1 chain nodes,
+    the child) until the chain meets the depth-budget terminal at depth D, whose backups update D + 1 nodes."""
+    D, E, H = 120, 16, 16
+    sd = synth_state_dict(1, 256, E, H, 4)
+    sd = {k: np.zeros_like(v) for k, v in sd.items()}
+    sd["action.0.bias"] = np.array([60.0, 40.0, 20.0, 0.0], np.float32)
+    pol = orc.Policy.from_torch_state_dict(sd)
+    spec = orc.puzzle_spec(4, 4, 5, 2, D)               # set_state gives the board D moves
+    start = list(range(1, 16)) + [0]                     # blank bottom right: left x3, up x3, then right / left forever
+    env = orc.Env(spec); env.set_state(start)
+    chain = []
+    for _ in range(D):
+        m = env.masks()
+        chain.append(next(a for a in range(4) if m[a]))
+        env.step(chain[-1])
+        assert not env.success()
+    assert chain[:8] == [0, 0, 0, 1, 1, 1, 2, 0] and env.is_final()
+    env = orc.Env(spec); env.set_state(start)
+    probs, visits, leaf, child, margin, plen = orc.mcts_trace(env, pol, D + 4, 1.41, 1, seed=3, collect_id=1, stream_id=5,
+                                                              path_lengths=True)
+    assert all(np.array_equal(x, y) for x, y in zip((probs, visits, leaf, child, margin),
+                                                     orc.mcts_trace(env, pol, D + 4, 1.41, 1, seed=3, collect_id=1, stream_id=5)))
+    assert plen.tolist()[:D] == list(range(3, D + 2)) + [D + 1]
+    assert leaf[D - 1] == child[D - 1]                  # the terminal leaf backs up its own reward
+    assert visits.tolist() == [D + 4, 0, 0, 0]          # blank bottom right: left (0) and up (1) are the legal moves
+    assert plen.max() == D + 1 > 96                     # deeper than the device's recorded descent path (TWR_MCTS_PATH)
