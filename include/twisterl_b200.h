@@ -324,6 +324,20 @@ int  twr_broadcast_weights(twr_engine* e, twr_policy* p, int32_t root);
 /* in-place all-reduce of n <= TWR_COMM_MAX_STATS host doubles (episodes, successes, reward sum, records, ...);
  * returns after the reduced values are in `stats`.  world == 1: no-op. */
 int  twr_allreduce_stats(twr_engine* e, double* stats, int32_t n, int32_t op /* twr_reduce_op */);
+/* Collective over the `world` engines: every rank has just finished a device-resident collect (twr_ppo_collect or
+ * twr_az_collect) of the same shape; rank `root` receives all of them, merged in the order ONE collect of
+ * world * num_episodes episodes lays out ([last, 0, 1, ..., n-2], collector/collector.rs:40-46).  On root `out` (and what
+ * twr_collected_to_host / the next twr_collected query return) describes the merged result; on the other ranks `out` is
+ * their own result, unchanged.  world == 1: returns the local result, needs no communicator.
+ * Every rank first all-gathers a small header and reaches the same verdict before any record moves: TWR_ERR_STATE on every
+ * rank when one holds no device-resident result (a failed or missing collect, a pipelined twr_ppo_collect_host of several
+ * sub-batches, a root that already holds a gathered result), TWR_ERR_INVALID when the ranks' env specs, shapes,
+ * num_episodes, seeds, precisions, collect ids or roots differ.  The merged buffers are engine-owned (grow-only) and stay
+ * valid until the next gather or destroy; NCCL p2p sends / receives carry the records on the engine stream, and the call
+ * returns once root's result is complete.  TWR_ERR_UNSUPPORTED when libnccl lacks ncclSend / ncclRecv / ncclAllGather.
+ * A rank's local failure before the exchange travels in its header and is returned by every rank; a CUDA or NCCL failure
+ * inside the collectives themselves can, as with any NCCL collective, leave the peers waiting. */
+int  twr_gather_collected(twr_engine* e, int32_t root, twr_collected* out);
 
 /* Parity API: twr_mcts_probs plus, per env and simulation, the leaf the UCB descent ended on and the node the value was
  * backed up from, as tree-local node indices in expansion order: trace [n_sims][n][2].  tests/ use it to find the first

@@ -49,7 +49,7 @@ inline twr_env_spec GridWorld(int width, int height, int max_steps, int difficul
 class Engine {
 public:
     explicit Engine(int device = 0, twr_precision precision = TWR_PREC_F16X2, uint64_t seed = 0x5EED5EEDull, int rank = 0,
-                    int world = 1, void* stream = nullptr) {
+                    int world = 1, void* stream = nullptr) : rank_(rank) {
         twr_engine_cfg cfg{device, (int32_t)precision, seed, rank, world, stream};
         check(twr_engine_create(&cfg, &h_));
     }
@@ -57,6 +57,7 @@ public:
     Engine(const Engine&) = delete;
     Engine& operator=(const Engine&) = delete;
     twr_engine* handle() const { return h_; }
+    int rank() const { return rank_; }
     void synchronize() { check(twr_engine_synchronize(h_)); }
     void set_collect_id(uint32_t id) { check(twr_engine_set_collect_id(h_, id)); }   // pins the Philox streams of the next collect
     int64_t launch_count() const { return twr_engine_launch_count(h_); }
@@ -75,6 +76,7 @@ public:
 
 private:
     twr_engine* h_ = nullptr;
+    int rank_ = 0;
 };
 
 // ------------------------------------------------------------------------------------------------ nn ---
@@ -278,6 +280,44 @@ public:
         return d;
     }
 };
+
+// Collective over the ranks, each of which has just run a device-resident collect (twr_ppo_collect / twr_az_collect) of
+// the same shape: rank `root` receives every rank's episodes, merged in the order ONE collect of all of them lays out
+// (twr_gather_collected), as CollectedData shaped like PPOCollector::collect's, or with `az` like AZCollector::collect's
+// (MCTS distributions in `logits`, additional_data["remaining_values"], perms None, no values / rewards / actions).
+// The other ranks get an empty CollectedData.
+inline CollectedData gather_collected(Engine& eng, int root = 0, bool az = false) {
+    twr_collected c{};
+    check(twr_gather_collected(eng.handle(), root, &c));
+    CollectedData d;
+    if (eng.rank() != root) return d;
+    const size_t R = (size_t)c.n_records, n = (size_t)c.n_cells, A = (size_t)c.num_actions, E = (size_t)c.num_episodes;
+    std::vector<uint16_t> obs(R * n + 1);
+    std::vector<float> logits(R * A + 1), values(R + 1), rewards(R + 1), advs(R + 1), rets(R + 1);
+    std::vector<uint8_t> actions(R + 1);
+    std::vector<int8_t> perms(R + 1);
+    d.ep_len.resize(E);
+    twr_host_buffers dst{(int64_t)R, obs.data(), logits.data(), values.data(), rewards.data(), advs.data(), rets.data(),
+                         actions.data(), perms.data(), d.ep_len.data(), nullptr};
+    check(twr_collected_to_host(eng.handle(), &dst));
+    d.obs.resize(R); d.logits.resize(R); d.perms.resize(R);
+    for (size_t r = 0; r < R; ++r) {
+        d.obs[r].assign(obs.begin() + r * n, obs.begin() + (r + 1) * n);
+        d.logits[r].assign(logits.begin() + r * A, logits.begin() + (r + 1) * A);
+        d.perms[r] = az || perms[r] < 0 ? std::nullopt : std::optional<size_t>((size_t)perms[r]);
+    }
+    d.successes = c.successes; d.reward_sum = c.reward_sum;
+    if (az) {                                                             // az.rs:97-104, as AZCollector::collect
+        d.additional_data["remaining_values"].assign(rets.begin(), rets.begin() + R);
+        return d;
+    }
+    d.values.assign(values.begin(), values.begin() + R);
+    d.rewards.assign(rewards.begin(), rewards.begin() + R);
+    d.actions.assign(actions.begin(), actions.begin() + R);
+    d.additional_data["advs"].assign(advs.begin(), advs.begin() + R);
+    d.additional_data["rets"].assign(rets.begin(), rets.begin() + R);
+    return d;
+}
 
 // A batch of envs of one spec on the device (the parity API of the C header): reset / set_state / step / queries
 class Envs {

@@ -34,7 +34,7 @@ def install_as_twisterl() -> types.ModuleType:
     return mod
 
 
-def accelerate(algorithm):
+def accelerate(algorithm, comm=None):
     """Opt-in fast paths for a reference `twisterl.rl` Algorithm object that already runs on this engine (SURVEY.md 8f
     rows f2 / f3).  The reference's source stays untouched; three of the INSTANCE's methods are replaced:
 
@@ -43,6 +43,11 @@ def accelerate(algorithm):
     * `collect` + `data_to_torch` (rl/algorithm.py:101-104, rl/ppo.py:25-61; PPO only): the collect stays on the device
       (`PPOCollector.collect_torch`) and the training tensors are built there -- same tuple, same arithmetic
       (advantage normalisation, Categorical log-probs of the recorded masked logits) as the reference's data_to_torch.
+
+    With a `dist.Comm` (on the root rank), `collect` runs on every rank's GPU: `algorithm.collector.num_episodes`
+    is the total, sharded over the ranks and gathered to this one (`dist.ShardedCollector`, kept as
+    `algorithm.sharded_collector`; its `close()` stops the other ranks, which run its `serve`).  PPO collects through
+    `collect_torch`, AZ through `collect`.
 
     Returns the algorithm."""
     import time
@@ -62,9 +67,13 @@ def accelerate(algorithm):
             self.rs_pol = self.policy.to_rust()
 
     algorithm.sync_rs_policy = types.MethodType(timed(sync_rs_policy), algorithm)
+    sharded = None
+    if comm is not None:
+        from .dist import ShardedCollector
+        sharded = algorithm.sharded_collector = ShardedCollector(algorithm.collector, comm)
     if isinstance(getattr(algorithm, "collector", None), collector.PPOCollector):
         def collect(self):
-            return self.collector.collect_torch(self.env, self.rs_pol, dense_obs=True)
+            return (sharded or self.collector).collect_torch(self.env, self.rs_pol, dense_obs=True)
 
         def data_to_torch(self, data):
             import torch
@@ -77,4 +86,9 @@ def accelerate(algorithm):
 
         algorithm.collect = types.MethodType(timed(collect), algorithm)
         algorithm.data_to_torch = types.MethodType(timed(data_to_torch), algorithm)
+    elif sharded is not None:
+        def collect(self):
+            return sharded.collect(self.env, self.rs_pol)
+
+        algorithm.collect = types.MethodType(timed(collect), algorithm)
     return algorithm

@@ -74,7 +74,7 @@ SYMBOLS = [
     "twr_envs_step", "twr_envs_get_state", "twr_envs_observe", "twr_envs_masks", "twr_envs_reward",
     "twr_envs_is_final", "twr_envs_success", "twr_envs_depth", "twr_policy_forward", "twr_policy_forward_obs", "twr_policy_full_predict", "twr_debug_forward_profile", "twr_debug_set_tc_terms", "twr_sample", "twr_gae",
     "twr_ppo_collect", "twr_engine_set_collect_id", "twr_collected_to_host", "twr_max_records",
-    "twr_ppo_collect_host", "twr_evaluate", "twr_evaluate_episodes", "twr_solve", "twr_az_collect", "twr_mcts_probs", "twr_debug_mcts_trace", "twr_comm_version", "twr_comm_unique_id", "twr_comm_init", "twr_comm_destroy", "twr_broadcast_weights", "twr_allreduce_stats",
+    "twr_ppo_collect_host", "twr_evaluate", "twr_evaluate_episodes", "twr_solve", "twr_az_collect", "twr_mcts_probs", "twr_debug_mcts_trace", "twr_comm_version", "twr_comm_unique_id", "twr_comm_init", "twr_comm_destroy", "twr_broadcast_weights", "twr_allreduce_stats", "twr_gather_collected",
     "twr_host_alloc", "twr_host_free", "twr_engine_set_timing", "twr_engine_last_timing",
 ]
 
@@ -154,6 +154,7 @@ def load():
         L.twr_comm_destroy.argtypes = [vp]; L.twr_comm_destroy.restype = None
         L.twr_broadcast_weights.argtypes = [vp, vp, C.c_int32]
         L.twr_allreduce_stats.argtypes = [vp, vp, C.c_int32, C.c_int32]
+        L.twr_gather_collected.argtypes = [vp, C.c_int32, C.POINTER(Collected)]
         L.twr_debug_mcts_trace.argtypes = [vp, vp, vp, C.c_int32, C.c_float, C.c_int32, C.c_uint32, C.c_uint32, C.c_int32, vp, vp, vp]
         L.twr_host_alloc.argtypes = [C.POINTER(vp), C.c_int64]
         L.twr_host_free.argtypes = [vp]; L.twr_host_free.restype = None

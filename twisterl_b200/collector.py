@@ -109,6 +109,34 @@ def _host_buffers(cap: int, n_cells: int, n_actions: int, num_episodes: int, pin
     return hb, arrays, holders
 
 
+def torch_views(c: _lib.Collected, device: int, dense_obs: bool = True) -> dict:
+    """Torch CUDA tensors over the device-resident result `c` describes (a collect, or root's gathered result of
+    twr_gather_collected), aliasing the engine's buffers: valid until the next collect / gather on that engine.
+    Keys: obs (dense one-hot float [R, obs_size] or int64 indices [R, cells]), logits, actions, advs, rets, perms,
+    values, rewards, stats."""
+    import torch
+    R, N, A = int(c.n_records), int(c.n_cells), int(c.num_actions)
+    dev = torch.device("cuda", int(device))
+
+    def view(ptr, shape, typestr):
+        class _H:
+            __cuda_array_interface__ = {"shape": shape, "typestr": typestr, "data": (int(ptr), False), "version": 2}
+        return torch.as_tensor(_H(), device=dev)
+
+    idx = view(c.obs, (R, N), "<u2").to(torch.int64)
+    out = {"logits": view(c.logits, (R, A), "<f4"), "values": view(c.values, (R,), "<f4"),
+           "rewards": view(c.rewards, (R,), "<f4"), "advs": view(c.advs, (R,), "<f4"), "rets": view(c.rets, (R,), "<f4"),
+           "actions": view(c.actions, (R,), "|u1").to(torch.int64), "perms": view(c.perms, (R,), "|i1").to(torch.int64)}
+    if dense_obs:
+        obs = torch.zeros((R, N * N), dtype=torch.float32, device=dev)
+        obs.scatter_(1, idx, 1.0)
+        out["obs"] = obs
+    else:
+        out["obs"] = idx
+    out["stats"] = dict(episodes=int(c.num_episodes), successes=int(c.successes), reward_sum=float(c.reward_sum), records=R)
+    return out
+
+
 class PyBaseCollector:
     """`collector.PyBaseCollector` (python_interface/collector.rs:139-152)."""
 
@@ -163,35 +191,16 @@ class PPOCollector(PyBaseCollector):
         """Device hand-off for a GPU trainer (SURVEY.md 8f row f2): run the collect and return torch CUDA tensors that
         alias the engine's output buffers (valid until the next collect on this engine) -- what
         `PPO.data_to_torch` (src/twisterl/rl/ppo.py:25-61) builds through Python lists and an H2D copy.
-        Keys: obs (dense one-hot float [R, obs_size] or int64 indices [R, cells]), logits, actions, advs, rets, perms,
-        values, rewards."""
-        import torch
-        c = self.collect_device(env, policy)
-        R, N, A = int(c.n_records), int(c.n_cells), int(c.num_actions)
-        dev = torch.device("cuda", self.engine.device)
-
-        def view(ptr, shape, typestr):
-            class _H:
-                __cuda_array_interface__ = {"shape": shape, "typestr": typestr, "data": (int(ptr), False), "version": 2}
-            return torch.as_tensor(_H(), device=dev)
-
-        idx = view(c.obs, (R, N), "<u2").to(torch.int64)
-        out = {"logits": view(c.logits, (R, A), "<f4"), "values": view(c.values, (R,), "<f4"),
-               "rewards": view(c.rewards, (R,), "<f4"), "advs": view(c.advs, (R,), "<f4"), "rets": view(c.rets, (R,), "<f4"),
-               "actions": view(c.actions, (R,), "|u1").to(torch.int64), "perms": view(c.perms, (R,), "|i1").to(torch.int64)}
-        if dense_obs:
-            obs = torch.zeros((R, N * N), dtype=torch.float32, device=dev)
-            obs.scatter_(1, idx, 1.0)
-            out["obs"] = obs
-        else:
-            out["obs"] = idx
-        out["stats"] = dict(episodes=int(c.num_episodes), successes=int(c.successes), reward_sum=float(c.reward_sum), records=R)
-        return out
+        Keys: see `torch_views`."""
+        return torch_views(self.collect_device(env, policy), self.engine.device, dense_obs)
 
     def collect(self, env, policy: Policy) -> CollectedData:
         if not isinstance(policy, Policy):
             raise TypeError("argument 'policy': expected twisterl.nn.Policy")
-        c = self.collect_device(env, policy)
+        return self.to_host(self.collect_device(env, policy))
+
+    def to_host(self, c: _lib.Collected) -> CollectedData:
+        """CollectedData of the engine's last device-resident result, which `c` describes (twr_collected_to_host)."""
         eng = self.engine
         R = int(c.n_records)
         hb, arr, holders = _host_buffers(R, c.n_cells, c.num_actions, int(c.num_episodes), self.pinned)
@@ -232,7 +241,10 @@ class AZCollector(PyBaseCollector):
         return c
 
     def collect(self, env, policy: Policy) -> CollectedData:
-        c = self.collect_device(env, policy)
+        return self.to_host(self.collect_device(env, policy))
+
+    def to_host(self, c: _lib.Collected) -> CollectedData:
+        """CollectedData of the engine's last device-resident result, which `c` describes (twr_collected_to_host)."""
         eng = self.engine
         R = int(c.n_records)
         hb, arr, holders = _host_buffers(R, c.n_cells, c.num_actions, int(c.num_episodes), False)

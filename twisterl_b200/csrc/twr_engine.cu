@@ -213,6 +213,11 @@ static void mcts_release(twr_engine* e) {
     c.cap_nodes = 0; c.cap_B = 0;
 }
 
+static void free_outset(twr_engine::OutSet& o) {
+    dev_free(o.obs); dev_free(o.logits); dev_free(o.values); dev_free(o.rewards);
+    dev_free(o.advs); dev_free(o.rets); dev_free(o.actions); dev_free(o.perms);
+}
+
 static void free_collect_buffers(twr_engine* e) {
     CollectBuffers& b = e->buf;
     dev_free(b.cells); dev_free(b.meta); dev_free(b.live_a); dev_free(b.live_b); dev_free(b.n_live);
@@ -220,10 +225,7 @@ static void free_collect_buffers(twr_engine* e) {
     dev_free(b.rec_state); dev_free(b.rec_logits); dev_free(b.rec_value); dev_free(b.rec_reward);
     dev_free(b.rec_adv); dev_free(b.rec_ret); dev_free(b.rec_action); dev_free(b.rec_perm);
     dev_free(b.ep_len); dev_free(b.ep_off); dev_free(b.stats);
-    for (auto& o : e->outs) {
-        dev_free(o.obs); dev_free(o.logits); dev_free(o.values); dev_free(o.rewards);
-        dev_free(o.advs); dev_free(o.rets); dev_free(o.actions); dev_free(o.perms);
-    }
+    for (auto& o : e->outs) free_outset(o);
     e->cap_B = 0; e->cap_T = 0; e->cap_R = 0; e->cap_cells = 0;
 }
 
@@ -235,6 +237,8 @@ void twr_engine_destroy(twr_engine* e) {
     mcts_release(e);
     if (e->trace_buf) { cudaFree(e->trace_buf); e->trace_buf = nullptr; }
     free_collect_buffers(e);
+    free_outset(e->merged);
+    dev_free(e->merged_ep_len);
     for (auto ev : e->ev) cudaEventDestroy(ev);
     dev_free(e->ep_len_id);
     for (int i = 0; i < 2; ++i) if (e->ev_done[i]) cudaEventDestroy(e->ev_done[i]);
@@ -903,6 +907,14 @@ static void select_outset(twr_engine* e, int which) {
     b.out_advs = o.advs; b.out_rets = o.rets; b.out_actions = o.actions; b.out_perms = o.perms;
 }
 
+static int alloc_outset(twr_engine::OutSet* o, size_t R, int cells) {
+    int rc;
+    if ((rc = dev_alloc(&o->obs, R * cells)) || (rc = dev_alloc(&o->logits, R * TWR_MAX_ACTIONS)) ||
+        (rc = dev_alloc(&o->values, R)) || (rc = dev_alloc(&o->rewards, R)) || (rc = dev_alloc(&o->advs, R)) ||
+        (rc = dev_alloc(&o->rets, R)) || (rc = dev_alloc(&o->actions, R)) || (rc = dev_alloc(&o->perms, R))) return rc;
+    return TWR_OK;
+}
+
 static int ensure_collect_buffers(twr_engine* e, int64_t B, int T, int cells, int64_t total_episodes) {
     if (total_episodes > e->cap_E) {
         CU_TRY(cudaStreamSynchronize(e->stream));
@@ -935,15 +947,30 @@ static int ensure_collect_buffers(twr_engine* e, int64_t B, int T, int cells, in
         return rc;
     }
     for (auto& o : e->outs) {
-        if ((rc = dev_alloc(&o.obs, R * cells)) || (rc = dev_alloc(&o.logits, R * TWR_MAX_ACTIONS)) ||
-            (rc = dev_alloc(&o.values, R)) || (rc = dev_alloc(&o.rewards, R)) || (rc = dev_alloc(&o.advs, R)) ||
-            (rc = dev_alloc(&o.rets, R)) || (rc = dev_alloc(&o.actions, R)) || (rc = dev_alloc(&o.perms, R))) {
+        if ((rc = alloc_outset(&o, R, cells))) {
             free_collect_buffers(e);
             return rc;
         }
     }
     e->cap_B = B; e->cap_T = T; e->cap_R = (int64_t)R; e->cap_cells = cells;
     b.B = B; b.Tmax = T;
+    return TWR_OK;
+}
+
+int twr_ensure_merged_buffers(twr_engine* e, int64_t R, int64_t E, int n_cells) {
+    if (E > e->cap_mE) {
+        dev_free(e->merged_ep_len);
+        e->cap_mE = 0;
+        int rc = dev_alloc(&e->merged_ep_len, (size_t)E);
+        if (rc) return rc;
+        e->cap_mE = E;
+    }
+    if (R <= e->cap_mR && n_cells <= e->cap_mcells) return TWR_OK;
+    free_outset(e->merged);
+    e->cap_mR = 0; e->cap_mcells = 0;
+    int rc = alloc_outset(&e->merged, (size_t)R, n_cells);
+    if (rc) { free_outset(e->merged); return rc; }
+    e->cap_mR = R; e->cap_mcells = n_cells;
     return TWR_OK;
 }
 
@@ -1087,6 +1114,7 @@ struct CollectPlan { EnvParams env; PolicyDev dev; int T; };
 static int plan_collect(twr_engine* e, const twr_env_spec* spec, const twr_policy* p, int64_t num_episodes, CollectPlan* plan) {
     if (!e || !p) return fail(TWR_ERR_INVALID, "NULL argument");
     if (p->eng != e) return fail(TWR_ERR_INVALID, "policy belongs to another engine");
+    e->last_kind = twr_engine::LAST_NONE;     // a collect that fails, even on its arguments, leaves nothing to gather
     // merge() errors on zero chunks (collector/collector.rs:41)
     if (num_episodes <= 0)
         return fail(TWR_ERR_INVALID, "Something went wrong. No data in collected data chunks to merge. ");
@@ -1108,18 +1136,26 @@ static CollectStats read_stats(const twr_engine* e) {
     return s;
 }
 
+// the output set a collect just compacted into, as a twr_collected's device pointers
+static twr_collected outset_view(const CollectBuffers& b) {
+    twr_collected c{};
+    c.obs = b.out_obs; c.logits = b.out_logits; c.values = b.out_values; c.rewards = b.out_rewards;
+    c.advs = b.out_advs; c.rets = b.out_rets; c.actions = b.out_actions; c.perms = b.out_perms;
+    return c;
+}
+
 // the end of a device-resident collect: its statistics to the host, then its result kept for twr_collected_to_host
-static int finish_collect(twr_engine* e, const CollectPlan& plan, int64_t num_episodes, twr_collected* out) {
+static int finish_collect(twr_engine* e, const CollectPlan& plan, int64_t num_episodes, int kind, const twr_env_spec* spec,
+                          uint32_t cid, twr_collected* out) {
     launch_publish_stats(e->stream, e->buf.stats, e->d_hstats);
     CU_TRY(cudaStreamSynchronize(e->stream));
     const CollectStats s = read_stats(e);
-    const CollectBuffers& b = e->buf;
     twr_collected& c = e->last;
+    c = outset_view(e->buf);
     c.n_records = s.n_records; c.num_episodes = num_episodes; c.n_cells = plan.env.N; c.num_actions = plan.dev.A;
-    c.successes = s.successes; c.reward_sum = s.reward_sum;
-    c.obs = b.out_obs; c.logits = b.out_logits; c.values = b.out_values; c.rewards = b.out_rewards;
-    c.advs = b.out_advs; c.rets = b.out_rets; c.actions = b.out_actions; c.perms = b.out_perms; c.ep_len = e->ep_len_id;
+    c.successes = s.successes; c.reward_sum = s.reward_sum; c.ep_len = e->ep_len_id;
     e->has_last = true;
+    e->last_kind = kind; e->last_spec = *spec; e->last_cid = cid;
     *out = c;
     return TWR_OK;
 }
@@ -1155,24 +1191,24 @@ int twr_ppo_collect(twr_engine* e, const twr_env_spec* spec, const twr_policy* p
     int n_fwd = 0;
     if ((rc = enqueue_collect(e, plan.env, plan.dev, num_episodes, ids, cid, gamma, lambda, 0, &n_fwd))) return rc;
     if (e->timing) cudaEventRecord(e->ev_t1, st);
-    if ((rc = finish_collect(e, plan, num_episodes, out))) return rc;
+    if ((rc = finish_collect(e, plan, num_episodes, twr_engine::LAST_PPO, spec, cid, out))) return rc;
     e->note_survival();
     finish_timing(e, n_fwd);
     return TWR_OK;
     });
 }
 
-static int copy_out(twr_engine* e, cudaStream_t st, const twr_host_buffers* dst, int64_t at, size_t R, int n_cells, int A) {
-    const CollectBuffers& b = e->buf;
-    if (dst->obs) CU_TRY(cudaMemcpyAsync(dst->obs + at * n_cells, b.out_obs, sizeof(uint16_t) * R * n_cells, cudaMemcpyDeviceToHost, st));
-    else if (dst->obs_u8) CU_TRY(cudaMemcpyAsync(dst->obs_u8 + at * n_cells, b.out_obs, R * n_cells, cudaMemcpyDeviceToHost, st));
-    if (dst->logits) CU_TRY(cudaMemcpyAsync(dst->logits + at * A, b.out_logits, sizeof(float) * R * A, cudaMemcpyDeviceToHost, st));
-    if (dst->values) CU_TRY(cudaMemcpyAsync(dst->values + at, b.out_values, sizeof(float) * R, cudaMemcpyDeviceToHost, st));
-    if (dst->rewards) CU_TRY(cudaMemcpyAsync(dst->rewards + at, b.out_rewards, sizeof(float) * R, cudaMemcpyDeviceToHost, st));
-    if (dst->advs) CU_TRY(cudaMemcpyAsync(dst->advs + at, b.out_advs, sizeof(float) * R, cudaMemcpyDeviceToHost, st));
-    if (dst->rets) CU_TRY(cudaMemcpyAsync(dst->rets + at, b.out_rets, sizeof(float) * R, cudaMemcpyDeviceToHost, st));
-    if (dst->actions) CU_TRY(cudaMemcpyAsync(dst->actions + at, b.out_actions, R, cudaMemcpyDeviceToHost, st));
-    if (dst->perms) CU_TRY(cudaMemcpyAsync(dst->perms + at, b.out_perms, R, cudaMemcpyDeviceToHost, st));
+// D2H of the R records `src` points at into dst, at record offset `at`
+static int copy_out(cudaStream_t st, const twr_collected& src, const twr_host_buffers* dst, int64_t at, size_t R, int n_cells, int A) {
+    if (dst->obs) CU_TRY(cudaMemcpyAsync(dst->obs + at * n_cells, src.obs, sizeof(uint16_t) * R * n_cells, cudaMemcpyDeviceToHost, st));
+    else if (dst->obs_u8) CU_TRY(cudaMemcpyAsync(dst->obs_u8 + at * n_cells, src.obs, R * n_cells, cudaMemcpyDeviceToHost, st));
+    if (dst->logits) CU_TRY(cudaMemcpyAsync(dst->logits + at * A, src.logits, sizeof(float) * R * A, cudaMemcpyDeviceToHost, st));
+    if (dst->values) CU_TRY(cudaMemcpyAsync(dst->values + at, src.values, sizeof(float) * R, cudaMemcpyDeviceToHost, st));
+    if (dst->rewards) CU_TRY(cudaMemcpyAsync(dst->rewards + at, src.rewards, sizeof(float) * R, cudaMemcpyDeviceToHost, st));
+    if (dst->advs) CU_TRY(cudaMemcpyAsync(dst->advs + at, src.advs, sizeof(float) * R, cudaMemcpyDeviceToHost, st));
+    if (dst->rets) CU_TRY(cudaMemcpyAsync(dst->rets + at, src.rets, sizeof(float) * R, cudaMemcpyDeviceToHost, st));
+    if (dst->actions) CU_TRY(cudaMemcpyAsync(dst->actions + at, src.actions, R, cudaMemcpyDeviceToHost, st));
+    if (dst->perms) CU_TRY(cudaMemcpyAsync(dst->perms + at, src.perms, R, cudaMemcpyDeviceToHost, st));
     return TWR_OK;
 }
 
@@ -1187,7 +1223,7 @@ int twr_collected_to_host(twr_engine* e, const twr_host_buffers* dst) {
         return fail(TWR_ERR_UNSUPPORTED, "obs_u8 is produced by twr_ppo_collect_host only (the device-resident result holds u16 indices)");
     CU_TRY(cudaSetDevice(e->device));
     cudaStream_t st = e->stream;
-    int rc = copy_out(e, st, dst, 0, R, c.n_cells, c.num_actions);
+    int rc = copy_out(st, c, dst, 0, R, c.n_cells, c.num_actions);    // what `last` describes: root's merged result after a gather
     if (rc) return rc;
     if (dst->ep_len) CU_TRY(cudaMemcpyAsync(dst->ep_len, c.ep_len, sizeof(int32_t) * (size_t)c.num_episodes, cudaMemcpyDeviceToHost, st));
     CU_TRY(cudaStreamSynchronize(st));
@@ -1307,17 +1343,18 @@ int twr_ppo_collect_host(twr_engine* e, const twr_env_spec* spec, twr_policy* p,
             reward_sum += s.reward_sum;
             if (at + (int64_t)R > dst->capacity) return fail(TWR_ERR_INVALID, "host buffers too small for the collected records");
             CU_TRY(cudaStreamWaitEvent(e->copy_stream, e->ev_done[which], 0));
+            const twr_collected part = outset_view(e->buf);
             if (pack) {
                 // the 9 bytes per record the host rebuild reads go first, so that it overlaps the bulk (obs, logits) of the
                 // same sub-batch instead of trailing the last copy
                 twr_host_buffers d2{};
                 d2.values = dst->values; d2.rets = dst->rets; d2.actions = dst->actions;
-                if ((r2 = copy_out(e, e->copy_stream, &d2, at, R, plan.env.N, plan.dev.A))) return r2;
+                if ((r2 = copy_out(e->copy_stream, part, &d2, at, R, plan.env.N, plan.dev.A))) return r2;
                 CU_TRY(cudaEventRecord(e->ev_small[k], e->copy_stream));
                 twr_host_buffers d3{};
                 d3.logits = dst->logits; d3.obs = dst->obs; d3.obs_u8 = dst->obs_u8;
-                if ((r2 = copy_out(e, e->copy_stream, &d3, at, R, plan.env.N, plan.dev.A))) return r2;
-            } else if ((r2 = copy_out(e, e->copy_stream, dst, at, R, plan.env.N, plan.dev.A))) return r2;
+                if ((r2 = copy_out(e->copy_stream, part, &d3, at, R, plan.env.N, plan.dev.A))) return r2;
+            } else if ((r2 = copy_out(e->copy_stream, part, dst, at, R, plan.env.N, plan.dev.A))) return r2;
             CU_TRY(cudaEventRecord(e->ev_copied[k], e->copy_stream));
             if (pack) {
                 cudaEvent_t ev = e->ev_small[k];
@@ -1800,7 +1837,7 @@ int twr_az_collect(twr_engine* e, const twr_env_spec* spec, const twr_policy* p,
     launch_episode_offsets(st, b, ids);
     launch_compact(st, plan.env, b, plan.dev.A);
     FWD_CHECK(e);
-    return finish_collect(e, plan, num_episodes, out);
+    return finish_collect(e, plan, num_episodes, twr_engine::LAST_AZ, spec, cid, out);
     });
 }
 

@@ -48,6 +48,17 @@ struct twr_engine {
     unsigned long long* d_hstats = nullptr;  // its device address
     bool has_last = false;
     twr_collected last{};
+    // what `last` holds, and the spec and collect id it was collected with (twr_gather_collected checks that every rank
+    // ran the same collect)
+    enum LastKind { LAST_NONE = 0, LAST_PPO = 1, LAST_AZ = 2, LAST_MERGED = 3 };
+    int last_kind = LAST_NONE;
+    twr_env_spec last_spec{};
+    uint32_t last_cid = 0;
+    // the gathered result on the root rank: engine-owned and grow-only, separate from outs[], which the pipelined host
+    // collect double-buffers
+    OutSet merged;
+    int32_t* merged_ep_len = nullptr;
+    int64_t cap_mR = 0, cap_mE = 0; int cap_mcells = 0;
     // timing
     bool timing = false;
     std::vector<cudaEvent_t> ev;
@@ -56,9 +67,13 @@ struct twr_engine {
     // NCCL plumbing (twr_comm.cu): communicator over the `world` engines of a job, device scratch for the stats reduction
     void* comm = nullptr;
     double* d_stats = nullptr;
+    int64_t* d_gather = nullptr;      // twr_gather_collected: every rank's header (world x TWR_GATHER_HDR words) + root's verdict
     MctsCache mcts;
     long long* trace_buf = nullptr;   // device counters of a traced forward launch (TWISTERL_B200_TRACE)
 };
+
+// root's merged output buffers for R records of n_cells cells over E episodes (twr_engine.cu; grow-only)
+extern "C" int twr_ensure_merged_buffers(twr_engine* e, int64_t R, int64_t E, int n_cells);
 
 struct twr_policy {
     twr_engine* eng = nullptr;

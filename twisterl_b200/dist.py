@@ -1,13 +1,16 @@
 """Multi-GPU plumbing: one process per GPU, independent env shards, replicated weights.
 
 The rollout itself has no exchange step (episodes are independent, SURVEY.md section 8e); per iteration there is one
-broadcast of the flat fp32 weight blob from the trainer rank and one all-reduce of a small statistics vector.  On the
-GPUs both are NCCL calls made by the library itself (`twr_broadcast_weights` / `twr_allreduce_stats` of the C ABI, on the
-engine's stream) -- what a Rust or C++ host would call; `torch.distributed` (gloo, CPU) only carries the 128-byte NCCL
-unique id from rank 0 to the other ranks, and stands in for NCCL in the CPU tests of this host logic.
+broadcast of the flat fp32 weight blob from the trainer rank and one all-reduce of a small statistics vector, and a
+trainer on one rank receives every rank's episodes with one gather (`ShardedCollector`).  On the GPUs these are NCCL
+calls made by the library itself (`twr_broadcast_weights` / `twr_allreduce_stats` / `twr_gather_collected` of the C ABI,
+on the engine's stream) -- what a Rust or C++ host would call; `torch.distributed` (gloo, CPU) only carries the 128-byte
+NCCL unique id from rank 0 to the other ranks and the ShardedCollector's per-iteration command, and stands in for NCCL in
+the CPU tests of this host logic.
 """
 from __future__ import annotations
 
+import copy
 import ctypes as C
 import os
 
@@ -85,6 +88,17 @@ class Comm:
     def allreduce_stats(self, episodes: int, successes: int, reward_sum: float, records: int) -> dict:
         return _stats_dict(self.allreduce([episodes, successes, reward_sum, records]))
 
+    def gather_collected(self, root: int = 0):
+        """twr_gather_collected: collective over the ranks, each of which has just run a device-resident collect of the
+        same shape.  Returns the `_lib.Collected` struct: on `root` the merged result of every rank (in the order one
+        collect of all their episodes lays out), elsewhere the rank's own result.  Needs the engine (NCCL) path."""
+        if self.engine is None:
+            raise RuntimeError("gather_collected needs a Comm over an engine")
+        from . import _lib
+        c = _lib.Collected()
+        _lib.check(_lib.load().twr_gather_collected(self.engine._h, int(root), C.byref(c)))
+        return c
+
     def max_over_ranks(self, x: float) -> float:
         return float(self.allreduce([x], op="max")[0])
 
@@ -98,3 +112,106 @@ class Comm:
             _lib.load().twr_comm_destroy(self.engine._h)
         if self.world > 1 and self._dist.is_initialized():
             self._dist.destroy_process_group()
+
+
+STOP = -1          # ShardedCollector command: the workers leave serve()
+
+
+class ShardedCollector:
+    """A `PPOCollector` / `AZCollector` of `collector.num_episodes` episodes IN TOTAL, sharded over the `comm.world` engines
+    of a job: rank r collects the global episode ids [r*E, (r+1)*E), E = total / world, and rank `root` receives every
+    shard, merged in the order one collect of all of them on one engine lays out -- byte for byte that collect, for the
+    same seed, collect id and precision.
+
+    Root calls `collect` / `collect_torch`; every other rank calls `serve`.  Each iteration root broadcasts one command over
+    the gloo group (its env's difficulty, or STOP, and the collect id), then the weights; every rank pins that collect id
+    on its engine, collects its shard and joins the gather.  The collect ids are this object's own counter, starting at
+    `collect_id` and advancing by one per iteration: whatever else root's engine runs between iterations (an evaluate,
+    a solve) leaves the ranks' Philox streams in step.  A rank whose collect raised still joins the gather, so no rank is
+    left waiting, and re-raises afterwards (the gather fails alike on every rank).  `close()` on root stops the workers."""
+
+    def __init__(self, collector, comm: Comm, root: int = 0, collect_id: int = 0):
+        total = int(collector.num_episodes)
+        if total <= 0 or total % comm.world:
+            raise ValueError(f"ShardedCollector: {total} episodes do not split into {comm.world} equal shards "
+                             "(global episode ids are rank * shard + i)")
+        if not 0 <= int(root) < comm.world:
+            raise ValueError("root out of range")
+        self.comm, self.root = comm, int(root)
+        self.local = copy.copy(collector)
+        self.local.num_episodes = total // comm.world
+        if comm.engine is not None:
+            self.local._engine = comm.engine
+        self.collect_id = int(collect_id)
+        self._stopped = False
+
+    @property
+    def is_root(self) -> bool:
+        return self.comm.rank == self.root
+
+    def _command(self, cmd: int = 0, collect_id: int = 0) -> tuple[int, int]:
+        """Root: sends (`cmd`, `collect_id`) to every rank, `cmd` an env difficulty >= 0 or STOP; other ranks: return
+        the pair root sent."""
+        if self.comm.world == 1:
+            return int(cmd), int(collect_id)
+        import torch
+        t = torch.tensor([int(cmd), int(collect_id)], dtype=torch.int64)
+        self.comm._dist.broadcast(t, src=self.root)
+        return int(t[0]), int(t[1])
+
+    def _iteration(self, env, policy, difficulty: int, collect_id: int):
+        env.difficulty = difficulty
+        eng = self.comm.engine
+        self.comm.broadcast_weights(policy.device_handle(eng), root=self.root)
+        eng.set_collect_id(collect_id)
+        err = None
+        try:
+            self.local.collect_device(env, policy)
+        except Exception as exc:
+            err = exc
+        try:
+            c = self.comm.gather_collected(self.root)
+        except RuntimeError as gather_err:
+            if err is not None:
+                raise err from gather_err
+            raise
+        if err is not None:
+            raise err
+        return c
+
+    def _root_iteration(self, env, policy):
+        if not self.is_root:
+            raise RuntimeError("ShardedCollector: only the root rank collects; the other ranks call serve()")
+        if self._stopped:
+            raise RuntimeError("ShardedCollector: closed")
+        cmd = self._command(int(env.difficulty), self.collect_id)
+        self.collect_id += 1
+        return self._iteration(env, policy, *cmd)
+
+    def collect(self, env, policy):
+        """Root: one sharded collect of every rank, as the wrapped collector's `CollectedData` of all episodes."""
+        return self.local.to_host(self._root_iteration(env, policy))
+
+    def collect_torch(self, env, policy, dense_obs: bool = True) -> dict:
+        """Root: one sharded PPO collect of every rank, as torch CUDA tensors on root's device over the gathered result
+        (`collector.torch_views`; valid until the next collect or gather on root's engine)."""
+        from .collector import PPOCollector, torch_views
+        if not isinstance(self.local, PPOCollector):
+            raise TypeError("collect_torch needs a PPOCollector")
+        return torch_views(self._root_iteration(env, policy), self.comm.engine.device, dense_obs)
+
+    def serve(self, env, policy) -> int:
+        """The other ranks: collect and send a shard per root iteration until root closes.  Returns the iterations served."""
+        if self.is_root:
+            raise RuntimeError("ShardedCollector: the root rank collects; serve() is for the other ranks")
+        n = 0
+        while (cmd := self._command())[0] != STOP:
+            self._iteration(env, policy, *cmd)
+            n += 1
+        return n
+
+    def close(self):
+        """Root: stops the workers (once)."""
+        if self.is_root and not self._stopped:
+            self._stopped = True
+            self._command(STOP)
