@@ -39,7 +39,10 @@ typedef enum {
     TWR_ERR_STATE = -4        /* call order (e.g. to_host before collect) */
 } twr_status;
 
-typedef enum { TWR_ENV_PUZZLE = 0, TWR_ENV_GRIDWORLD = 1 } twr_env_kind;
+/* TWR_ENV_PUZZLE takes boards of up to 16 cells (one byte per cell in the env state); TWR_ENV_PUZZLE_WIDE is the same
+ * env for boards of up to 25 cells (5x5, 4x6, ...: 5-bit cells in the same 16 bytes), and what a Puzzle above 16 cells
+ * must be created as.  Both behave exactly as envs::Puzzle. */
+typedef enum { TWR_ENV_PUZZLE = 0, TWR_ENV_GRIDWORLD = 1, TWR_ENV_PUZZLE_WIDE = 2 } twr_env_kind;
 
 /* arithmetic of the policy forward (kernel K2) */
 typedef enum {
@@ -84,7 +87,9 @@ int64_t twr_engine_launch_count(const twr_engine* e);
 /* --------------------------------------------------------------------- env --- */
 /* Device-side equivalent of a `Box<dyn Env>` (rust/src/rl/env.rs:18-66): the constructor
  * arguments of envs::Puzzle (rust/src/envs/puzzle.rs:34-42, python_interface/env.rs:124-134)
- * or of grid_world::GridWorld (examples/grid_world/src/lib.rs:23-41) plus its difficulty. */
+ * or of grid_world::GridWorld (examples/grid_world/src/lib.rs:23-41) plus its difficulty.
+ * Puzzle boards of up to 25 cells run on the device (above 16 cells as TWR_ENV_PUZZLE_WIDE); larger
+ * ones are refused with TWR_ERR_UNSUPPORTED.  GridWorld takes 3..32 cells. */
 typedef struct {
     int32_t kind;        /* twr_env_kind */
     int32_t width, height;

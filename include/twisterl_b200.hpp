@@ -39,7 +39,7 @@ inline void check(int rc) {
 
 // ---------------------------------------------------------------------------------------------- envs ---
 inline twr_env_spec Puzzle(int width, int height, int difficulty, int depth_slope, int max_depth) {   // envs/puzzle.rs:34-42
-    return twr_env_spec{TWR_ENV_PUZZLE, width, height, difficulty, depth_slope, max_depth};
+    return twr_env_spec{width * height > 16 ? TWR_ENV_PUZZLE_WIDE : TWR_ENV_PUZZLE, width, height, difficulty, depth_slope, max_depth};
 }
 inline twr_env_spec GridWorld(int width, int height, int max_steps, int difficulty) {                  // grid_world/src/lib.rs:23-41
     return twr_env_spec{TWR_ENV_GRIDWORLD, width, height, difficulty, 0, max_steps};

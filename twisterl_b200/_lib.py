@@ -16,7 +16,7 @@ PKG = Path(__file__).resolve().parent
 LIB_PATH = PKG / "lib" / "libtwisterl_b200.so"
 
 OK = 0
-ENV_PUZZLE, ENV_GRIDWORLD = 0, 1
+ENV_PUZZLE, ENV_GRIDWORLD, ENV_PUZZLE_WIDE = 0, 1, 2   # twr_env_kind; ENV_PUZZLE_WIDE: Puzzle of 17..25 cells
 ABI_VERSION = 3                      # TWR_ABI_VERSION of the header these struct layouts / prototypes were written against
 PREC_FP32, PREC_F16X2, PREC_F16X2_W16, PREC_F16_F8C = 0, 1, 2, 3
 PRECISIONS = {"fp32": PREC_FP32, "f16x2": PREC_F16X2, "f16x2w16": PREC_F16X2_W16, "f16f8c": PREC_F16_F8C}

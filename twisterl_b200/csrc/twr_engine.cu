@@ -73,9 +73,15 @@ int check_spec(const twr_env_spec* s, EnvParams* out) {
     p.kind = s->kind; p.W = s->width; p.H = s->height; p.N = s->width * s->height;
     p.difficulty = s->difficulty; p.depth_slope = s->depth_slope; p.max_depth = s->max_depth;
     if (s->difficulty < 0 || s->max_depth < 0) return fail(TWR_ERR_INVALID, "difficulty/max_depth must be >= 0");
-    if (s->kind == TWR_ENV_PUZZLE) {
+    if (s->kind == TWR_ENV_PUZZLE || s->kind == TWR_ENV_PUZZLE_WIDE) {
+        // one env; the kernels see one Puzzle kind and pick the cell encoding from the board size (twr_common.cuh)
+        p.kind = TWR_ENV_PUZZLE;
+        if (s->kind == TWR_ENV_PUZZLE && p.N > TWR_MAX_CELLS_BYTES)
+            return fail(TWR_ERR_UNSUPPORTED, "Puzzle boards above 16 cells are env kind TWR_ENV_PUZZLE_WIDE "
+                                             "(5-bit cells, up to 25 cells)");
         if (p.N > TWR_MAX_CELLS_PUZZLE)
-            return fail(TWR_ERR_UNSUPPORTED, "Puzzle boards above 16 cells are not implemented on the device path");
+            return fail(TWR_ERR_UNSUPPORTED, "Puzzle boards above 25 cells are not implemented on the device path "
+                                             "(the 128-bit env state holds at most 25 five-bit cells)");
         if (s->depth_slope < 0) return fail(TWR_ERR_INVALID, "depth_slope must be >= 0");
         if ((int64_t)s->depth_slope * s->difficulty >= (1 << 24)) return fail(TWR_ERR_INVALID, "depth budget too large");
     } else if (s->kind == TWR_ENV_GRIDWORLD) {
@@ -639,9 +645,14 @@ int twr_envs_set_cell(twr_envs* v, int64_t env, int32_t cell, int32_t value) {
     if (value < 0 || value >= v->p.N) return fail(TWR_ERR_INVALID, "set_cell: Puzzle cell values must be tiles 0..cells-1");
     twr_engine* e = v->eng;
     CU_TRY(cudaSetDevice(e->device));
-    // byte `cell` of the env's 16-byte board; blank index and depth stay as they are (puzzle.rs:71-73)
-    const uint8_t b = (uint8_t)value;
-    CU_TRY(cudaMemcpyAsync(reinterpret_cast<uint8_t*>(v->cells + env) + cell, &b, 1, cudaMemcpyHostToDevice, e->stream));
+    // one cell of the env's board, rewritten in the board's encoding; blank index and depth stay as they are (puzzle.rs:71-73)
+    uint4 c;
+    CU_TRY(cudaMemcpyAsync(&c, v->cells + env, sizeof(c), cudaMemcpyDeviceToHost, e->stream));
+    CU_TRY(cudaStreamSynchronize(e->stream));
+    EnvState s = env_from_cells(c);
+    cell_set(s, cell, (uint32_t)value, cells_wide(v->p));
+    c = env_pack_cells(s);
+    CU_TRY(cudaMemcpyAsync(v->cells + env, &c, sizeof(c), cudaMemcpyHostToDevice, e->stream));
     CU_TRY(cudaStreamSynchronize(e->stream));
     return TWR_OK;
 }

@@ -68,14 +68,10 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_forward_fp32(PolicyDev p, Forwa
     if (tid < TM) {
         const int64_t pos = tile0 + tid;
         int perm = -1;
-        EnvState s; s.lo = 0; s.hi = 0; s.blank = 0; s.depth = 0;
+        EnvState s = env_from_cells(make_uint4(0, 0, 0, 0));
         if (pos < n) {
             const int64_t e = a.live ? a.live[pos] : pos;
-            if (!a.obs_rows) {
-                const uint4 c = a.cells[e];
-                s.lo = (uint64_t)c.x | ((uint64_t)c.y << 32);
-                s.hi = (uint64_t)c.z | ((uint64_t)c.w << 32);
-            }
+            if (!a.obs_rows) s = env_from_cells(a.cells[e]);
             if (a.perm_idx) {
                 perm = a.perm_idx[pos];
             } else if (p.n_perms > 0 && a.t >= 0) {       // get_perm_id, nn/policy.rs:67-77

@@ -765,9 +765,7 @@ k_forward_tc2(PolicyDev p, ForwardArgs a, Tc2Params t, const __grid_constant__ C
             const int64_t pos = q.pos;
             const int t_cur = a.t + q.step;
             int perm = -1;
-            EnvState s; s.blank = 0; s.depth = 0;
-            s.lo = (uint64_t)q.c.x | ((uint64_t)q.c.y << 32);
-            s.hi = (uint64_t)q.c.z | ((uint64_t)q.c.w << 32);
+            const EnvState s = env_from_cells(q.c);
             if (pos < n) {
                 if (a.perm_idx) {
                     perm = a.perm_idx[pos];
@@ -827,7 +825,7 @@ k_forward_tc2(PolicyDev p, ForwardArgs a, Tc2Params t, const __grid_constant__ C
                 for (int i = 0; i < n_obs; ++i) {
                     uint32_t r = 0;
                     if (pos < n) {
-                        r = a.obs_rows ? (uint32_t)a.obs_rows[pos * n_obs + i] : (uint32_t)(i * a.env.N) + env_board(a.env, s, i);
+                        r = a.obs_rows ? (uint32_t)a.obs_rows[pos * n_obs + i] : (uint32_t)(i * a.env.N) + env_board<TWR_CELLS_BYTES>(a.env, s, i);
                         if (perm >= 0)                                                         // twist-in, policy.rs:81-83
                             r = operm_smem ? (uint32_t)operm_s[perm * p.obs_size + (int)r] : (uint32_t)p.obs_perms[(size_t)perm * p.obs_size + r];
                         if (t.cN > 0) r = (r / (uint32_t)t.cN) * 4u + (r % (uint32_t)t.cN);   // compact GridWorld table (values 0..3)
@@ -942,7 +940,7 @@ k_forward_tc2(PolicyDev p, ForwardArgs a, Tc2Params t, const __grid_constant__ C
                 sa.t = a.t + v.step;
                 // inside a multi-step chunk an env that already recorded its terminal state idles
                 const bool alive = active && (t_count == 1 || a.cb.ep_len[e] == 0);
-                collect_step_body(sa, a.cb, alive, e, make_float4(v.out[0], v.out[1], v.out[2], v.out[3]), v.value, v.perm,
+                collect_step_body<TWR_CELLS_BYTES>(sa, a.cb, alive, e, make_float4(v.out[0], v.out[1], v.out[2], v.out[3]), v.value, v.perm,
                                   a.live_next);
             } else if (active) {
                 a.logits[v.pos] = make_float4(v.out[0], v.out[1], v.out[2], v.out[3]);

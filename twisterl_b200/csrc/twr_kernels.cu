@@ -42,20 +42,20 @@ __global__ void __launch_bounds__(256) k_envs_set_state(EnvParams p, uint4* __re
     EnvState s = env_load(cells, meta, e);
     const int64_t* st = states + e * p.N;
     if (p.kind == 0) {
-        s.lo = TWR_IDENT_LO; s.hi = TWR_IDENT_HI;
+        env_set_identity(p, s);
         bool found = false;
         for (int i = 0; i < p.N; ++i) {
             const int64_t v = st[i];
-            cell_set(s, i, (uint32_t)v);
+            cell_set(s, i, (uint32_t)v, cells_wide(p));
             if (v == 0 && !found) { s.blank = (uint32_t)i; found = true; }
         }
         s.depth = (uint32_t)p.max_depth;
     } else {
         for (int i = 0; i < p.N; ++i) {
             const int64_t v = st[i];
-            if (v == 1) cell_set(s, 0, (uint32_t)i);
-            else if (v == 2) cell_set(s, 1, (uint32_t)i);
-            else if (v == 3) cell_set(s, 2, (uint32_t)i);
+            if (v == 1) cell_set(s, 0, (uint32_t)i, false);
+            else if (v == 2) cell_set(s, 1, (uint32_t)i, false);
+            else if (v == 3) cell_set(s, 2, (uint32_t)i, false);
         }
         s.depth = (uint32_t)p.max_depth;
     }
@@ -446,11 +446,7 @@ __global__ void __launch_bounds__(256) k_compact(EnvParams p, CollectBuffers b, 
             continue;
         }
         for (int j = x; j < nt * p.N; j += 32) {
-            const uint4 q = tl.q[1][j / p.N][ey];
-            EnvState s;
-            s.lo = (uint64_t)q.x | ((uint64_t)q.y << 32);
-            s.hi = (uint64_t)q.z | ((uint64_t)q.w << 32);
-            s.blank = 0; s.depth = 0;
+            const EnvState s = env_from_cells(tl.q[1][j / p.N][ey]);
             const int i = j % p.N;
             const int idx = i * p.N + (int)env_board(p, s, i);
             if (b.obs_u8) dst8[j] = (uint8_t)idx; else dst[j] = (uint16_t)idx;

@@ -638,9 +638,7 @@ k_mcts_persistent(MctsArgs a, PolicyDev p, const int32_t* __restrict__ live, con
             int pi;
             const int j = slot_tree(g, pi);
             if ((TW && j < 0) || !leaf_flag[j]) continue;
-            const uint4 c = leaf_cells[j];
-            EnvState s; s.blank = 0; s.depth = 0;
-            s.lo = (uint64_t)c.x | ((uint64_t)c.y << 32); s.hi = (uint64_t)c.z | ((uint64_t)c.w << 32);
+            const EnvState s = env_from_cells(leaf_cells[j]);
             float4 acc = *reinterpret_cast<const float4*>(embb + f4);                       // bias first, then the rows in
             for (int i = 0; i < a.env.N; ++i) {                                              // observation order (layers.rs:58-62)
                 int r = i * a.env.N + (int)env_board(a.env, s, i);

@@ -7,7 +7,8 @@
 // Must be called by all 32 lanes of a warp (`active` false for padding lanes): reward(s_t), masked
 // logits, value, Gumbel-max action and twist index go to record [t][env]; terminal states are recorded
 // and retire (their action is not applied), the rest step and are appended to the next live list with
-// one atomicAdd per warp (ballot + popc prefix).
+// one atomicAdd per warp (ballot + popc prefix).  F: the cell encodings the caller is compiled for (twr_common.cuh).
+template <int F = TWR_CELLS_ANY>
 __device__ __forceinline__ void collect_step_body(const StepArgs& a, const CollectBuffers& b, bool active, int e,
                                                   float4 raw, float value, int perm, int32_t* __restrict__ live_next) {
     bool survives = false;
@@ -24,8 +25,8 @@ __device__ __forceinline__ void collect_step_body(const StepArgs& a, const Colle
         philox4x32_10(gid, (uint32_t)a.t, TWR_RNG_SAMPLE, a.cid, k0, k1, w);
         const float u[4] = {u32_to_unit_f32(w[0]), u32_to_unit_f32(w[1]), u32_to_unit_f32(w[2]), u32_to_unit_f32(w[3])};
         const int act = sample_from_logits4(l, u, a.A);
-        const float rew = env_reward(a.env, s);
-        const bool fin = env_is_final(a.env, s);
+        const float rew = env_reward<F>(a.env, s);
+        const bool fin = env_is_final<F>(a.env, s);
 
         const int64_t r = (int64_t)a.t * b.B + e;
         b.rec_state[r] = env_pack_cells(s);
@@ -37,10 +38,10 @@ __device__ __forceinline__ void collect_step_body(const StepArgs& a, const Colle
 
         if (fin) {
             b.ep_len[e] = a.t + 1;
-            if (env_success(a.env, s)) atomicAdd(&b.stats[0], 1ull);
+            if (env_success<F>(a.env, s)) atomicAdd(&b.stats[0], 1ull);
             atomicAdd(reinterpret_cast<double*>(&b.stats[2]), (double)rew);
         } else {
-            env_step(a.env, s, act);
+            env_step<F>(a.env, s, act);
             env_store(b.cells, b.meta, e, s);
             survives = true;
         }

@@ -145,14 +145,15 @@ def spec_from_env(env) -> _lib.EnvSpec:
 
 
 class Puzzle(PyBaseEnv):
-    """`env.Puzzle(width, height, difficulty, depth_slope, max_depth)` (python_interface/env.rs:117-160)."""
+    """`env.Puzzle(width, height, difficulty, depth_slope, max_depth)` (python_interface/env.rs:117-160).  Boards of up to
+    25 cells (the 24-puzzle, 5x5, among them) run on the device; a larger board raises RuntimeError at its first use."""
 
     def __init__(self, width: int, height: int, difficulty: int, depth_slope: int, max_depth: int, add_perms: bool = False):
         for v in (width, height, difficulty, depth_slope, max_depth):
             if int(v) < 0:
                 raise OverflowError("can't convert negative int to unsigned")
-        self._init_spec(_lib.EnvSpec(_lib.ENV_PUZZLE, int(width), int(height), int(difficulty), int(depth_slope),
-                                     int(max_depth)))
+        kind = _lib.ENV_PUZZLE_WIDE if int(width) * int(height) > 16 else _lib.ENV_PUZZLE
+        self._init_spec(_lib.EnvSpec(kind, int(width), int(height), int(difficulty), int(depth_slope), int(max_depth)))
         # Opt-in twist set (docs/twists.md: "gate toggles through config ... an `add_perms` flag"): the reference's Puzzle
         # declares no twists (Env::twists default, rl/env.rs:59), and neither does this one unless asked to
         self._add_perms = bool(add_perms)
