@@ -89,7 +89,8 @@ int64_t twr_engine_launch_count(const twr_engine* e);
  * arguments of envs::Puzzle (rust/src/envs/puzzle.rs:34-42, python_interface/env.rs:124-134)
  * or of grid_world::GridWorld (examples/grid_world/src/lib.rs:23-41) plus its difficulty.
  * Puzzle boards of up to 25 cells run on the device (above 16 cells as TWR_ENV_PUZZLE_WIDE); larger
- * ones are refused with TWR_ERR_UNSUPPORTED.  GridWorld takes 3..32 cells. */
+ * ones are refused with TWR_ERR_UNSUPPORTED.  GridWorld takes 3..64 cells (up to 8x8) with the same encoding at
+ * every size; larger boards are refused with TWR_ERR_UNSUPPORTED. */
 typedef struct {
     int32_t kind;        /* twr_env_kind */
     int32_t width, height;
@@ -182,7 +183,7 @@ int  twr_policy_forward(twr_engine* e, const twr_policy* p, twr_envs* v, const i
                         int32_t apply_masks, float* logits, float* values);
 
 /* Policy::_raw_predict for n sparse observations given directly: obs [n][n_obs] one-hot indices
- * (what Env::observe returns), as python_interface/policy.rs:33-44 receives them.  n_obs <= 32. */
+ * (what Env::observe returns), as python_interface/policy.rs:33-44 receives them.  n_obs <= 64. */
 int  twr_policy_forward_obs(twr_engine* e, const twr_policy* p, const int32_t* obs, int64_t n, int32_t n_obs,
                             const int32_t* perm_idx, float* logits, float* values);
 

@@ -1,0 +1,4 @@
+"""test_gpu_grid_world_large.py once more on precision "f16x2": GridWorld forwards of 33..64 cells on the pair kernel."""
+from suite_loader import clone_suite
+
+globals().update(clone_suite("test_gpu_grid_world_large", "f16x2"))

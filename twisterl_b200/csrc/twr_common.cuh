@@ -16,7 +16,8 @@
 #define TWR_MAX_ACTIONS 4
 #define TWR_MAX_CELLS_PUZZLE 25   // 5-bit cells in the 128-bit state
 #define TWR_MAX_CELLS_BYTES 16    // the byte encoding
-#define TWR_MAX_CELLS 32
+#define TWR_MAX_CELLS 32          // boards whose N*N-row table the forwards stage whole (and the observation length a policy's fit assumes)
+#define TWR_MAX_OBS 64            // observation indices per env: GridWorld of up to 64 cells (4 * 64 compact rows, 256)
 
 enum : uint32_t { TWR_RNG_RESET = 0, TWR_RNG_PERM = 1, TWR_RNG_SAMPLE = 2, TWR_RNG_SOLVE = 3, TWR_RNG_MCTS = 4, TWR_RNG_AZ_ACT = 5 };
 

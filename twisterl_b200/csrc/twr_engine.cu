@@ -85,8 +85,10 @@ int check_spec(const twr_env_spec* s, EnvParams* out) {
         if (s->depth_slope < 0) return fail(TWR_ERR_INVALID, "depth_slope must be >= 0");
         if ((int64_t)s->depth_slope * s->difficulty >= (1 << 24)) return fail(TWR_ERR_INVALID, "depth budget too large");
     } else if (s->kind == TWR_ENV_GRIDWORLD) {
-        if (p.N > TWR_MAX_CELLS || p.N < 3)
-            return fail(TWR_ERR_UNSUPPORTED, "GridWorld needs 3..32 cells on the device path");
+        // bytes 0..2 of the state hold any cell index; the bound is the forward's: above 64 cells the compact table
+        // (4 rows per cell) leaves the pair kernel's 256-row operand and a record carries more than 64 indices
+        if (p.N > TWR_MAX_OBS || p.N < 3)
+            return fail(TWR_ERR_UNSUPPORTED, "GridWorld needs 3..64 cells on the device path");
         const int cap = s->width + s->height;                      // lib.rs:36,92-94
         p.difficulty = s->difficulty < cap ? s->difficulty : cap;
         if (s->max_depth >= (1 << 24)) return fail(TWR_ERR_INVALID, "max_steps too large");
@@ -468,29 +470,37 @@ int twr_policy_create(twr_engine* e, const twr_policy_desc* d_in, twr_policy** o
     if (standard) {
         PolicyDev probe = p->dev;
         probe.n_obs = 1;
-        EnvParams dummy{};
         const char* why = "";
         // TWR_PREC_F16X2 = tensor cores where the shape fits the tcgen05 kernel (obs_size <= 256, E % 128 == 0 and
         // E <= 1024, H in {128, 256}); other shapes (GridWorld's 625-row table) run the fp32 SIMT kernel -- still on the device.
         // GridWorld-shaped tables (obs_size = N*N > 256, only rows i*N + {0,1,2,3} reachable): the pair kernel runs on
         // the compact 4N-row table when the twists (if any) keep the reachable rows among themselves
-        if (e->precision != TWR_PREC_FP32 && d->obs_size > 256) {
-            const int N = board_side(d->obs_size);
-            bool ok = N * N == d->obs_size && N <= TWR_MAX_CELLS && 4 * N <= 256;
+        const int N = board_side(d->obs_size);
+        const bool square = N * N == d->obs_size;
+        if (d->obs_size > 256) {
+            bool ok = square && 4 * N <= 256;
             for (int64_t i = 0; ok && i < (int64_t)d->n_perms * d->obs_size; ++i)
                 if ((i % d->obs_size) % N < 4 && d->obs_perms[i] % N >= 4) ok = false;
-            if (ok) probe.tc_compact_n = p->dev.tc_compact_n = N;
+            if (ok) p->grid_n = N;
+            if (ok && e->precision != TWR_PREC_FP32) probe.compact_n = p->dev.compact_n = N;
         }
         use_tc = e->precision != TWR_PREC_FP32 && forward_tc2_supported(probe);
+        // The fp32 kernel's fit holds for the longest observation the policy can meet: N indices for the table of a board
+        // above 32 cells.  Such a table (up to 64 cells) is taken whether or not it fits whole: call_dev sends GridWorld
+        // forwards to the compact table and any forward the fp32 kernel cannot hold to the generic one.
+        const int max_obs = square && N > TWR_MAX_CELLS ? N : TWR_MAX_CELLS;
+        const bool big_board = max_obs > TWR_MAX_CELLS && N <= TWR_MAX_OBS && max_width <= 1024;
         // a compact-table policy still meets non-GridWorld callers (twr_policy_forward_obs): those run the fp32 kernel
-        if ((!use_tc || p->dev.tc_compact_n > 0) && !forward_fp32_supported(probe, dummy, &why)) {
+        PolicyDev full = probe;
+        full.compact_n = 0;
+        if ((!use_tc || p->dev.compact_n > 0) && !forward_fp32_supported(full, max_obs, &why) && !big_board) {
             if (!use_tc) {
                 delete p;
                 return fail(TWR_ERR_UNSUPPORTED, std::string("policy shape not supported on the device: ") + why);
             }
             use_tc = false;
         }
-        if (!use_tc) p->dev.tc_compact_n = 0;
+        if (!use_tc) p->dev.compact_n = 0;
     } else if (max_width > 1024) {
         delete p;
         return fail(TWR_ERR_UNSUPPORTED, "general layer stacks are implemented for layer widths up to 1024");
@@ -693,15 +703,24 @@ int twr_envs_depth(twr_envs* v, int32_t* d) { return query_field<int32_t>(v, d, 
 // -------------------------------------------------------------------- forward ---
 // The policy as one forward runs it, over envs `env` or (env NULL) the n rows of n_obs indices in `obs`: tc_pack cleared,
 // so the fp32 kernel runs, for a compact-table policy outside GridWorld envs of its size, or a row that repeats an index
-// (the one-hot GEMM operand cannot express one).
-static PolicyDev call_dev(const PolicyDev& pol, const EnvParams* env, const int32_t* obs, int64_t n, int n_obs) {
+// (the one-hot GEMM operand cannot express one).  The fp32 kernel stages the compact table for GridWorld boards above
+// 32 cells; a forward whose table or rows it cannot hold in shared memory runs the generic kernel, which reads the
+// table from global memory.
+static PolicyDev call_dev(const twr_policy* p, const EnvParams* env, const int32_t* obs, int64_t n, int n_obs) {
+    const PolicyDev& pol = p->dev;
     PolicyDev dev = pol;
     dev.n_obs = env ? env->N : n_obs;
-    bool tc = pol.tc_pack && (pol.tc_compact_n == 0 || (env && env->kind == TWR_ENV_GRIDWORLD && env->N == pol.tc_compact_n));
+    const bool grid = env && env->kind == TWR_ENV_GRIDWORLD && env->N == p->grid_n;
+    bool tc = pol.tc_pack && (pol.compact_n == 0 || grid);
     for (int64_t i = 0; tc && obs && i < n; ++i)
         for (int a = 0; tc && a < n_obs; ++a)
             for (int b = a + 1; tc && b < n_obs; ++b) tc = obs[i * n_obs + a] != obs[i * n_obs + b];
-    if (!tc) dev.tc_pack = nullptr;
+    if (!tc) {
+        dev.tc_pack = nullptr;
+        dev.compact_n = grid && env->N > TWR_MAX_CELLS ? env->N : 0;
+        const char* why = "";
+        if (!dev.generic && !forward_fp32_supported(dev, dev.n_obs, &why)) dev.generic = 1;
+    }
     return dev;
 }
 
@@ -709,7 +728,7 @@ static int check_policy_env(const twr_policy* p, const EnvParams& env, PolicyDev
     if (p->dev.obs_size != env.N * env.N)
         return fail(TWR_ERR_INVALID, "policy obs_size does not match the env's obs_shape (cells*cells)");
     if (p->dev.A != 4) return fail(TWR_ERR_INVALID, "policy has " + std::to_string(p->dev.A) + " actions, env has 4");
-    *dev = call_dev(p->dev, &env, nullptr, 0, 0);
+    *dev = call_dev(p, &env, nullptr, 0, 0);
     return TWR_OK;
 }
 
@@ -832,7 +851,7 @@ int twr_policy_forward_obs(twr_engine* e, const twr_policy* p, const int32_t* ob
     return twr_guard([&]() -> int {
     if (!e || !p || !obs || !logits || !values) return fail(TWR_ERR_INVALID, "NULL argument");
     if (p->eng != e) return fail(TWR_ERR_INVALID, "policy belongs to another engine");
-    if (n_obs < 1 || n_obs > TWR_MAX_CELLS) return fail(TWR_ERR_UNSUPPORTED, "n_obs must be in 1..32");
+    if (n_obs < 1 || n_obs > TWR_MAX_OBS) return fail(TWR_ERR_UNSUPPORTED, "n_obs must be in 1..64");
     if (n <= 0) return TWR_OK;
     for (int64_t i = 0; i < n * n_obs; ++i)
         if (obs[i] < 0 || obs[i] >= p->dev.obs_size) return fail(TWR_ERR_INVALID, "observation index out of range");
@@ -843,7 +862,7 @@ int twr_policy_forward_obs(twr_engine* e, const twr_policy* p, const int32_t* ob
         for (int a2 = 0; a2 < n_obs; ++a2) seen |= 1ull << (obs[i * n_obs + a2] / p->dev.tc_fold);
         blocks = seen == (n_obs >= 64 ? ~0ull : (1ull << n_obs) - 1);
     }
-    const PolicyDev dev = call_dev(p->dev, nullptr, obs, n, n_obs);
+    const PolicyDev dev = call_dev(p, nullptr, obs, n, n_obs);
     EnvParams obs_env{};                     // only the index count: the rows are given, not read from env state
     obs_env.N = n_obs;
     HostForward f;

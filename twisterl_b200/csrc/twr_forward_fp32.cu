@@ -12,6 +12,10 @@
 // conflict-free shared-memory gather, and the 128 x H output tile lives in registers
 // (8 envs x H/16 columns per thread).  Bound: fp32 FMA pipe (2*E*H flop per env) -- this variant
 // exists for the 1e-5 parity bar; the tensor-core variant is twr_forward_tc2.cu.
+//
+// COMPACT (GridWorld boards of 33..64 cells, PolicyDev::compact_n = N): a GridWorld observation only reaches table
+// rows i*N + v with v in 0..3 (examples/grid_world/src/lib.rs:74-81), so each KC slice stages those 4N rows alone, row
+// i*N + v at i*4 + v.  The cells are summed in the same order from the same values: the full-table arithmetic, bit for bit.
 #include "twr_kernels.cuh"
 
 #include <atomic>
@@ -30,7 +34,7 @@ __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commi
 template <int N>
 __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;\n" ::"n"(N)); }
 
-template <int H, int KC>
+template <int H, int KC, bool COMPACT>
 __global__ void __launch_bounds__(NTHREADS, 1) k_forward_fp32(PolicyDev p, ForwardArgs a) {
     constexpr int TN = H / 16;      // output columns per thread
     constexpr int LPF = KC / 4;     // lanes covering one env's KC features with float4
@@ -43,19 +47,22 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_forward_fp32(PolicyDev p, Forwa
 
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int n_obs = p.n_obs, obs_size = p.obs_size, E = p.E;
+    const int cn = COMPACT ? p.compact_n : 0;
+    const int tab_rows = COMPACT ? 4 * cn : obs_size;              // staged rows of the table
 
-    float* Es = reinterpret_cast<float*>(smem_raw);                 // [2][obs_size*KC]
-    float* Ws = Es + 2 * (size_t)obs_size * KC;                     // [2][KC*H]
+    float* Es = reinterpret_cast<float*>(smem_raw);                 // [2][tab_rows*KC]
+    float* Ws = Es + 2 * (size_t)tab_rows * KC;                     // [2][KC*H]
     float* As = Ws + 2 * (size_t)KC * H;                            // [TM][KC]
     uint16_t* rows_s = reinterpret_cast<uint16_t*>(As + TM * KC);   // [TM][n_obs]
     int8_t* perm_s = reinterpret_cast<int8_t*>(rows_s + TM * n_obs); // [TM]
 
     auto issue_chunk = [&](int kc, int buf) {
-        float* es = Es + (size_t)buf * obs_size * KC;
-        const int e_pieces = obs_size * LPF;
+        float* es = Es + (size_t)buf * tab_rows * KC;
+        const int e_pieces = tab_rows * LPF;
         for (int q = tid; q < e_pieces; q += NTHREADS) {
             const int row = q / LPF, c4 = q % LPF;
-            cp_async16(es + row * KC + c4 * 4, p.emb + (size_t)row * E + kc * KC + c4 * 4);
+            const int src = COMPACT ? (row >> 2) * cn + (row & 3) : row;
+            cp_async16(es + row * KC + c4 * 4, p.emb + (size_t)src * E + kc * KC + c4 * 4);
         }
         float* ws = Ws + (size_t)buf * KC * H;
         const float* wsrc = p.w1 + (size_t)kc * KC * H;
@@ -86,6 +93,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_forward_fp32(PolicyDev p, Forwa
             int row = 0;
             if (pos < n) row = a.obs_rows ? a.obs_rows[pos * n_obs + i] : i * a.env.N + (int)env_board(a.env, s, i);
             if (perm >= 0) row = p.obs_perms[(size_t)perm * obs_size + row];
+            if (COMPACT) row = (row / cn) * 4 + row % cn;             // the twists keep v in 0..3 (twr_policy_create)
             rows_s[tid * n_obs + i] = (uint16_t)row;
         }
     }
@@ -106,7 +114,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_forward_fp32(PolicyDev p, Forwa
 
         // ---- embedding slice: As[env][f] = relu(bias[f] + sum_i Es[row_i][f])
         {
-            const float* es = Es + (size_t)buf * obs_size * KC;
+            const float* es = Es + (size_t)buf * tab_rows * KC;
             const int f4 = lane % LPF, eg = lane / LPF;
             const float4 bias = *reinterpret_cast<const float4*>(p.emb_b + kc * KC + f4 * 4);
 #pragma unroll 2
@@ -214,27 +222,33 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_forward_fp32(PolicyDev p, Forwa
 }
 
 template <int H, int KC>
-size_t smem_bytes(const PolicyDev& p) {
-    size_t b = sizeof(float) * (2 * (size_t)p.obs_size * KC + 2 * (size_t)KC * H + (size_t)TM * KC);
-    b += sizeof(uint16_t) * (size_t)TM * p.n_obs + TM;
+size_t smem_bytes(const PolicyDev& p, int n_obs) {
+    const size_t rows = p.compact_n > 0 ? 4 * (size_t)p.compact_n : (size_t)p.obs_size;
+    size_t b = sizeof(float) * (2 * rows * KC + 2 * (size_t)KC * H + (size_t)TM * KC);
+    b += sizeof(uint16_t) * (size_t)TM * n_obs + TM;
     return (b + 15) & ~(size_t)15;
 }
 
 constexpr size_t SMEM_LIMIT = 227 * 1024;
 
+template <int H, int KC>
+void launch_kc(cudaStream_t st, const PolicyDev& p, const ForwardArgs& a, unsigned grid) {
+    const size_t sm = smem_bytes<H, KC>(p, p.n_obs);
+    auto kern = p.compact_n > 0 ? k_forward_fp32<H, KC, true> : k_forward_fp32<H, KC, false>;
+    cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
+    kern<<<grid, NTHREADS, sm, st>>>(p, a);
+}
+
+// n_obs: the observation length the fit is sized for (the launch's own, p.n_obs, when not dry)
 template <int H>
-bool launch_h(cudaStream_t st, const PolicyDev& p, const ForwardArgs& a, bool dry) {
+bool launch_h(cudaStream_t st, const PolicyDev& p, const ForwardArgs& a, int n_obs, bool dry) {
     const unsigned grid = (unsigned)((a.n + TM - 1) / TM);
-    if (p.E % 32 == 0 && smem_bytes<H, 32>(p) <= SMEM_LIMIT) {
+    if (p.E % 32 == 0 && smem_bytes<H, 32>(p, n_obs) <= SMEM_LIMIT) {
         if (dry) return true;
-        const size_t sm = smem_bytes<H, 32>(p);
-        cudaFuncSetAttribute(k_forward_fp32<H, 32>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
-        k_forward_fp32<H, 32><<<grid, NTHREADS, sm, st>>>(p, a);
-    } else if (p.E % 16 == 0 && smem_bytes<H, 16>(p) <= SMEM_LIMIT) {
+        launch_kc<H, 32>(st, p, a, grid);
+    } else if (p.E % 16 == 0 && smem_bytes<H, 16>(p, n_obs) <= SMEM_LIMIT) {
         if (dry) return true;
-        const size_t sm = smem_bytes<H, 16>(p);
-        cudaFuncSetAttribute(k_forward_fp32<H, 16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
-        k_forward_fp32<H, 16><<<grid, NTHREADS, sm, st>>>(p, a);
+        launch_kc<H, 16>(st, p, a, grid);
     } else {
         return false;
     }
@@ -242,34 +256,31 @@ bool launch_h(cudaStream_t st, const PolicyDev& p, const ForwardArgs& a, bool dr
     return true;
 }
 
-bool dispatch(cudaStream_t st, const PolicyDev& p, const ForwardArgs& a, bool dry) {
+bool dispatch(cudaStream_t st, const PolicyDev& p, const ForwardArgs& a, int n_obs, bool dry) {
     switch (p.H) {
-        case 64: return launch_h<64>(st, p, a, dry);
-        case 128: return launch_h<128>(st, p, a, dry);
-        case 192: return launch_h<192>(st, p, a, dry);
-        case 256: return launch_h<256>(st, p, a, dry);
+        case 64: return launch_h<64>(st, p, a, n_obs, dry);
+        case 128: return launch_h<128>(st, p, a, n_obs, dry);
+        case 192: return launch_h<192>(st, p, a, n_obs, dry);
+        case 256: return launch_h<256>(st, p, a, n_obs, dry);
         default: return false;
     }
 }
 
 }  // namespace
 
-int forward_fp32_supported(const PolicyDev& p, const EnvParams& env, const char** why) {
+int forward_fp32_supported(const PolicyDev& p, int n_obs, const char** why) {
     static const char* msg_h = "common width must be 64, 128, 192 or 256";
     static const char* msg_e = "embedding size must be a multiple of 16 and the table slice must fit shared memory";
-    static const char* msg_o = "obs_size must be < 65536 and obs per env <= 32";
-    (void)env;
+    static const char* msg_o = "obs_size must be < 65536 and obs per env <= 64";
     if (p.H != 64 && p.H != 128 && p.H != 192 && p.H != 256) { *why = msg_h; return 0; }
-    if (p.obs_size >= 65536 || p.n_obs > TWR_MAX_CELLS) { *why = msg_o; return 0; }
+    if (p.obs_size >= 65536 || n_obs > TWR_MAX_OBS) { *why = msg_o; return 0; }
     ForwardArgs a{};
     a.n = 1;
-    PolicyDev q = p;
-    q.n_obs = TWR_MAX_CELLS;                 // the fit must hold for any observation length a later launch may carry
-    if (!dispatch(nullptr, q, a, true)) { *why = msg_e; return 0; }
+    if (!dispatch(nullptr, p, a, n_obs, true)) { *why = msg_e; return 0; }
     return 1;
 }
 
 bool launch_forward_fp32(cudaStream_t st, const PolicyDev& p, const ForwardArgs& a) {
     if (a.n <= 0) return true;
-    return dispatch(st, p, a, false);
+    return dispatch(st, p, a, p.n_obs, false);
 }

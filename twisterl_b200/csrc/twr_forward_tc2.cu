@@ -1112,8 +1112,8 @@ k_forward_tc2(PolicyDev p, ForwardArgs a, Tc2Params t, const __grid_constant__ C
 
 Tc2Params make_params2(const PolicyDev& p, bool f8 = false) {
     Tc2Params t;
-    t.E = p.E; t.H = p.H; t.NC = 2 * ((p.E + 255) / 256); t.cN = p.tc_compact_n;   // E % 256 == 128: zero-padded to a chunk pair
-    t.NKB1 = ((p.tc_compact_n > 0 ? 4 * p.tc_compact_n : p.obs_size) + 63) / 64;
+    t.E = p.E; t.H = p.H; t.NC = 2 * ((p.E + 255) / 256); t.cN = p.compact_n;   // E % 256 == 128: zero-padded to a chunk pair
+    t.NKB1 = ((p.compact_n > 0 ? 4 * p.compact_n : p.obs_size) + 63) / 64;
     t.NKB8 = (t.NKB1 + 1) / 2;
     t.f8 = 0; t.row0 = 0; t.fold = 0;
     if (f8) {                                   // the fp8-correction image follows the standard one; it carries the folded bias
@@ -1175,7 +1175,7 @@ bool get_tmap(DevState& d, const void* pack, size_t bytes, CUtensorMap* out) {
 // E in 128-feature chunks (an odd count is padded to a pair), the one-hot operand holds <= 256 (compact) rows, GEMM2 is
 // N = H in {128, 256}
 int forward_tc2_supported(const PolicyDev& p) {
-    const int k1 = p.tc_compact_n > 0 ? 4 * p.tc_compact_n : p.obs_size;
+    const int k1 = p.compact_n > 0 ? 4 * p.compact_n : p.obs_size;
     return (p.H == 256 || p.H == 128) && p.E % 128 == 0 && p.E <= 1024 && k1 <= 64 * MAX_KB1;
 }
 

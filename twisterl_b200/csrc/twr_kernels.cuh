@@ -20,10 +20,12 @@ struct PolicyDev {
     // operand image of the tensor-core kernel (fp16 hi/lo split and fp8 corrections, pre-swizzled K-major tiles in
     // streaming order), see k_tc2_pack in twr_forward_tc2.cu; NULL: the policy runs another kernel
     const void* tc_pack;
-    // > 0: the pair kernel's GEMM1 image holds only the 4 * tc_compact_n reachable rows of a GridWorld table
-    // (row (i, v) = i * tc_compact_n + v, v in 0..3; examples/grid_world/src/lib.rs:74-81,161-163); such a policy takes
-    // the tensor-core path only for GridWorld envs of that size whose observation comes from the env state
-    int tc_compact_n;
+    // > 0: the forward runs on the COMPACT table of a GridWorld board of compact_n cells, only its 4 * compact_n reachable
+    // rows (row (i, v) = i * compact_n + v, v in 0..3; examples/grid_world/src/lib.rs:74-81,161-163) at i * 4 + v.
+    // With tc_pack: the pair kernel's GEMM1 image is built so at policy creation, and such a policy takes the tensor-core
+    // path only for GridWorld envs of that size whose observation comes from the env state.  Without: set per forward by
+    // the engine for GridWorld boards above 32 cells, k_forward_fp32 stages only those rows.
+    int compact_n;
     // > 0: obs_size = tc_fold^2 and every twist maps each block of tc_fold consecutive rows onto another block, so an
     // observation that holds exactly ONE index per block (what Puzzle / GridWorld envs produce) selects exactly one row of
     // block 0 before and after a twist: the f16f8c operand image carries the embedding bias on the rows of block 0 and
@@ -132,7 +134,9 @@ struct ForwardArgs {
 #define TWR_DBG_CTAS 148
 #define TWR_DBG_TRACE (TWR_DBG_CTAS * 16)
 #define TWR_DBG_WORDS (TWR_DBG_TRACE + 256)
-int  forward_fp32_supported(const PolicyDev& p, const EnvParams& env, const char** why);
+// does k_forward_fp32 take this policy (its table, or the compact one when compact_n > 0) for observations of up to
+// n_obs indices?
+int  forward_fp32_supported(const PolicyDev& p, int n_obs, const char** why);
 bool launch_forward_fp32(cudaStream_t s, const PolicyDev& p, const ForwardArgs& a);   // false: shape does not fit shared memory
 // Tensor-core (CTA-pair, tcgen05 cta_group::2) variant, twr_forward_tc2.cu; `pack` is its operand image (PolicyDev::tc_pack)
 int    forward_tc2_supported(const PolicyDev& p);

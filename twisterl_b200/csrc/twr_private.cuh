@@ -83,6 +83,9 @@ struct twr_policy {
     int32_t* d_obs_perms = nullptr;
     int32_t* d_act_perms = nullptr;
     void* tc_pack = nullptr;
+    // N of a GridWorld-shaped table (obs_size = N * N > 256, N <= 64) whose twists keep the reachable rows i * N + 0..3
+    // among themselves: GridWorld envs of N cells may run it on the compact table (PolicyDev::compact_n); 0 otherwise
+    int grid_n = 0;
     int64_t off_emb_b = 0;
     std::vector<int64_t> off_w, off_b;   // blob offsets of every Linear (common..., action_net..., value_net...)
 };

@@ -192,7 +192,8 @@ class Puzzle(PyBaseEnv):
 
 
 class GridWorld(PyBaseEnv):
-    """`grid_world.GridWorld(width, height, max_steps, difficulty)` (examples/grid_world/src/lib.rs:166-211)."""
+    """`grid_world.GridWorld(width, height, max_steps, difficulty)` (examples/grid_world/src/lib.rs:166-211).  Boards of
+    3 to 64 cells (up to 8x8, or 4x16, 1x64, ...) run on the device; a larger board raises RuntimeError at its first use."""
 
     def __init__(self, width: int, height: int, max_steps: int, difficulty: int):
         for v in (width, height, max_steps, difficulty):
